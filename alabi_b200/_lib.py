@@ -10,7 +10,7 @@ import ctypes
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# ALABI_B200_LIB: development override (kernel variants built by tools/ens_variants.sh)
+# ALABI_B200_LIB: load another build of the library instead (compare two builds from one tree)
 LIB_PATH = os.environ.get("ALABI_B200_LIB") or os.path.join(HERE, "libalabi_b200.so")
 
 c_double_p = ctypes.POINTER(ctypes.c_double)
@@ -62,7 +62,6 @@ SIGNATURES = {
     "ab_gp_profile_read": (ctypes.c_int, [_P, ctypes.c_int, c_double_p, ctypes.POINTER(ctypes.c_longlong)]),
     "ab_gp_create": (ctypes.c_int, [ctypes.POINTER(_P), ctypes.c_int, _P]),
     "ab_gp_destroy": (ctypes.c_int, [_P]),
-    "ab_gp_set_lookahead": (ctypes.c_int, [_P, ctypes.c_int]),
     "ab_gp_set_few_query_path": (ctypes.c_int, [_P, ctypes.c_int]),
     "ab_gp_set_variance_schedule": (ctypes.c_int, [_P, ctypes.c_int]),
     "ab_gp_append_point": (ctypes.c_int, [_P, _P]),

@@ -99,9 +99,7 @@ static int ensure_kinv(ab_gp* h) {
 static int create_resources(ab_gp* h) {
     int lo = 0, hi = 0;
     AB_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    AB_CUDA(cudaStreamCreateWithPriority(&h->panel_stream, cudaStreamNonBlocking, hi));
-    AB_CUDA(cudaEventCreateWithFlags(&h->ev_panel, cudaEventDisableTiming));
-    AB_CUDA(cudaEventCreateWithFlags(&h->ev_col, cudaEventDisableTiming));
+    AB_CUDA(cudaStreamCreateWithPriority(&h->copy_stream, cudaStreamNonBlocking, hi));
     AB_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     AB_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     AB_CUDA(cudaMalloc(&h->d_info, sizeof(int)));
@@ -155,8 +153,8 @@ int ab_gp_destroy(ab_gp* h) {
     if (h->df_tasks) cudaFree(h->df_tasks);
     if (h->cov_items) cudaFree(h->cov_items);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);
-    if (h->panel_stream) cudaStreamDestroy(h->panel_stream);
-    cudaEvent_t evs[] = {h->ev_panel, h->ev_col, h->ev_fork, h->ev_join};
+    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+    cudaEvent_t evs[] = {h->ev_fork, h->ev_join};
     for (cudaEvent_t e : evs)
         if (e) cudaEventDestroy(e);
     for (auto& fam : h->prof_ev)
@@ -168,12 +166,6 @@ int ab_gp_destroy(ab_gp* h) {
 int ab_gp_debug_stamps(ab_gp* h, void* d_buf) {
     AB_REQUIRE(h, -1, "null handle");
     h->df_dbg = d_buf;
-    return 0;
-}
-
-int ab_gp_set_lookahead(ab_gp* h, int enabled) {
-    AB_REQUIRE(h, -1, "null handle");
-    h->lookahead = enabled;
     return 0;
 }
 
@@ -294,7 +286,7 @@ int ab_gp_factor(ab_gp* h) {
     rc = ab_launch_cov(h, h->L, h->npad, 0, 1);
     if (rc) return rc;
     *reinterpret_cast<int*>(h->h_pinned + 9) = 0;
-    rc = (h->lookahead == 2) ? ab_launch_factor_dataflow(h) : ab_launch_factor(h);
+    rc = ab_launch_factor_dataflow(h);
     if (rc) return rc;
     AB_CUDA(cudaMemcpyAsync(h->h_pinned + 8, h->d_info, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     AB_CUDA(cudaStreamSynchronize(h->stream));
@@ -429,9 +421,9 @@ int ab_gp_predict_host(ab_gp* h, const double* h_Xq, int64_t m, double* h_mu, do
     // next panel has been enqueued.
     cudaEvent_t ev[2] = {h->ev_fork, h->ev_join};
     auto copy_out = [&](int64_t off, int64_t cnt, cudaEvent_t e) -> int {
-        AB_CUDA(cudaStreamWaitEvent(h->panel_stream, e, 0));
-        AB_CUDA(cudaMemcpyAsync(h_mu + off, dmu + off, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, h->panel_stream));
-        AB_CUDA(cudaMemcpyAsync(h_var + off, dvar + off, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, h->panel_stream));
+        AB_CUDA(cudaStreamWaitEvent(h->copy_stream, e, 0));
+        AB_CUDA(cudaMemcpyAsync(h_mu + off, dmu + off, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, h->copy_stream));
+        AB_CUDA(cudaMemcpyAsync(h_var + off, dvar + off, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, h->copy_stream));
         return 0;
     };
     int64_t prev_off = -1, prev_cnt = 0;
@@ -450,7 +442,7 @@ int ab_gp_predict_host(ab_gp* h, const double* h_Xq, int64_t m, double* h_mu, do
     }
     rc = copy_out(prev_off, prev_cnt, ev[(c - 1) & 1]);
     if (rc) return rc;
-    AB_CUDA(cudaStreamSynchronize(h->panel_stream));
+    AB_CUDA(cudaStreamSynchronize(h->copy_stream));
     AB_CUDA(cudaStreamSynchronize(h->stream));
     return 0;
 }

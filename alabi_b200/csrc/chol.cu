@@ -1,20 +1,16 @@
-// K2: the multi-launch blocked right-looking FP64 Cholesky with DMMA trailing updates
-// (factor schedules 0 / 1, kept as a cross-check of the dataflow kernel in
-// chol_dataflow.cu, which is the default), plus the triangular inverse and K^-1 that
-// the log-likelihood gradient and the predictive variance need, and small solve /
-// reduction helpers.  The block triangular solves live in trsv_dataflow.cu.
+// K2 around the factorisation: the factor itself is the dataflow kernel in
+// chol_dataflow.cu; this file holds what the log-likelihood, its gradient and the
+// predictive variance need from an existing factor L:
+//   * the triangular inverse L^-1 (recursive halving, DMMA GEMMs) and K^-1 = L^-T L^-1;
+//   * the rebuild of the diagonal-block inverses D_k^-1 and log-determinant parts of
+//     an imported or bordered factor (potf2_inv_kernel);
+//   * the triangular solves of a one-block factor, the residual and the final sums.
+// The block triangular solves of larger factors live in trsv_dataflow.cu.
 //
-// Replaces george BasicSolver.compute / apply_inverse / get_inverse (scipy
-// cholesky + cho_solve) reached from alabi/gp_utils.py:243, alabi/core.py:1158,
-// 1248, 1261, 1430.  Matrix layout: row-major, lower triangle, padded to a
-// multiple of AB_NB = 128 with an identity block so every tile is full.
-//
-//   step k:  potf2_inv   one CTA factors the 128x128 diagonal block in shared
-//                        memory and inverts it (D_k^-1)
-//            trsm_panel  L_ik = A_ik D_k^-T      (DMMA GEMM, K = 128)
-//            syrk        A_ij -= L_ik L_jk^T     (DMMA GEMM, K = 128)
-//   With look-ahead the panel of step k+1 runs on a high-priority stream while
-//   the rest of trailing update k is still in flight.
+// With chol_dataflow.cu, replaces george BasicSolver.compute / apply_inverse /
+// get_inverse (scipy cholesky + cho_solve) reached from alabi/gp_utils.py:243,
+// alabi/core.py:1158, 1248, 1261, 1430.  Matrix layout: row-major, lower triangle,
+// padded to a multiple of AB_NB = 128 with an identity block so every tile is full.
 #include <vector>
 #include "handle.h"
 #include "dmma_gemm.cuh"
@@ -24,73 +20,52 @@ namespace {
 
 constexpr int NB = AB_NB;
 
-using abp::potf2_inv_kernel;
-
-// ---------------------------------------------------------------------------
-// panel solve and trailing update (DMMA GEMM core)
-// ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(abg::THREADS, 1)
-trsm_panel_kernel(double* __restrict__ A, int64_t ld, int64_t o, const double* __restrict__ Dinv) {
-    extern __shared__ __align__(16) double smem[];
-    abg::Acc acc;
-    acc.zero();
-    double* Cp = A + (o + (int64_t)NB * (1 + blockIdx.x)) * ld + o;
-    abg::mainloop<true, true>(acc, Cp, ld, Dinv, NB, NB / abg::BK, smem);
-    abg::store_tile(acc, Cp, ld, 1.0, 0.0);
-}
-
-// mode 0: lower-triangular tiles of the trailing matrix starting at r0
-// mode 1: tile (blockIdx.x, 0)  — first block column
-// mode 2: first TWO block columns of an nt-row trailing matrix:
-//         blockIdx.x < nt -> (blockIdx.x, 0), else (blockIdx.x - nt + 1, 1)
-__global__ void __launch_bounds__(abg::THREADS, 1)
-syrk_kernel(double* __restrict__ A, int64_t ld, int64_t o, int64_t r0, int kdim, int mode, int nt) {
-    extern __shared__ __align__(16) double smem[];
-    int ti, tj;
-    if (mode == 0) abg::tri_decode(blockIdx.x, ti, tj);
-    else if (mode == 1 || (int)blockIdx.x < nt) { ti = blockIdx.x; tj = 0; }
-    else { ti = blockIdx.x - nt + 1; tj = 1; }
-    abg::Acc acc;
-    acc.zero();
-    const double* Ap = A + (r0 + (int64_t)ti * NB) * ld + o;
-    const double* Bp = A + (r0 + (int64_t)tj * NB) * ld + o;
-    abg::mainloop<true, true>(acc, Ap, ld, Bp, ld, kdim / abg::BK, smem);
-    abg::store_tile(acc, A + (r0 + (int64_t)ti * NB) * ld + r0 + (int64_t)tj * NB, ld, -1.0, 1.0);
-}
-
-// Small-tile variants for the panel chain (the critical path of the factorisation):
-// a panel has only T-k-1 128-tiles, far fewer than 148 SMs for N <= 16384, and a
-// 128 x 128 x 128 tile alone costs >= 17 us on one SM.  64-row tiles spread the same
-// work over 2-4x more SMs.
-using Half = abg::Core<16, 3, 1, 1, 4>;     // 64 x 128 tile, 128 threads, 90 KB (2 CTAs / SM)
-using Small = abg::Core<16, 3, 1, 1, 2>;    // 64 x 64 tile, 64 threads, 60 KB (3 CTAs / SM)
-
-// in place: the CTA reads and writes its own 64 rows x 128 columns only
-__global__ void __launch_bounds__(Half::THREADS, 2)
-trsm_half_kernel(double* __restrict__ A, int64_t ld, int64_t o, const double* __restrict__ Dinv) {
-    extern __shared__ __align__(16) double smem[];
-    abg::Acc acc;
-    acc.zero();
-    double* Cp = A + (o + (int64_t)NB * (1 + (blockIdx.x >> 1)) + 64 * (blockIdx.x & 1)) * ld + o;
-    Half::mainloop<true, true>(acc, Cp, ld, Dinv, NB, NB / Half::BK, smem);
-    Half::store_tile(acc, Cp, ld, 1.0, 0.0);
-}
-
-// modes 1 and 2 of syrk_kernel on 64 x 64 sub-tiles (4 CTAs per 128-tile; the
-// strictly-upper sub-tile of a diagonal tile is skipped)
-__global__ void __launch_bounds__(Small::THREADS, 3)
-syrk_small_kernel(double* __restrict__ A, int64_t ld, int64_t o, int64_t r0, int kdim, int mode, int nt) {
-    extern __shared__ __align__(16) double smem[];
-    const int p = blockIdx.x >> 2, sm = (blockIdx.x >> 1) & 1, sn = blockIdx.x & 1;
-    int ti, tj;
-    if (mode == 1 || p < nt) { ti = p; tj = 0; }
-    else { ti = p - nt + 1; tj = 1; }
-    if (ti == tj && sn > sm) return;
-    abg::Acc acc;
-    acc.zero();
-    const int64_t row = r0 + (int64_t)ti * NB + 64 * sm, col = r0 + (int64_t)tj * NB + 64 * sn;
-    Small::mainloop<true, true>(acc, A + row * ld + o, ld, A + col * ld + o, ld, kdim / Small::BK, smem);
-    Small::store_tile(acc, A + row * ld + col, ld, -1.0, 1.0);
+// grid = number of diagonal blocks; the matrix already holds L (an imported or bordered
+// factor): rebuild D^-1 and the log-determinant parts with the sweep of potf2.cuh.
+// CTA b works on the block at offset b * NB (the argument o is overwritten).
+__global__ void __launch_bounds__(256, 1)
+potf2_inv_kernel(double* __restrict__ A, int64_t ld, int64_t o, double* __restrict__ Dinv,
+                 double* __restrict__ logdet_part, int* __restrict__ info) {
+    o = (int64_t)blockIdx.x * NB;
+    Dinv += (int64_t)blockIdx.x * NB * NB;
+    logdet_part += blockIdx.x;
+    __shared__ abp::SweepShared sh;
+    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+    if (tid == 0) abp::mbar_init((unsigned)__cvta_generic_to_shared(&sh.mbar), 256);
+    __syncthreads();
+    double a[8][8], b[8][8];
+#pragma unroll
+    for (int r = 0; r < 8; r++)
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            // only the lower block triangle (r >= c) is ever referenced: the rest
+            // must not occupy registers
+            if (r >= c) {
+                const int i = ty + 16 * r, k = tx + 16 * c;
+                a[r][c] = (k <= i) ? A[(o + i) * ld + o + k] : 0.0;
+                b[r][c] = (k == i) ? 1.0 : 0.0;
+            }
+        }
+    unsigned phase = 0;
+    abp::potf2_sweep<false, 8>(a, b, sh, tx, ty, o, info, phase);
+    double* sdiag = sh.sdiag;
+    double* sinv = sh.sinv;
+    if (tid < 32) {
+        double s = 0.0;
+        for (int j = tid; j < NB; j += 32) s += 2.0 * log(sdiag[j]);
+        s = ab_warp_sum(s);
+        if (tid == 0) *logdet_part = s;
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const int i = ty + 16 * r;
+        const double si = sinv[i];
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int k = tx + 16 * c;
+            Dinv[i * NB + k] = (r >= c && k <= i) ? b[r][c] * si : 0.0;
+        }
+    }
 }
 
 // ---------------------------------------------------------------------------
@@ -285,10 +260,6 @@ int configure_once() {
     const bool done = dev < 64 && ((done_mask >> dev) & 1ULL);
     if (done) return 0;
     int rc = 0;
-    rc |= set_smem(trsm_panel_kernel, abg::SMEM_BYTES);
-    rc |= set_smem(syrk_kernel, abg::SMEM_BYTES);
-    rc |= set_smem(trsm_half_kernel, Half::SMEM_BYTES);
-    rc |= set_smem(syrk_small_kernel, Small::SMEM_BYTES);
     rc |= set_smem(trinv_kernel<1>, abg::SMEM_BYTES);
     rc |= set_smem(trinv_kernel<2>, abg::SMEM_BYTES);
     rc |= set_smem(kinv_kernel, abg::SMEM_BYTES);
@@ -309,85 +280,11 @@ int inv_tree(int r0, int nblk, std::vector<std::vector<InvNode>>& levels) {
 }
 }  // namespace
 
-// Right-looking factorisation with 128-wide panels whose trailing updates are
-// applied two panels at a time (K = 256 DMMA GEMMs: half the C traffic and half
-// the per-tile prologue/epilogue of a K = 128 sweep).  Pair (k, k+1):
-//   potf2(k) trsm(k) | update column k+1 with panel k | potf2(k+1) trsm(k+1)
-//   trailing(rows, cols >= k+2) -= [L_k L_k+1] [L_k L_k+1]^T
-// Look-ahead: the first two block columns of the trailing update go first, then
-// the next pair's panel chain runs on the high-priority stream while the rest
-// of the trailing update is still in flight.
-int ab_launch_factor(ab_gp* h) {
-    int rc = configure_once();
-    if (rc) return rc;
-    const int T = (int)(h->npad / NB);
-    const int64_t ld = h->npad;
-    cudaStream_t ms = h->stream;
-    AB_CUDA(cudaMemsetAsync(h->d_info, 0, sizeof(int), ms));
-    ab_prof_begin(h, AB_PROF_FACTOR);
-    ab_count_launches(3LL * T);
-    const bool la = h->lookahead != 0 && T >= 4;
-    cudaStream_t ps = la ? h->panel_stream : ms;
-    const int G = abg::THREADS, SM = abg::SMEM_BYTES;
-    auto Dk = [&](int k) { return h->Dinv + (int64_t)k * NB * NB; };
-    // panel chain of the pair starting at block k (its columns are fully updated)
-    // panel operations: 64-row tiles while a panel has fewer 128-tiles than SMs
-    auto trsm = [&](int nblk, int64_t o, const double* D) {
-        if (nblk <= 0) return;
-        if (nblk < h->nsm) trsm_half_kernel<<<2 * nblk, Half::THREADS, Half::SMEM_BYTES, ps>>>(h->L, ld, o, D);
-        else trsm_panel_kernel<<<nblk, G, SM, ps>>>(h->L, ld, o, D);
-    };
-    auto syrk_cols = [&](cudaStream_t st, int ntiles, int64_t o, int64_t r0, int kdim, int mode, int nt) {
-        if (ntiles < h->nsm) syrk_small_kernel<<<4 * ntiles, Small::THREADS, Small::SMEM_BYTES, st>>>(h->L, ld, o, r0, kdim, mode, nt);
-        else syrk_kernel<<<ntiles, G, SM, st>>>(h->L, ld, o, r0, kdim, mode, nt);
-    };
-    auto pair_panels = [&](int k) {
-        const int64_t o = (int64_t)k * NB;
-        potf2_inv_kernel<true><<<1, 256, 0, ps>>>(h->L, ld, o, Dk(k), h->logdet_parts + k, h->d_info);
-        trsm(T - k - 1, o, Dk(k));
-        if (k + 1 < T) {
-            syrk_cols(ps, T - k - 1, o, o + NB, NB, 1, 0);                               // column k+1 -= L_k L_k^T
-            potf2_inv_kernel<true><<<1, 256, 0, ps>>>(h->L, ld, o + NB, Dk(k + 1), h->logdet_parts + k + 1, h->d_info);
-            trsm(T - k - 2, o + NB, Dk(k + 1));
-        }
-    };
-    if (la) {
-        AB_CUDA(cudaEventRecord(h->ev_fork, ms));
-        AB_CUDA(cudaStreamWaitEvent(ps, h->ev_fork, 0));
-    }
-    pair_panels(0);
-    if (la) AB_CUDA(cudaEventRecord(h->ev_panel, ps));
-    for (int k = 0; k < T; k += 2) {
-        const int64_t o = (int64_t)k * NB;
-        if (la) AB_CUDA(cudaStreamWaitEvent(ms, h->ev_panel, 0));
-        const int nt = T - k - 2;                    // block rows of the trailing matrix
-        if (nt <= 0) break;
-        const int kdim = 2 * NB;
-        if (!la) {
-            syrk_kernel<<<nt * (nt + 1) / 2, G, SM, ms>>>(h->L, ld, o, o + 2 * NB, kdim, 0, nt);
-            pair_panels(k + 2);
-            continue;
-        }
-        // (a) first two block columns of the trailing update, (b) next pair's panels, (c) the rest
-        const int nfirst = nt >= 2 ? 2 * nt - 1 : nt;
-        syrk_cols(ms, nfirst, o, o + 2 * NB, kdim, 2, nt);
-        AB_CUDA(cudaEventRecord(h->ev_col, ms));
-        AB_CUDA(cudaStreamWaitEvent(ps, h->ev_col, 0));
-        pair_panels(k + 2);
-        AB_CUDA(cudaEventRecord(h->ev_panel, ps));
-        if (nt > 2)
-            syrk_kernel<<<(nt - 2) * (nt - 1) / 2, G, SM, ms>>>(h->L, ld, o, o + 4 * NB, kdim, 0, nt - 2);
-    }
-    ab_prof_end(h, AB_PROF_FACTOR);
-    AB_CHECK_LAUNCH();
-    return 0;
-}
-
 int ab_launch_rebuild_dinv(ab_gp* h) {
     int rc = configure_once();
     if (rc) return rc;
     const int T = (int)(h->npad / NB);
-    potf2_inv_kernel<false><<<T, 256, 0, h->stream>>>(h->L, h->npad, 0, h->Dinv, h->logdet_parts, h->d_info);
+    potf2_inv_kernel<<<T, 256, 0, h->stream>>>(h->L, h->npad, 0, h->Dinv, h->logdet_parts, h->d_info);
     AB_CHECK_LAUNCH();
     return 0;
 }
@@ -397,8 +294,8 @@ int ab_launch_rebuild_dinv_block(ab_gp* h, int kb) {
     int rc = configure_once();
     if (rc) return rc;
     const int64_t o = (int64_t)kb * NB;
-    potf2_inv_kernel<false><<<1, 256, 0, h->stream>>>(h->L + o * h->npad + o, h->npad, 0, h->Dinv + o * NB,
-                                                      h->logdet_parts + kb, h->d_info);
+    potf2_inv_kernel<<<1, 256, 0, h->stream>>>(h->L + o * h->npad + o, h->npad, 0, h->Dinv + o * NB,
+                                               h->logdet_parts + kb, h->d_info);
     AB_CHECK_LAUNCH();
     return 0;
 }

@@ -1,8 +1,7 @@
 // K2, dataflow form: the whole blocked Cholesky in ONE persistent kernel.
 //
 // Replaces george BasicSolver.compute (scipy cholesky) reached from
-// alabi/gp_utils.py:243, alabi/core.py:1158,1430 — same result as chol.cu's
-// multi-launch right-looking sweep, different schedule:
+// alabi/gp_utils.py:243, alabi/core.py:1158,1430:
 //
 //   * one task per 128 x 128 tile (i, j), j <= i, of the lower triangle, handed
 //     out in column-major order through an atomic counter (one CTA per SM);
@@ -75,7 +74,7 @@ __device__ __forceinline__ void gemm64(double (&acc)[4][2][2], const double* A, 
     }
 }
 
-// One matrix (strides 0) or a BATCH of equally sized matrices (k-fold cross-validation jobs,
+// One matrix or a BATCH of equally sized matrices (k-fold cross-validation jobs,
 // cv_batch.cu): matrix b lives at A + b strideA, its diagonal-block inverses at Dinv + b strideD,
 // its per-block-row words (prog, logdet_parts) at + b T, its status at info + b.  A task is
 // (i | b << 12, j); the task list orders the tiles of ALL matrices column by column, so every
@@ -88,7 +87,7 @@ struct DfArgs {
     int* abort_flag;
     const int2* tasks; int ntasks;
     unsigned long long* dbg;      // optional: 6 globaltimer stamps per task (development)
-    int64_t strideA, strideD;     // batch strides in doubles (0: single matrix)
+    int64_t strideA, strideD;     // batch strides in doubles
 };
 
 __device__ __forceinline__ unsigned long long gtime() {
@@ -400,19 +399,47 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
     }
 }
 
-}  // namespace
-
-int ab_launch_factor_dataflow(ab_gp* h) {
+// Factorisation of `nmat` matrices of T x T tiles (leading dimension T * 128), matrix b at
+// A + b * strideA etc. as described at DfArgs.  ctrl: 2 + nmat * T ints ([0] task counter,
+// [1] abort word, then prog), zeroed here with the info words; tasks: nmat * T (T + 1) / 2
+// entries.  Only the handle's own factor is timed (`profile`) and carries debug stamps.
+int launch_dataflow(ab_gp* h, double* A, int64_t strideA, int T, int nmat, double* Dinv, double* logdet_parts,
+                    int* info, int* ctrl, const int2* tasks, unsigned long long* dbg, bool profile) {
     static unsigned long long configured = 0;   // per-device bit: cudaFuncSetAttribute is per device
     if (h->device >= 64 || !((configured >> h->device) & 1ULL)) {
         AB_CUDA(cudaFuncSetAttribute(chol_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DF_SMEM_BYTES));
         if (h->device < 64) configured |= 1ULL << h->device;
     }
+    const long long ntasks = (long long)nmat * T * (T + 1) / 2;
+    cudaStream_t s = h->stream;
+    AB_CUDA(cudaMemsetAsync(ctrl, 0, (2 + (size_t)nmat * T) * sizeof(int), s));
+    AB_CUDA(cudaMemsetAsync(info, 0, (size_t)nmat * sizeof(int), s));
+    DfArgs a;
+    a.A = A; a.ld = (int64_t)T * NB; a.T = T;
+    a.Dinv = Dinv; a.logdet_parts = logdet_parts; a.info = info;
+    a.next_task = reinterpret_cast<unsigned int*>(ctrl);
+    a.abort_flag = ctrl + 1;
+    a.prog = ctrl + 2;
+    a.tasks = tasks; a.ntasks = (int)ntasks;
+    a.dbg = dbg;
+    a.strideA = strideA; a.strideD = (int64_t)T * NB * NB;
+    const int grid = ntasks < h->nsm ? (int)ntasks : h->nsm;
+    if (profile) ab_prof_begin(h, AB_PROF_FACTOR);
+    chol_dataflow_kernel<<<grid, Core::THREADS, DF_SMEM_BYTES, s>>>(a);
+    if (profile) ab_prof_end(h, AB_PROF_FACTOR);
+    ab_count_launches(1);
+    AB_CHECK_LAUNCH();
+    return 0;
+}
+
+}  // namespace
+
+// The handle's factor: L, Dinv and logdet_parts of the handle, d_info; the abort word goes to
+// h_pinned[9].  The control block sits in scratch; the task list is cached per size.
+int ab_launch_factor_dataflow(ab_gp* h) {
     const int T = (int)(h->npad / NB);
     const int ntasks = T * (T + 1) / 2;
-    // control block in scratch: [0] next_task, [1] abort, [2..2+T) prog
-    const size_t ctrl_ints = 2 + (size_t)T;
-    int rc = ab_ensure_scratch(h, ctrl_ints * sizeof(int));
+    int rc = ab_ensure_scratch(h, (2 + (size_t)T) * sizeof(int));
     if (rc) return rc;
     if (h->df_tasks_T != T) {                      // column-major task list for this T (host -> device once per size)
         std::vector<int2> tasks;
@@ -426,59 +453,20 @@ int ab_launch_factor_dataflow(ab_gp* h) {
         AB_CUDA(cudaStreamSynchronize(h->stream));
         h->df_tasks_T = T;
     }
-    cudaStream_t s = h->stream;
     int* ctrl = reinterpret_cast<int*>(h->scratch);
-    AB_CUDA(cudaMemsetAsync(ctrl, 0, ctrl_ints * sizeof(int), s));
-    AB_CUDA(cudaMemsetAsync(h->d_info, 0, sizeof(int), s));
-    DfArgs a;
-    a.A = h->L; a.ld = h->npad; a.T = T;
-    a.Dinv = h->Dinv; a.logdet_parts = h->logdet_parts; a.info = h->d_info;
-    a.next_task = reinterpret_cast<unsigned int*>(ctrl);
-    a.abort_flag = ctrl + 1;
-    a.prog = ctrl + 2;
-    a.tasks = reinterpret_cast<const int2*>(h->df_tasks); a.ntasks = ntasks;
-    a.dbg = reinterpret_cast<unsigned long long*>(h->df_dbg);
-    a.strideA = 0; a.strideD = 0;
-    const int grid = ntasks < h->nsm ? ntasks : h->nsm;
-    ab_prof_begin(h, AB_PROF_FACTOR);
-    chol_dataflow_kernel<<<grid, Core::THREADS, DF_SMEM_BYTES, s>>>(a);
-    ab_prof_end(h, AB_PROF_FACTOR);
-    ab_count_launches(1);
-    AB_CHECK_LAUNCH();
-    AB_CUDA(cudaMemcpyAsync(h->h_pinned + 9, ctrl + 1, sizeof(int), cudaMemcpyDeviceToHost, s));
+    rc = launch_dataflow(h, h->L, 0, T, 1, h->Dinv, h->logdet_parts, h->d_info, ctrl,
+                         reinterpret_cast<const int2*>(h->df_tasks), reinterpret_cast<unsigned long long*>(h->df_dbg), true);
+    if (rc) return rc;
+    AB_CUDA(cudaMemcpyAsync(h->h_pinned + 9, ctrl + 1, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     return 0;
 }
 
-// Batched factorisation of `nmat` matrices of T x T tiles each (leading dimension T * 128):
-// d_A + b * strideA etc. as described at DfArgs.  d_ctrl: at least 2 + nmat * T ints (zeroed here),
-// d_tasks: nmat * T (T + 1) / 2 int2 filled by ab_build_batch_tasks.  Asynchronous on h->stream;
-// the abort word is d_ctrl[1].
+// Batched factorisation (cv_batch.cu): d_ctrl at least 2 + nmat * T ints, d_tasks filled by
+// ab_build_batch_tasks.  Asynchronous on h->stream; the abort word is d_ctrl[1].
 int ab_launch_factor_dataflow_batch(ab_gp* h, double* d_A, int64_t strideA, int T, int nmat, double* d_Dinv,
                                     double* d_logdet_parts, int* d_info, int* d_ctrl, const int2* d_tasks) {
-    static unsigned long long configured = 0;
-    if (h->device >= 64 || !((configured >> h->device) & 1ULL)) {
-        AB_CUDA(cudaFuncSetAttribute(chol_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DF_SMEM_BYTES));
-        if (h->device < 64) configured |= 1ULL << h->device;
-    }
     if (T < 1 || T > 4095 || nmat < 1 || nmat >= (1 << 19)) { ab_set_error("batched factorisation: bad shape"); return -1; }
-    const long long ntasks = (long long)nmat * T * (T + 1) / 2;
-    cudaStream_t s = h->stream;
-    AB_CUDA(cudaMemsetAsync(d_ctrl, 0, (2 + (size_t)nmat * T) * sizeof(int), s));
-    AB_CUDA(cudaMemsetAsync(d_info, 0, (size_t)nmat * sizeof(int), s));
-    DfArgs a;
-    a.A = d_A; a.ld = (int64_t)T * NB; a.T = T;
-    a.Dinv = d_Dinv; a.logdet_parts = d_logdet_parts; a.info = d_info;
-    a.next_task = reinterpret_cast<unsigned int*>(d_ctrl);
-    a.abort_flag = d_ctrl + 1;
-    a.prog = d_ctrl + 2;
-    a.tasks = d_tasks; a.ntasks = (int)ntasks;
-    a.dbg = nullptr;
-    a.strideA = strideA; a.strideD = (int64_t)T * NB * NB;
-    const int grid = ntasks < h->nsm ? (int)ntasks : h->nsm;
-    chol_dataflow_kernel<<<grid, Core::THREADS, DF_SMEM_BYTES, s>>>(a);
-    ab_count_launches(1);
-    AB_CHECK_LAUNCH();
-    return 0;
+    return launch_dataflow(h, d_A, strideA, T, nmat, d_Dinv, d_logdet_parts, d_info, d_ctrl, d_tasks, nullptr, false);
 }
 
 // task list of a batch: column by column over all matrices (host vector)

@@ -189,21 +189,6 @@ __device__ __forceinline__ double ab_warp_sum(double v) {
     return v;
 }
 
-// Grid-wide barrier for kernels launched with cudaLaunchCooperativeKernel (all
-// CTAs co-resident).  `counter` starts at 0 and only grows; `target` is the
-// caller's running total.
-__device__ __forceinline__ void ab_grid_barrier(unsigned long long* counter, unsigned long long& target) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += gridDim.x;
-        __threadfence();
-        atomicAdd(counter, 1ULL);
-        while (*((volatile unsigned long long*)counter) < target) { }
-        __threadfence();
-    }
-    __syncthreads();
-}
-
 // error plumbing (api.cu owns the storage)
 void ab_set_error(const char* fmt, ...);
 #define AB_CUDA(call)                                                             \

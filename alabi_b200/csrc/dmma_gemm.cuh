@@ -312,7 +312,6 @@ struct Core {
 
 // configuration used by the product kernels
 using Main = Core<16, 4, 1>;            // 128 x 128 tile, 256 threads, 160 KB
-using Small = Core<16, 4, 1, 1, 2>;     // 64 x 64 tile, 64 threads, 80 KB (2 CTAs / SM)
 constexpr int BK = Main::BK, STAGES = Main::STAGES;
 constexpr int SMEM_BYTES = Main::SMEM_BYTES;
 

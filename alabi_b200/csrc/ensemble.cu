@@ -8,7 +8,7 @@
 // by a grid barrier, never by a host round trip.
 //
 // Work decomposition: small ensembles use "units" of 1, 2, 4 or 8 warps that evaluate
-// P = 2 (or 4) proposals at a time, lanes striding over the training points; large
+// P = 2 proposals at a time, lanes striding over the training points; large
 // ensembles use the wide unit (P = 32: one lane per proposal, the warps of a CTA split
 // the training points and read them as shared-memory broadcasts).  Training points are
 // SoA in shared memory, resident for the whole run when they fit, else streamed in
@@ -37,7 +37,7 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     // segment sums of split wide units (3 kinds of half-step x units x AB_ENS_MAXSEG segments x 32 proposals)
     const int max_units = (cfg->nwalkers + 31) / 32;
     const size_t cnt_bytes = ((size_t)3 * max_units * sizeof(unsigned) + 255) / 256 * 256;
-    // proposals per half-step; P = 4 per unit once 2 per unit would need several passes per CTA
+    // proposals per half-step
     int n_half = (cfg->nwalkers + 1) / 2;
     if (cfg->init_logp && cfg->nsteps == 0) n_half = cfg->nwalkers;
     const int nsm = h->nsm;
@@ -46,9 +46,6 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     int p = (n_half >= 16 * nsm) ? 32 : 2;
     if (cfg->reserved >= 2)                                                        // development override
         p = (cfg->reserved == 32) ? 32 : 2;
-#ifdef AB_ENS_WITH_P4
-    if (cfg->reserved == 4 && h->d <= 24) p = 4;
-#endif
     // dataflow schedule (ab_ensemble_config.schedule 0 = automatic, 1 = grid barriers): small ensembles
     // whose half-steps are latency bound; the launcher drops it when the training set is not resident
     const int dpad = h->d <= 2 ? 2 : h->d <= 4 ? 4 : h->d <= 8 ? 8 : h->d <= 24 ? (h->d + 3) / 4 * 4 : 32;   // the dispatch below
@@ -213,18 +210,18 @@ extern "C" int ab_ensemble_run_host(ab_gp* h, const ab_ensemble_config* cfg, dou
         cudaMemcpyAsync(h->h_pinned, h->scratch, 256, cudaMemcpyDeviceToHost, h->stream);
         for (size_t b = 0; b < pieces.size() && !rc; b++) {
             const Piece& p = pieces[b];
-            cudaError_t e = cudaStreamWaitEvent(h->panel_stream, evs[b], 0);
+            cudaError_t e = cudaStreamWaitEvent(h->copy_stream, evs[b], 0);
             if (e == cudaSuccess && p.nrows > 0) {
                 e = cudaMemcpyAsync(h_chain + p.row0 * nw * d, d_chain + p.row0 * nw * d, (size_t)(p.nrows * nw * d) * sizeof(double),
-                                    cudaMemcpyDeviceToHost, h->panel_stream);
+                                    cudaMemcpyDeviceToHost, h->copy_stream);
                 if (e == cudaSuccess)
                     e = cudaMemcpyAsync(h_logp_chain + p.row0 * nw, d_logp_chain + p.row0 * nw, (size_t)(p.nrows * nw) * sizeof(double),
-                                        cudaMemcpyDeviceToHost, h->panel_stream);
+                                        cudaMemcpyDeviceToHost, h->copy_stream);
             }
             if (e != cudaSuccess) { ab_set_error("ab_ensemble_run_host: copy failed: %s", cudaGetErrorString(e)); rc = -100 - (int)e; }
         }
     }
-    cudaStreamSynchronize(h->panel_stream);
+    cudaStreamSynchronize(h->copy_stream);
     cudaError_t es = cudaStreamSynchronize(h->stream);
     for (cudaEvent_t e : evs) cudaEventDestroy(e);
     if (rc) return rc;

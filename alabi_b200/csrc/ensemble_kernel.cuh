@@ -8,7 +8,7 @@
 // by a grid barrier, never by a host round trip.
 //
 // Work decomposition: small ensembles use "units" of 1, 2, 4 or 8 warps that evaluate
-// P = 2 (or 4) proposals at a time, lanes striding over the training points; large
+// P = 2 proposals at a time, lanes striding over the training points; large
 // ensembles use the wide unit (P = 32: one lane per proposal, the warps of a CTA split
 // the training points and read them as shared-memory broadcasts).  Training points are
 // SoA in shared memory, resident for the whole run when they fit, else streamed in
@@ -27,18 +27,9 @@
 #include <vector>
 #include "ensemble_args.h"
 
-#ifndef AB_ENS_WIDE_UNROLL
-#define AB_ENS_WIDE_UNROLL 2      // point pairs per iteration of the wide unit's inner loop (1 and 4 measured: tools/ens_variants.sh)
-#endif
-
-#ifndef AB_ENS_WARP_RING
-#define AB_ENS_WARP_RING 2        // streamed wide unit: 2 = a private ring per warp filled by bulk copies (cp.async.bulk + mbarrier: one
-                                  // instruction per 256-byte row slice), 1 = the same ring filled by 16-byte cp.async, 0 = one ring per CTA
-#endif
-
 namespace {
 
-constexpr int kWideUnroll = AB_ENS_WIDE_UNROLL;
+constexpr int kWideUnroll = 2;    // point pairs per iteration of the wide unit's inner loop (1 and 4 measured: profiles/r02b_sampler_unroll_variants.txt)
 
 // warps per CTA (EW): 8; 16 was measured slower on the c2 workload (longer proposal and compute phases)
 
@@ -107,7 +98,7 @@ __device__ __forceinline__ void grid_wait(unsigned long long* counter, unsigned 
 // AB_ENS_THROTTLE steps, arrived at once and waited for one period later, keeps any two CTAs less
 // than 2 * AB_ENS_THROTTLE steps apart, so a slot is never overwritten while a reader needs it.
 //
-// Small units (P = 2 or 4) carry one extra warp, the PREP warp: it draws the random-stream part
+// Small units (P = 2) carry one extra warp, the PREP warp: it draws the random-stream part
 // (walker, partner, stretch factor, accept threshold: three Philox blocks and two logarithms, ~1 us
 // as a serial chain) of the CTA's work items TWO items ahead of the EW compute warps, into a ring of
 // three buffers, so that chain never sits between a half-step's accept and the next gather and has a
@@ -124,8 +115,7 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
     const int CH = CHT > 0 ? CHT : A.ch;
     double* sX = sm;                 // [D][CH]
     double* sAl = sm + D * CH;       // [CH]
-    // P proposals per unit (2: small ensembles, more units; 4: large ensembles, each
-    // training point read from shared memory once per 4 kernel evaluations)
+    // P proposals per unit (2: small ensembles, more units)
     // P = 32 ("wide"): ONE unit per CTA whose proposal e belongs to LANE e of every warp; the
     // eight warps split the training points and read them as shared-memory broadcasts, so
     // there is no cross-lane reduction and the proposal / accept phases use all 32 lanes.
@@ -187,7 +177,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
     if (resident) { load_resident(); __syncthreads(); }
-#if AB_ENS_WARP_RING == 2
     // bulk-copy ring of the streamed wide unit: one mbarrier per (buffer, warp); the rows k >= d of both
     // buffers (padding dimensions) are zeroed once, no copy ever touches them
     __shared__ __align__(8) unsigned long long wbar[2][WIDE ? EW : 1];
@@ -204,7 +193,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
         }
         __syncthreads();
     }
-#endif
     unsigned long long flow_prev_target = 0;
     bool flow_have_prev = false;
     if constexpr (FLOW) {
@@ -351,7 +339,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                 item_sync();                                         // small units: this item's prep buffer is complete
                 // ---- gather (proposal lanes): own state and partner position, proposal ----
                 bool first_chunk_issued = false;
-#if AB_ENS_WARP_RING == 2
                 if constexpr (WIDE) {
                     // streamed wide unit: the first chunk of this item is requested before the gather, so it
                     // arrives while the proposal lanes fetch the walkers (the warp's buffers are free: its
@@ -373,7 +360,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                         first_chunk_issued = true;
                     }
                 }
-#endif
                 // (the compile-time-chunk kernel of the large ensembles keeps the per-lane gather: with the
                 // cooperative one its inner loop was scheduled 5 % slower, for a gather that is 1 % of its time)
                 if constexpr (WIDE && CHT == 0) {
@@ -542,27 +528,9 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                         eval_wide(sX, sAl, CH);
                     } else {
                         // every warp streams ITS slice of a chunk (the CH / EW points it evaluates) through
-                        // its own two-deep cp.async ring: no CTA barrier in the chunk loop, a warp that
-                        // falls behind delays nobody
+                        // its own two-deep ring: no CTA barrier in the chunk loop, a warp that falls behind
+                        // delays nobody
                         const int per = CH / EW, j0 = warp * per;
-                        auto issue_slice = [&](long long c0, int buf) {
-                            double* bX = sm + buf * BUF + j0;
-                            for (int idx = lane; idx < (D + 1) * (per / 2); idx += 32) {
-                                const int k = idx / (per / 2), j2 = (idx - k * (per / 2)) * 2;
-                                const double* src = (k < D) ? ((k < d) ? A.XsT + (long long)k * A.npad + c0 + j0 + j2 : nullptr)
-                                                            : A.alpha + c0 + j0 + j2;
-                                double* dst = bX + k * CH + j2;
-                                if (src) {
-                                    unsigned sa = (unsigned)__cvta_generic_to_shared(dst);
-                                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(src) : "memory");
-                                } else {
-                                    dst[0] = 0.0; dst[1] = 0.0;
-                                }
-                            }
-                            asm volatile("cp.async.commit_group;" ::: "memory");
-                        };
-#if AB_ENS_WARP_RING == 2
-                        (void)issue_slice;
                         // row slices of `per` points (256 B at per = 32) by bulk copies: lane k issues row k (lane d
                         // the alpha row), completion on the warp's own mbarrier of that buffer
                         auto issue_bulk = [&](long long c0, int buf) {
@@ -597,30 +565,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                             eval_wide(bX, bX + D * CH, CH);
                             __syncwarp();
                         }
-#elif AB_ENS_WARP_RING
-                        if (c_lo < c_hi) issue_slice((long long)c_lo * CH, 0);
-                        for (int c = c_lo; c < c_hi; c++) {
-                            if (c + 1 < c_hi) issue_slice((long long)(c + 1) * CH, (c + 1 - c_lo) & 1);
-                            else asm volatile("cp.async.commit_group;" ::: "memory");
-                            asm volatile("cp.async.wait_group 1;" ::: "memory");
-                            __syncwarp();
-                            const double* bX = sm + ((c - c_lo) & 1) * BUF;
-                            eval_wide(bX, bX + D * CH, CH);
-                            __syncwarp();
-                        }
-#else
-                        (void)issue_slice;
-                        if (c_lo < c_hi) issue_chunk((long long)c_lo * CH, 0);
-                        for (int c = c_lo; c < c_hi; c++) {
-                            if (c + 1 < c_hi) issue_chunk((long long)(c + 1) * CH, (c + 1 - c_lo) & 1);
-                            else asm volatile("cp.async.commit_group;" ::: "memory");
-                            asm volatile("cp.async.wait_group 1;" ::: "memory");
-                            csync();
-                            const double* bX = sm + ((c - c_lo) & 1) * BUF;
-                            eval_wide(bX, bX + D * CH, CH);
-                            csync();
-                        }
-#endif
                     }
                     sPart[warp][lane] = accw;
                 } else {
@@ -904,9 +848,6 @@ int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws8) 
     // wide unit: 16 warps split the training points (4 warps per scheduler hide the FP64 dependency
     // latency that 2 leave exposed: ncu, c5 share, FP64 pipe 56 % with 8 warps); one CTA per SM
     if (p == 32) return launch_ens_p<KIND, D, 32, 16>(h, A, n_half);
-#ifdef AB_ENS_WITH_P4              // 4 proposals per unit: measured, never selected; development builds only
-    if (D <= 24 && p == 4) return launch_ens_p<KIND, (D <= 24 ? D : 2), 4>(h, A, n_half);
-#endif
     if (small_cta) {
         // One 4-warp unit (+ prep warp) per CTA, two or more CTAs per SM: units that would share an
         // 8-warp CTA in lockstep instead run as independent CTAs, so one unit's publish -> poll latency
@@ -926,11 +867,6 @@ template <int KIND>
 int launch_ens_kind(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws) {
     const int d = h->d;
 #define AB_ENS(DD) return launch_ens<KIND, DD>(h, A, n_half, p, small_cta, ws)
-#ifdef AB_ENS_DEV_D2               // development: compile the d <= 2 kernels only (seconds instead of minutes)
-    if (d <= 2) AB_ENS(2);
-    ab_set_error("development build: d <= 2 only");
-    return -1;
-#else
     if (d <= 2) AB_ENS(2);
     else if (d <= 4) AB_ENS(4);
     else if (d <= 8) AB_ENS(8);
@@ -939,7 +875,6 @@ int launch_ens_kind(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int 
     else if (d <= 20) AB_ENS(20);
     else if (d <= 24) AB_ENS(24);
     else AB_ENS(32);
-#endif
 #undef AB_ENS
 }
 

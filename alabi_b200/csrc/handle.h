@@ -11,8 +11,8 @@ struct ab_gp {
     int device = 0;
     int nsm = 148;                        // SM count of the device
     cudaStream_t stream = nullptr;        // caller's stream (borrowed)
-    cudaStream_t panel_stream = nullptr;  // high-priority stream for look-ahead panels (owned)
-    cudaEvent_t ev_panel = nullptr, ev_col = nullptr, ev_fork = nullptr, ev_join = nullptr;
+    cudaStream_t copy_stream = nullptr;   // device-to-host copies that overlap the next kernels on `stream` (owned)
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 
     int64_t n = 0, npad = 0;              // training points, padded to AB_NB
     int d = 0;
@@ -49,7 +49,6 @@ struct ab_gp {
 
     int var_schedule = 0;                 // variance GEMM over full panels: 0 auto, 1 one CTA per query tile, 2 row-block pairs per CTA
     bool few_path = true;                 // m <= 8 queries: the spread-one-query kernels of predict.cu (false: batched kernels)
-    int lookahead = 2;                    // factor schedule: 0 plain sweep, 1 look-ahead streams, 2 dataflow kernel
     void* df_tasks = nullptr;             // dataflow task list (device) for df_tasks_T block rows
     int df_tasks_T = 0;
     void* cov_items = nullptr;            // work list of cov_strip_kernel for cov_items_nt tile rows
@@ -75,9 +74,8 @@ int ab_launch_scale_inputs(ab_gp* h);
 int ab_launch_scale_points(ab_gp* h, const double* X, int64_t m, double* XT, int64_t ldm);
 int ab_launch_cross_cov(ab_gp* h, const double* AT, int64_t lda, int64_t na, const double* BT, int64_t ldb,
                         int64_t nb, double* K, int64_t ld);
-// chol.cu
-int ab_launch_factor(ab_gp* h);
 int ab_launch_factor_dataflow(ab_gp* h);   // chol_dataflow.cu
+// chol.cu
 int ab_launch_trsv_dataflow(ab_gp* h, const double* r, int backward);   // trsv_dataflow.cu
 int ab_launch_trsv_single(ab_gp* h, const double* r);      // chol.cu: z = D_0^-1 r for a one-block factor
 int ab_launch_rebuild_dinv_block(ab_gp* h, int kb);        // chol.cu

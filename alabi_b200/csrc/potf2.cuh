@@ -1,5 +1,6 @@
-// Diagonal-block kernel of the blocked Cholesky: factor a 128 x 128 SPD block
-// and invert the factor, in ONE register-tiled sweep by a single CTA.
+// Diagonal-block step of the blocked Cholesky: factor an SPD block and invert the
+// factor, in ONE register-tiled sweep by a single CTA (the diagonal tasks of
+// chol_dataflow.cu; chol.cu's potf2_inv_kernel runs it on an existing factor).
 //
 // 256 threads form a 16 x 16 grid; thread (ty, tx) owns the 8 x 8 cyclic
 // sub-matrix rows {ty + 16 r}, columns {tx + 16 c} of both A (-> L) and B
@@ -157,64 +158,6 @@ __device__ __forceinline__ void potf2_sweep(double (&a)[R][R], double (&b)[R][R]
         sh.sinv[threadIdx.x] = 1.0 / dj;
     }
     __syncthreads();
-}
-
-// FACTOR = true : grid 1; factor the block at offset o, write L (upper part zeroed),
-//                 D^-1 and the log-determinant part.
-// FACTOR = false: grid = number of diagonal blocks; the matrix already holds L
-//                 (imported factor); rebuild D^-1 and the log-determinant parts.
-template <bool FACTOR>
-__global__ void __launch_bounds__(256, 1)
-potf2_inv_kernel(double* __restrict__ A, int64_t ld, int64_t o, double* __restrict__ Dinv,
-                 double* __restrict__ logdet_part, int* __restrict__ info) {
-    if (!FACTOR) {
-        o = (int64_t)blockIdx.x * NB;
-        Dinv += (int64_t)blockIdx.x * NB * NB;
-        logdet_part += blockIdx.x;
-    }
-    __shared__ SweepShared sh;
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    if (tid == 0) mbar_init((unsigned)__cvta_generic_to_shared(&sh.mbar), 256);
-    __syncthreads();
-    double a[8][8], b[8][8];
-#pragma unroll
-    for (int r = 0; r < 8; r++)
-#pragma unroll
-        for (int c = 0; c < 8; c++) {
-            // only the lower block triangle (r >= c) is ever referenced: the rest
-            // must not occupy registers
-            if (r >= c) {
-                const int i = ty + 16 * r, k = tx + 16 * c;
-                a[r][c] = (k <= i) ? A[(o + i) * ld + o + k] : 0.0;
-                b[r][c] = (k == i) ? 1.0 : 0.0;
-            }
-        }
-    unsigned phase = 0;
-    potf2_sweep<FACTOR, 8>(a, b, sh, tx, ty, o, info, phase);
-    double* sdiag = sh.sdiag;
-    double* sinv = sh.sinv;
-    if (tid < 32) {
-        double s = 0.0;
-        for (int j = tid; j < NB; j += 32) s += 2.0 * log(sdiag[j]);
-        s = ab_warp_sum(s);
-        if (tid == 0) *logdet_part = s;
-    }
-#pragma unroll
-    for (int r = 0; r < 8; r++) {
-        const int i = ty + 16 * r;
-        const double si = sinv[i];
-#pragma unroll
-        for (int c = 0; c < 8; c++) {
-            const int k = tx + 16 * c;
-            if (r >= c) {
-                if (FACTOR) A[(o + i) * ld + o + k] = (k < i) ? a[r][c] * sinv[k] : ((k == i) ? sdiag[i] : 0.0);
-                Dinv[i * NB + k] = (k <= i) ? b[r][c] * si : 0.0;
-            } else {
-                if (FACTOR) A[(o + i) * ld + o + k] = 0.0;
-                Dinv[i * NB + k] = 0.0;
-            }
-        }
-    }
 }
 
 }  // namespace abp

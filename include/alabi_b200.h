@@ -74,7 +74,6 @@ int ab_gp_profile_read(ab_gp* h, int family, double* h_ms, long long* h_count);
  *      alabi/gp_utils.py:233, alabi/core.py:1141 ------------------------------- */
 int ab_gp_create(ab_gp** out, int device, void* cuda_stream);
 int ab_gp_destroy(ab_gp* h);
-int ab_gp_set_lookahead(ab_gp* h, int enabled);
 /* predictions of <= 8 queries (GP.predict with M = 1 inside optimisers and samplers,
  * alabi/utility.py:629-946) use kernels that spread one query over the GPU and reproduce the
  * batched kernels' bits; 0 sends them through the batched kernels (cross-check), default 1 */
@@ -179,7 +178,7 @@ typedef struct ab_ensemble_config {
                             * then has a co-resident CTA) */
     int y_kind;            /* y = ys*y_scale + y_offset (0), -10^ys (1), 10^ys (2) */
     int reserved;            /* 0 in production.  Development aids: 1 = print per-phase cycle counts of
-                              * block 0 to stderr; 2 / 4 / 32 = force that many proposals per unit */
+                              * block 0 to stderr; 2 / 32 = force that many proposals per unit */
     double a;              /* stretch scale (emcee default 2.0) */
     uint64_t seed;
     int64_t first_step;    /* step counter of the first step (continuing chains) */

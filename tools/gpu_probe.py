@@ -60,11 +60,9 @@ def main():
         res["cov_ms"] = t * 1e3
         res["cov_gbs"] = 8.0 * n * n / t * 1e-9
         del K
-        for la in (0, 1):
-            lib.ab_gp_set_lookahead(h, la)
-            t = ev_time(lambda: lib.ab_gp_factor(h), reps=3)
-            res[f"factor_la{la}_ms"] = t * 1e3
-            res[f"factor_la{la}_tflops"] = n ** 3 / 3 / t * 1e-12
+        t = ev_time(lambda: lib.ab_gp_factor(h), reps=3)
+        res["factor_ms"] = t * 1e3
+        res["factor_tflops"] = n ** 3 / 3 / t * 1e-12
         yd = torch.from_numpy(y).cuda()
         ll = ctypes.c_double()
         t = ev_time(lambda: lib.ab_gp_log_likelihood(h, _lib.ptr(yd), ctypes.byref(ll)), reps=3)
