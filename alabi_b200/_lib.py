@@ -70,6 +70,8 @@ SIGNATURES = {
     "ab_gp_set_inputs": (ctypes.c_int, [_P, _P, ctypes.c_int64, ctypes.c_int]),
     "ab_gp_set_kernel": (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_double, c_double_p, ctypes.c_double,
                                         ctypes.c_double, ctypes.c_double]),
+    "ab_gp_set_kernel_rq": (ctypes.c_int, [_P, ctypes.c_double, ctypes.c_double, c_double_p, ctypes.c_double,
+                                           ctypes.c_double, ctypes.c_double]),
     "ab_gp_build_cov": (ctypes.c_int, [_P, _P, ctypes.c_int]),
     "ab_gp_cross_cov": (ctypes.c_int, [_P, _P, ctypes.c_int64, _P, ctypes.c_int64, _P]),
     "ab_gp_factor": (ctypes.c_int, [_P]),

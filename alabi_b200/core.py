@@ -36,7 +36,7 @@ from .gp import GP
 __all__ = ["SurrogateModel", "CachedSurrogateLikelihood"]
 
 _KERNELS = {"ExpSquaredKernel": kernels.ExpSquaredKernel, "Matern32Kernel": kernels.Matern32Kernel,
-            "Matern52Kernel": kernels.Matern52Kernel}
+            "Matern52Kernel": kernels.Matern52Kernel, "RationalQuadraticKernel": kernels.RationalQuadraticKernel}
 
 
 class CachedSurrogateLikelihood:
@@ -247,6 +247,8 @@ class SurrogateModel(object):
                 [v * 10 ** self.gp_amp_rng[0], v * 10 ** self.gp_amp_rng[1]]
         if self.fit_white_noise:
             hp_bounds[pnames.index("white_noise:value")] = [self.white_noise - 3, self.white_noise + 3]
+        if self._alpha_key() in pnames:
+            hp_bounds[pnames.index(self._alpha_key())] = self.gp_alpha_rng
         if self.uniform_scales:
             hp_bounds[pnames.index(f"{self.kernel_scale_key}:metric:log_M")] = self.gp_scale_rng
         else:
@@ -267,10 +269,16 @@ class SurrogateModel(object):
                          (self.fit_white_noise, "white_noise:value")):
             if on:
                 full[pf.index(name)] = optimized_params[po.index(name)]
+        if self._alpha_key() in pf:
+            full[pf.index(self._alpha_key())] = optimized_params[po.index(self._alpha_key())]
         for ii in range(self.ndim):
             full[pf.index(f"{self.kernel_scale_key}:metric:log_M_{ii}_{ii}")] = \
                 optimized_params[po.index(f"{self.kernel_scale_key}:metric:log_M")]
         return np.array(full)
+
+    def _alpha_key(self):
+        """Name of the rational quadratic kernel's log_alpha in the george vector (absent for the other kernels)."""
+        return f"{self.kernel_scale_key}:log_alpha"
 
     def set_hyperparameter_vector(self, tmp_gp, optimized_params):
         if optimized_params is None:
@@ -303,7 +311,8 @@ class SurrogateModel(object):
 
     # -- GP initialisation (alabi/core.py:736-1094) ---------------------------------------
     def init_gp(self, kernel="ExpSquaredKernel", fit_amp=True, fit_mean=True, fit_white_noise=True,
-                white_noise=-12, gp_scale_rng=[-2, 2], gp_amp_rng=[-1, 1], uniform_scales=False, overwrite=False,
+                white_noise=-12, gp_scale_rng=[-2, 2], gp_amp_rng=[-1, 1], gp_alpha_rng=[-2, 2], uniform_scales=False,
+                overwrite=False,
                 theta_scaler=ut.no_scaler, y_scaler=ut.no_scaler, gp_opt_method="l-bfgs-b", gp_nopt=3,
                 optimizer_kwargs={"maxiter": 100, "xatol": 1e-4, "fatol": 1e-3, "adaptive": True},
                 hyperopt_method="cv", regularize=True, amp_0=1.0, mu_0=1.0, sigma_0=2.0, cv_folds=5,
@@ -335,13 +344,19 @@ class SurrogateModel(object):
             "training_mse", "test_mse", "training_scaled_mse", "test_scaled_mse", "gp_kl_divergence",
             "gp_train_time", "obj_fn_opt_time", "acquisition_optimizer_niter")}
         self.gp_scale_rng, self.gp_amp_rng = gp_scale_rng, gp_amp_rng
+        self.gp_alpha_rng = gp_alpha_rng      # bounds of ln(alpha) (RationalQuadraticKernel only)
         log_metric_bounds = [(min(gp_scale_rng), max(gp_scale_rng)) for _ in range(self.ndim)]
         if kernel not in _KERNELS:
             raise ValueError(f"Kernel '{kernel}' is not a valid option. Valid options: " + ", ".join(_KERNELS))
         self.gp = None
         for attempt in range(1, 11):       # retry with new random scale lengths (alabi/core.py:980-1048)
             log_l = np.random.uniform(min(gp_scale_rng), max(gp_scale_rng), self.ndim)
-            self.kernel = _KERNELS[kernel](metric=np.exp(log_l), metric_bounds=log_metric_bounds, ndim=self.ndim)
+            if kernel == "RationalQuadraticKernel":
+                # starts at alpha = 1; the reference's starting value for this kernel could not be checked
+                self.kernel = _KERNELS[kernel](log_alpha=0.0, metric=np.exp(log_l), metric_bounds=log_metric_bounds,
+                                               ndim=self.ndim)
+            else:
+                self.kernel = _KERNELS[kernel](metric=np.exp(log_l), metric_bounds=log_metric_bounds, ndim=self.ndim)
             self.kernel_name = kernel
             self.gp = gp_utils.configure_gp(self._theta, self._y, self.kernel, fit_amp=fit_amp, fit_mean=fit_mean,
                                             fit_white_noise=fit_white_noise, white_noise=white_noise,
@@ -365,6 +380,8 @@ class SurrogateModel(object):
             self.param_names_optimized.append(f"{self.kernel_amp_key}:log_constant")
         if fit_white_noise:
             self.param_names_optimized.append("white_noise:value")
+        if self._alpha_key() in self.param_names_full:
+            self.param_names_optimized.append(self._alpha_key())
         if self.uniform_scales:
             self.param_names_optimized.append(f"{self.kernel_scale_key}:metric:log_M")
         else:

@@ -2,6 +2,7 @@
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
+#include <cmath>
 #include "handle.h"
 #include "alabi_b200.h"
 
@@ -220,11 +221,8 @@ int ab_gp_set_inputs(ab_gp* h, const double* d_X, int64_t n, int d) {
     return 0;
 }
 
-int ab_gp_set_kernel(ab_gp* h, int kernel_id, double amp, const double* h_log_M, double mean, double white_noise,
-                     double yerr2) {
-    AB_REQUIRE(h && h_log_M, -1, "ab_gp_set_kernel: null argument");
-    AB_REQUIRE(kernel_id >= 0 && kernel_id <= 2, -1, "ab_gp_set_kernel: unknown kernel id %d", kernel_id);
-    AB_REQUIRE(h->have_inputs, -2, "ab_gp_set_kernel: call ab_gp_set_inputs first");
+static int set_kernel(ab_gp* h, int kernel_id, double amp, double alpha, const double* h_log_M, double mean,
+                      double white_noise, double yerr2) {
     h->kp.kind = kernel_id;
     h->kp.d = h->d;
     h->kp.amp = amp;
@@ -233,12 +231,32 @@ int ab_gp_set_kernel(ab_gp* h, int kernel_id, double amp, const double* h_log_M,
         h->log_M[k] = (k < h->d) ? h_log_M[k] : 0.0;
         h->kp.inv_len[k] = (k < h->d) ? exp(-0.5 * h_log_M[k]) : 0.0;
     }
+    h->kp.alpha = alpha;
+    h->kp.inv2a = (alpha > 0.0) ? 0.5 / alpha : 0.0;
     h->mean = mean;
     h->white_noise = white_noise;
     h->yerr2 = yerr2;
     h->have_kernel = true;
     h->scaled = h->factored = h->have_linv = h->have_kinv = h->have_alpha = false;
     return 0;
+}
+
+int ab_gp_set_kernel(ab_gp* h, int kernel_id, double amp, const double* h_log_M, double mean, double white_noise,
+                     double yerr2) {
+    AB_REQUIRE(h && h_log_M, -1, "ab_gp_set_kernel: null argument");
+    AB_REQUIRE(kernel_id >= 0 && kernel_id <= 2, -1, "ab_gp_set_kernel: unknown kernel id %d", kernel_id);
+    AB_REQUIRE(h->have_inputs, -2, "ab_gp_set_kernel: call ab_gp_set_inputs first");
+    return set_kernel(h, kernel_id, amp, 0.0, h_log_M, mean, white_noise, yerr2);
+}
+
+int ab_gp_set_kernel_rq(ab_gp* h, double amp, double log_alpha, const double* h_log_M, double mean,
+                        double white_noise, double yerr2) {
+    AB_REQUIRE(h && h_log_M, -1, "ab_gp_set_kernel_rq: null argument");
+    const double alpha = exp(log_alpha);
+    AB_REQUIRE(std::isfinite(alpha) && alpha > 0.0 && std::isfinite(0.5 / alpha), -1,
+               "ab_gp_set_kernel_rq: alpha = exp(%g) is not finite and positive (or 1 / (2 alpha) overflows)", log_alpha);
+    AB_REQUIRE(h->have_inputs, -2, "ab_gp_set_kernel_rq: call ab_gp_set_inputs first");
+    return set_kernel(h, AB_KERNEL_RATQUAD, amp, alpha, h_log_M, mean, white_noise, yerr2);
 }
 
 static int ensure_scaled(ab_gp* h) {
@@ -356,7 +374,7 @@ int ab_gp_grad_log_likelihood(ab_gp* h, const double* d_y, double* h_out) {
     rc = ab_launch_grad(h, nullptr);
     if (rc) return rc;
     AB_CUDA(cudaStreamSynchronize(h->stream));
-    memcpy(h_out, h->h_pinned, (h->d + 3) * sizeof(double));
+    memcpy(h_out, h->h_pinned, (h->d + 3 + (h->kp.kind == AB_KERNEL_RATQUAD ? 1 : 0)) * sizeof(double));
     return 0;
 }
 

@@ -32,7 +32,7 @@ __global__ void append_cross_kernel(const double* __restrict__ Xs, int64_t n0, i
             const double df = Xs[j * d + k] - Xs[n0 * d + k];
             r2 = fma(df, df, r2);
         }
-        v = kp.amp * ab_radial<KIND>(r2);
+        v = kp.amp * ab_radial<KIND>(r2, kp.alpha, kp.inv2a);
     }
     out[j] = v;
 }
@@ -52,7 +52,7 @@ append_row_kernel(double* __restrict__ L, int64_t ld, int64_t n0, const double* 
     if (threadIdx.x == 0) {
         double q = 0.0;
         for (int w = 0; w < 32; w++) q += sh[w];
-        const double lam2 = kp.amp * ab_radial<KIND>(0.0) + kp.diag_add - q;
+        const double lam2 = kp.amp * ab_radial<KIND>(0.0, kp.alpha, kp.inv2a) + kp.diag_add - q;
         if (!(lam2 > 0.0)) { *info = (int)(n0 + 1); s_lam = -1.0; }
         else s_lam = sqrt(lam2);
     }

@@ -15,11 +15,13 @@
 // 1/sqrt(M_k) so r^2 is a plain squared distance (george: r^2 = sum dx_k^2 / M_k;
 // reference call site alabi/core.py:998-1014).
 struct KernParams {
-    int kind;                     // 0 ExpSquared, 1 Matern32, 2 Matern52
+    int kind;                     // 0 ExpSquared, 1 Matern32, 2 Matern52, 3 RationalQuadratic
     int d;
     double amp;                   // exp(log_constant), 1 without an amplitude
     double diag_add;              // yerr^2 + exp(white_noise)
     double inv_len[AB_MAX_DIM];   // exp(-0.5 log_M_k)
+    double alpha;                 // RationalQuadratic: exp(log_alpha); 0 for kinds 0-2
+    double inv2a;                 // RationalQuadratic: 1 / (2 alpha); 0 for kinds 0-2
 };
 
 // 2^(j/64), j = 0..63, correctly rounded (global memory, L1 resident: 512 B)
@@ -144,32 +146,73 @@ __device__ __forceinline__ double ab_exp_sel(double x) { return TAB ? ab_exp_neg
 template <bool TAB>
 __device__ __forceinline__ double ab_exp_half_sel(double r2) { return TAB ? ab_exp_neg_half(r2) : ab_exp_neg_poly(-0.5 * r2); }
 
+// The radial profiles k(r^2).  alpha and inv2a = 1 / (2 alpha) are read by the rational quadratic
+// kernel (KIND 3) only, k = (1 + r^2 / (2 alpha))^(-alpha) = exp(-alpha log1p(x)), x = r^2 inv2a;
+// kinds 0-2 ignore them.
 template <int KIND, bool TAB = true>
-__device__ __forceinline__ double ab_radial(double r2) {
+__device__ __forceinline__ double ab_radial(double r2, double alpha, double inv2a) {
     if (KIND == 0) return ab_exp_half_sel<TAB>(r2);
     if (KIND == 1) { double r = ab_sqrt_pos(3.0 * r2); return (1.0 + r) * ab_exp_sel<TAB>(-r); }
+    if (KIND == 3) return ab_exp_sel<TAB>(-alpha * log1p(r2 * inv2a));
     double r = ab_sqrt_pos(5.0 * r2);
     return (1.0 + r + r * r * 0.3333333333333333) * ab_exp_sel<TAB>(-r);
 }
 
 // dk/d(r^2)
 template <int KIND, bool TAB = true>
-__device__ __forceinline__ double ab_radial_grad(double r2) {
+__device__ __forceinline__ double ab_radial_grad(double r2, double alpha, double inv2a) {
     if (KIND == 0) return -0.5 * ab_exp_half_sel<TAB>(r2);
     if (KIND == 1) { double r = ab_sqrt_pos(3.0 * r2); return -1.5 * ab_exp_sel<TAB>(-r); }
+    if (KIND == 3) {
+        const double x = r2 * inv2a;
+        return -0.5 * ab_exp_sel<TAB>(-alpha * log1p(x)) / (1.0 + x);
+    }
     double r = ab_sqrt_pos(5.0 * r2);
     return -5.0 * (1.0 + r) * ab_exp_sel<TAB>(-r) * 0.16666666666666666;
 }
 
-// k(r^2) and dk/d(r^2) from ONE exponential (the gradient kernels need both)
+// g(x) = log1p(x) - x / (1 + x) >= 0 for x >= 0, the rational quadratic kernel's dk/dlog(alpha) =
+// -alpha k g(x).  For small x the two terms cancel: evaluated directly, g's relative error is about
+// 5 eps / x (log1p and the quotient each carry ~1 ulp of a number ~x, g ~ x^2 / 2), which is total
+// for x < eps.  Below x = 1/16 the alternating series g = sum_{n>=2} (-1)^n (n-1)/n x^n is used
+// instead: through x^15 its truncation is below 2 (15/16) x^14 ~ 3e-17 relative at x = 1/16, and
+// the direct form's error at the switch is <= 80 eps ~ 2e-14 relative.  inv1px = 1 / (1 + x).
+__device__ __forceinline__ double ab_rq_g(double x, double l, double inv1px) {
+    double p = -0.93333333333333333;                   // -14/15 (x^15)
+    p = fma(p, x, 0.92857142857142857);                // 13/14
+    p = fma(p, x, -0.92307692307692308);               // -12/13
+    p = fma(p, x, 0.91666666666666667);                // 11/12
+    p = fma(p, x, -0.90909090909090909);               // -10/11
+    p = fma(p, x, 0.9);                                // 9/10
+    p = fma(p, x, -0.88888888888888889);               // -8/9
+    p = fma(p, x, 0.875);                              // 7/8
+    p = fma(p, x, -0.85714285714285714);               // -6/7
+    p = fma(p, x, 0.83333333333333333);                // 5/6
+    p = fma(p, x, -0.8);                               // -4/5
+    p = fma(p, x, 0.75);                               // 3/4
+    p = fma(p, x, -0.66666666666666667);               // -2/3
+    p = fma(p, x, 0.5);                                // 1/2 (x^2)
+    const double series = p * x * x;
+    return (x < 0.0625) ? series : l - x * inv1px;
+}
+
+// k(r^2) and dk/d(r^2) from ONE exponential (the gradient kernels need both); for the rational
+// quadratic kernel also av = dk/dlog(alpha) = -alpha k g(x), from the same log1p and exponential and
+// one reciprocal (kinds 0-2 set av = 0)
 template <int KIND, bool TAB = true>
-__device__ __forceinline__ void ab_radial_both(double r2, double& kv, double& gv) {
+__device__ __forceinline__ void ab_radial_both(double r2, double alpha, double inv2a, double& kv, double& gv,
+                                               double& av) {
+    av = 0.0;
     if (KIND == 0) {
         const double e = ab_exp_half_sel<TAB>(r2);
         kv = e; gv = -0.5 * e;
     } else if (KIND == 1) {
         const double r = ab_sqrt_pos(3.0 * r2), e = ab_exp_sel<TAB>(-r);
         kv = (1.0 + r) * e; gv = -1.5 * e;
+    } else if (KIND == 3) {
+        const double x = r2 * inv2a, l = log1p(x), e = ab_exp_sel<TAB>(-alpha * l);
+        const double inv1px = 1.0 / (1.0 + x);
+        kv = e; gv = -0.5 * e * inv1px; av = -alpha * e * ab_rq_g(x, l, inv1px);
     } else {
         const double r = ab_sqrt_pos(5.0 * r2), e = ab_exp_sel<TAB>(-r);
         kv = (1.0 + r + r * r * 0.3333333333333333) * e; gv = -5.0 * (1.0 + r) * e * 0.16666666666666666;
@@ -180,7 +223,8 @@ __device__ __forceinline__ void ab_radial_both(double r2, double& kv, double& gv
     do {                                                              \
         if ((kind) == 0) { constexpr int KIND = 0; __VA_ARGS__; }     \
         else if ((kind) == 1) { constexpr int KIND = 1; __VA_ARGS__; }\
-        else { constexpr int KIND = 2; __VA_ARGS__; }                 \
+        else if ((kind) == 2) { constexpr int KIND = 2; __VA_ARGS__; }\
+        else { constexpr int KIND = 3; __VA_ARGS__; }                 \
     } while (0)
 
 __device__ __forceinline__ double ab_warp_sum(double v) {

@@ -83,7 +83,7 @@ cov_kernel(const double* __restrict__ AT, int64_t lda, int64_t na, const double*
 #pragma unroll
         for (int c = 0; c < 4; c++) {
             int64_t gi = i0 + ty * 4 + r, gj = j0 + tx * 4 + c;
-            double x = kp.amp * ab_radial<KIND, false>(r2[r][c]);
+            double x = kp.amp * ab_radial<KIND, false>(r2[r][c], kp.alpha, kp.inv2a);
             if (symmetric) {
                 if (gi == gj) x += kp.diag_add;
                 if (pad_identity && (gi >= n_valid || gj >= n_valid)) x = (gi == gj) ? 1.0 : 0.0;
@@ -183,7 +183,7 @@ cov_strip_kernel(const double* __restrict__ XT, int64_t ldx, int64_t n_valid, Ke
 #pragma unroll
             for (int c = 0; c < 4; c++) {
                 const int64_t gj = j0 + tx * 4 + c;
-                double x = kp.amp * ab_radial<KIND, false>(r2[r][c]);
+                double x = kp.amp * ab_radial<KIND, false>(r2[r][c], kp.alpha, kp.inv2a);
                 if (gi == gj) x += kp.diag_add;
                 if (gi >= n_valid || gj >= n_valid) x = (gi == gj) ? 1.0 : 0.0;
                 v[c] = x;

@@ -17,6 +17,7 @@
 //
 // Jobs are processed in chunks sized to a workspace budget.  Results per job: predictions, the
 // log-likelihood and the Cholesky status (first non-positive pivot, 0 = ok).
+#include <cmath>
 #include <vector>
 #include "handle.h"
 #include "alabi_b200.h"
@@ -32,6 +33,7 @@ constexpr int NB = AB_NB;
 struct CandParams {
     double amp, diag_add, mean;
     double inv_len[AB_MAX_DIM];
+    double alpha, inv2a;          // rational quadratic kernel only (0 for kinds 0-2)
 };
 
 struct CvArgs {
@@ -109,7 +111,7 @@ cvb_cov_kernel(const CvArgs a) {
                     const double df = sR[lr * pitch + k] - sCo[lc * pitch + k];
                     r2 = fma(df, df, r2);
                 }
-                v = c.amp * ab_radial<KIND>(r2) + ((gi == gj) ? c.diag_add : 0.0);
+                v = c.amp * ab_radial<KIND>(r2, c.alpha, c.inv2a) + ((gi == gj) ? c.diag_add : 0.0);
             } else {
                 v = (gi == gj) ? 1.0 : 0.0;                  // identity padding
             }
@@ -200,7 +202,7 @@ cvb_solve_predict_kernel(const CvArgs a) {
                 const double df = xv[k] - Xs[(int64_t)j * d + k];
                 r2 = fma(df, df, r2);
             }
-            m = fma(ab_radial<KIND>(r2), x[j], m);
+            m = fma(ab_radial<KIND>(r2, c.alpha, c.inv2a), x[j], m);
         }
         a.pred[(int64_t)job * a.ld_val + v] = fma(c.amp, m, c.mean);
     }
@@ -233,7 +235,7 @@ extern "C" int ab_gp_cv_batch(ab_gp* h, const double* d_X, const double* d_y, in
                               double* d_pred, double* h_loglik, int* h_status, void* d_work, size_t work_bytes) {
     if (!h || !d_X || !d_y || !h_params || !h_job_cand || !h_ntrain || !h_nval || !d_train_idx || !d_val_idx || !d_pred ||
         !h_loglik || !h_status) { ab_set_error("ab_gp_cv_batch: null argument"); return -1; }
-    if (n < 2 || d < 1 || d > AB_MAX_DIM || kernel_id < 0 || kernel_id > 2 || ncand < 1 || njobs < 1 || ld_train < 1 || ld_val < 1) {
+    if (n < 2 || d < 1 || d > AB_MAX_DIM || kernel_id < 0 || kernel_id > AB_KERNEL_RATQUAD || ncand < 1 || njobs < 1 || ld_train < 1 || ld_val < 1) {
         ab_set_error("ab_gp_cv_batch: bad argument"); return -1;
     }
     AB_CUDA(cudaSetDevice(h->device));
@@ -245,14 +247,21 @@ extern "C" int ab_gp_cv_batch(ab_gp* h, const double* d_X, const double* d_y, in
         if (h_ntrain[j] > nt_max) nt_max = h_ntrain[j];
     }
     const int npad = (nt_max + NB - 1) / NB * NB, T = npad / NB;
-    // candidates: [mean, white_noise, amp, log_M...]
+    // candidates: [mean, white_noise, amp, log_M...], [mean, white_noise, amp, log_alpha, log_M...] (RQ)
+    const int nx = (kernel_id == AB_KERNEL_RATQUAD) ? 1 : 0;
     std::vector<CandParams> cp(ncand);
     for (int c = 0; c < ncand; c++) {
-        const double* p = h_params + (size_t)c * (3 + d);
+        const double* p = h_params + (size_t)c * (3 + nx + d);
         cp[c].mean = p[0];
         cp[c].diag_add = exp(p[1]);
         cp[c].amp = p[2];
-        for (int k = 0; k < AB_MAX_DIM; k++) cp[c].inv_len[k] = (k < d) ? exp(-0.5 * p[3 + k]) : 0.0;
+        for (int k = 0; k < AB_MAX_DIM; k++) cp[c].inv_len[k] = (k < d) ? exp(-0.5 * p[3 + nx + k]) : 0.0;
+        cp[c].alpha = nx ? exp(p[3]) : 0.0;
+        cp[c].inv2a = nx ? 0.5 / cp[c].alpha : 0.0;
+        if (nx && !(std::isfinite(cp[c].alpha) && cp[c].alpha > 0.0 && std::isfinite(cp[c].inv2a))) {
+            ab_set_error("ab_gp_cv_batch: candidate %d: alpha = exp(%g) is not finite and positive", c, p[3]);
+            return -1;
+        }
     }
     // the caller's workspace decides how many jobs are factorised per launch
     const size_t fixed = sizeof(CandParams) * ncand + (size_t)njobs * (3 * sizeof(int) + sizeof(double)) + 4096;

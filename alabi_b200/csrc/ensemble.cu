@@ -141,7 +141,8 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     const int small_cta = (p != 2) ? 0 : (cfg->warps_per_unit == 104) ? 2 : (cfg->warps_per_unit == 0 && ws < 8) ? 1 : 0;
     rc = (h->kp.kind == 0) ? ab_ens_launch_k0(h, A, n_half, p, small_cta, ws)
        : (h->kp.kind == 1) ? ab_ens_launch_k1(h, A, n_half, p, small_cta, ws)
-                           : ab_ens_launch_k2(h, A, n_half, p, small_cta, ws);
+       : (h->kp.kind == 2) ? ab_ens_launch_k2(h, A, n_half, p, small_cta, ws)
+                           : ab_ens_launch_k3(h, A, n_half, p, small_cta, ws);
     if (rc) return rc;
     h->ens_dbg = A.dbg != nullptr; h->ens_ws = A.ws;
     return 0;

@@ -52,3 +52,4 @@ struct EnsArgs {
 int ab_ens_launch_k0(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
 int ab_ens_launch_k1(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
 int ab_ens_launch_k2(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
+int ab_ens_launch_k3(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);

@@ -520,8 +520,8 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                                 s1 = fma(e1, e1, s1);
                             }
                             const double2 al = *reinterpret_cast<const double2*>(&bAl[j]);
-                            accw = fma(ab_radial<KIND>(r0 + s0), al.x, accw);
-                            accw = fma(ab_radial<KIND>(r1 + s1), al.y, accw);
+                            accw = fma(ab_radial<KIND>(r0 + s0, A.kp.alpha, A.kp.inv2a), al.x, accw);
+                            accw = fma(ab_radial<KIND>(r1 + s1, A.kp.alpha, A.kp.inv2a), al.y, accw);
                         }
                     };
                     if (resident) {
@@ -592,7 +592,7 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                         }
                         const double al = bAl[jj];
 #pragma unroll
-                        for (int e = 0; e < P; e++) acc[e] = fma(ab_radial<KIND>(r[e]), al, acc[e]);
+                        for (int e = 0; e < P; e++) acc[e] = fma(ab_radial<KIND>(r[e], A.kp.alpha, A.kp.inv2a), al, acc[e]);
                     }
                 };
                 if (resident) {

@@ -156,8 +156,8 @@ nested_walk_kernel(const __grid_constant__ WalkArgs A) {
                     r1 = fma(d1, d1, r1);
                 }
                 const double2 al = *reinterpret_cast<const double2*>(&sAl[j]);
-                acc = fma(ab_radial<KIND>(r0), al.x, acc);
-                acc = fma(ab_radial<KIND>(r1), al.y, acc);
+                acc = fma(ab_radial<KIND>(r0, A.kp.alpha, A.kp.inv2a), al.x, acc);
+                acc = fma(ab_radial<KIND>(r1, A.kp.alpha, A.kp.inv2a), al.y, acc);
             }
         };
         if (resident) {

@@ -71,7 +71,7 @@ predict_mean_kernel(const double* __restrict__ Xq, int64_t m, int64_t q_off, con
                 ra = fma(da0, da0, ra); ra = fma(da1, da1, ra);
                 rb = fma(db0, db0, rb); rb = fma(db1, db1, rb);
             }
-            double ka = ab_radial<KIND>(ra), kb = ab_radial<KIND>(rb);
+            double ka = ab_radial<KIND>(ra, kp.alpha, kp.inv2a), kb = ab_radial<KIND>(rb, kp.alpha, kp.inv2a);
             const double al = sAl[jj];
             ma = fma(ka, al, ma);
             mb = fma(kb, al, mb);
@@ -316,7 +316,7 @@ predict_grad_kernel(const double* __restrict__ Xq, int64_t m, int64_t q_off, con
                 df[k] = x[k] - sX[jj * D + k];
                 r2 = fma(df[k], df[k], r2);
             }
-            const double g = ab_radial_grad<KIND>(r2);
+            const double g = ab_radial_grad<KIND>(r2, kp.alpha, kp.inv2a);
             const double c1 = sAl[jj] * g, c2 = V[(j0 + jj) * ldp + q] * g;
 #pragma unroll
             for (int k = 0; k < D; k++) {
@@ -483,7 +483,7 @@ few_cross_kernel(const double* __restrict__ Xq, int m, const double* __restrict_
                 const double df = sQ[q][k] - x[k];
                 r = fma(df, df, r);
             }
-            kq = ab_radial<KIND>(r);
+            kq = ab_radial<KIND>(r, kp.alpha, kp.inv2a);
         }
         sK[q][tid] = kq;
         if (P && j < npad) P[j * FEW_MQ + q] = (q < m && j < n) ? kp.amp * kq : 0.0;
@@ -693,7 +693,7 @@ few_grad_kernel(const double* __restrict__ Xq, int m, const double* __restrict__
                     const double df = sQ[eq][k] - sX[ejj * D + k];
                     r2 = fma(df, df, r2);
                 }
-                g = ab_radial_grad<KIND>(r2);
+                g = ab_radial_grad<KIND>(r2, kp.alpha, kp.inv2a);
                 vv = V[(int64_t)eq * ldv + j0 + ejj];
             }
             sG[eq][ejj] = g;

@@ -182,8 +182,8 @@ class GP:
 
     def _spec_key(self):
         kid, amp, log_M = self.kernel.spec()
-        return (int(kid), float(amp), np.asarray(log_M, dtype=np.float64).tobytes(), float(self.mean_value),
-                float(self.white_noise_value), float(self._yerr2))
+        return (int(kid), float(amp), np.asarray(log_M, dtype=np.float64).tobytes(), _log_alpha(self.kernel),
+                float(self.mean_value), float(self.white_noise_value), float(self._yerr2))
 
     def get_parameter_dict(self, include_frozen=False):
         return dict(zip(self.get_parameter_names(include_frozen), self.get_parameter_vector(include_frozen)))
@@ -242,9 +242,7 @@ class GP:
             self._inputs_pushed = True
             self._kernel_pushed = False
         if not self._kernel_pushed:
-            kid, amp, log_M = self.kernel.spec()
-            _lib.check(hd.lib.ab_gp_set_kernel(hd.h, kid, amp, log_M.ctypes.data_as(_lib.c_double_p), self.mean_value,
-                                               self.white_noise_value, float(self._yerr2)), "ab_gp_set_kernel")
+            _set_kernel(hd, self.kernel, self.mean_value, self.white_noise_value, float(self._yerr2))
             self._kernel_pushed = True
             self._targets_pushed = False
 
@@ -364,7 +362,8 @@ class GP:
         y = np.ascontiguousarray(np.asarray(y, dtype=np.float64).reshape(-1))
         hd = self._hd
         d = self._x.shape[1]
-        out = (ctypes.c_double * (d + 3))()
+        nx = 1 if self.kernel.kernel_id == RQ_KERNEL_ID else 0   # the log_alpha entry
+        out = (ctypes.c_double * (d + 3 + nx))()
         if self._targets_pushed and self._y is not None and np.array_equal(y, self._y):
             yp = None                    # alpha of the preceding log_likelihood / predict is still valid
         else:
@@ -383,9 +382,9 @@ class GP:
         if self.fit_kernel:
             if isinstance(self.kernel, Product):
                 g.append(full[2])
-                gm = full[3:3 + d]
-            else:
-                gm = full[3:3 + d]
+            if nx:
+                g.append(full[3])
+            gm = full[3 + nx:3 + nx + d]
             g += [gm.sum()] if getattr(self.kernel if not isinstance(self.kernel, Product) else self.kernel.k2,
                                        "isotropic", False) else list(gm)
         return np.array(g, dtype=np.float64)
@@ -539,14 +538,17 @@ class GP:
                 raise ValueError("folds must hold the same number of folds for every candidate (or pass job_cand)")
             job_cand = np.repeat(np.arange(ncand), per)
         job_cand = np.ascontiguousarray(job_cand, dtype=np.int32)
-        # candidate vectors -> [mean, white_noise, amp, log_M...] through a scratch copy of this GP
+        # candidate vectors -> [mean, white_noise, amp, (log_alpha,) log_M...] through a scratch copy of this GP
         probe = self.__copy__()
-        params = np.empty((ncand, 3 + d))
+        nx = 1 if self.kernel.kernel_id == RQ_KERNEL_ID else 0
+        params = np.empty((ncand, 3 + nx + d))
         for c, v in enumerate(cands):
             probe.set_parameter_vector(v)
             kid, amp, log_M = probe.kernel.spec()
             params[c, 0], params[c, 1], params[c, 2] = probe.mean_value, probe.white_noise_value, amp
-            params[c, 3:] = log_M
+            if nx:
+                params[c, 3] = probe.kernel.log_alpha
+            params[c, 3 + nx:] = log_M
         ntr = np.array([len(f[0]) for f in folds], dtype=np.int32)
         nva = np.array([len(f[1]) for f in folds], dtype=np.int32)
         ld_tr, ld_va = int(ntr.max()), max(int(nva.max()), 1)
@@ -578,6 +580,25 @@ class GP:
         return [ph[b, :nva[b]] for b in range(njobs)], loglik, status
 
 
+RQ_KERNEL_ID = 3       # AB_KERNEL_RATQUAD: the kernel with a parameter of its own
+
+
+def _log_alpha(kernel):
+    return float(kernel.log_alpha) if kernel.kernel_id == RQ_KERNEL_ID else None
+
+
+def _set_kernel(hd, kernel, mean, white_noise, yerr2):
+    """Push ``kernel``'s hyper-parameters to the handle (ab_gp_set_kernel, or ab_gp_set_kernel_rq for
+    the rational quadratic kernel)."""
+    kid, amp, log_M = kernel.spec()
+    lm = log_M.ctypes.data_as(_lib.c_double_p)
+    if kid == RQ_KERNEL_ID:
+        _lib.check(hd.lib.ab_gp_set_kernel_rq(hd.h, amp, float(kernel.log_alpha), lm, mean, white_noise, yerr2),
+                   "ab_gp_set_kernel_rq")
+    else:
+        _lib.check(hd.lib.ab_gp_set_kernel(hd.h, kid, amp, lm, mean, white_noise, yerr2), "ab_gp_set_kernel")
+
+
 _SCRATCH_HANDLES = {}
 
 
@@ -600,8 +621,7 @@ def _kernel_value(kernel, x1, x2=None, diag=False):
     a = torch.from_numpy(np.ascontiguousarray(x1)).to(dev)
     b = torch.from_numpy(np.ascontiguousarray(x2)).to(dev)
     _lib.check(hd.lib.ab_gp_set_inputs(hd.h, _lib.ptr(a), a.shape[0], a.shape[1]), "ab_gp_set_inputs")
-    _lib.check(hd.lib.ab_gp_set_kernel(hd.h, kid, amp, log_M.ctypes.data_as(_lib.c_double_p), 0.0, -50.0, 0.0),
-               "ab_gp_set_kernel")
+    _set_kernel(hd, kernel, 0.0, -50.0, 0.0)
     out = torch.empty((a.shape[0], b.shape[0]), dtype=torch.float64, device=dev)
     _lib.check(hd.lib.ab_gp_cross_cov(hd.h, _lib.ptr(a), a.shape[0], _lib.ptr(b), b.shape[0], _lib.ptr(out)),
                "ab_gp_cross_cov")

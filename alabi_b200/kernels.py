@@ -1,4 +1,4 @@
-"""george.kernels look-alikes for the three kernels of the surrogate hot path.
+"""george.kernels look-alikes for the four kernels of the surrogate hot path.
 
 Mirrors the constructor and parameter protocol alabi uses
 (``kernels.ExpSquaredKernel(metric=vec, metric_bounds=[...], ndim=d)`` at
@@ -10,7 +10,8 @@ arithmetic happens in the CUDA library (K1 / cross-covariance kernels).
 """
 import numpy as np
 
-__all__ = ["ExpSquaredKernel", "Matern32Kernel", "Matern52Kernel", "ConstantKernel", "Product"]
+__all__ = ["ExpSquaredKernel", "Matern32Kernel", "Matern52Kernel", "RationalQuadraticKernel", "ConstantKernel",
+           "Product"]
 
 
 class Kernel:
@@ -131,6 +132,36 @@ class Matern52Kernel(_Stationary):
     kernel_id = 2
 
 
+class RationalQuadraticKernel(_Stationary):
+    """k(r^2) = (1 + r^2 / (2 alpha))^(-alpha),  alpha = exp(log_alpha).
+
+    The kernel's own parameter comes before the metric, as in george:
+    names ``("log_alpha", "metric:log_M_0_0", ...)``, vector ``[log_alpha, log_M...]``.
+    ``spec()`` keeps the (kernel_id, amp, log_M) form of the other kernels; the device
+    reads ``log_alpha`` separately (``ab_gp_set_kernel_rq``)."""
+    kernel_id = 3
+
+    def __init__(self, log_alpha, metric, metric_bounds=None, ndim=1, axes=None, lower=True, block=None, bounds=None):
+        super().__init__(metric=metric, metric_bounds=metric_bounds, ndim=ndim, axes=axes, lower=lower, block=block)
+        self.log_alpha = float(log_alpha)
+
+    def get_parameter_names(self, include_frozen=False):
+        return ("log_alpha",) + super().get_parameter_names()
+
+    def get_parameter_vector(self, include_frozen=False):
+        return np.concatenate([[self.log_alpha], self.log_M])
+
+    def set_parameter_vector(self, v, include_frozen=False):
+        v = np.atleast_1d(np.asarray(v, dtype=np.float64))
+        if len(v) != 1 + len(self.log_M):
+            raise ValueError("dimension mismatch")
+        self.log_alpha = float(v[0])
+        self.log_M = v[1:].copy()
+
+    def get_parameter_bounds(self, include_frozen=False):
+        return [(None, None)] + super().get_parameter_bounds()
+
+
 class Product(Kernel):
     """ConstantKernel * stationary kernel (the only product alabi builds)."""
 
@@ -138,13 +169,19 @@ class Product(Kernel):
         if isinstance(k2, ConstantKernel) and not isinstance(k1, ConstantKernel):
             k1, k2 = k2, k1
         if not isinstance(k1, ConstantKernel) or not isinstance(k2, _Stationary):
-            raise NotImplementedError("only ConstantKernel * {ExpSquared, Matern32, Matern52}Kernel is supported")
+            raise NotImplementedError("only ConstantKernel * {ExpSquared, Matern32, Matern52, RationalQuadratic}Kernel "
+                                      "is supported")
         self.k1, self.k2 = k1, k2
         self.ndim = k2.ndim
 
     @property
     def kernel_id(self):
         return self.k2.kernel_id
+
+    @property
+    def log_alpha(self):
+        """log_alpha of a RationalQuadraticKernel factor (AttributeError for the other kernels)."""
+        return self.k2.log_alpha
 
     def get_parameter_names(self, include_frozen=False):
         return tuple("k1:" + n for n in self.k1.get_parameter_names()) + \

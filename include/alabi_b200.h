@@ -37,6 +37,7 @@ extern "C" {
 #define AB_KERNEL_EXPSQUARED 0
 #define AB_KERNEL_MATERN32 1
 #define AB_KERNEL_MATERN52 2
+#define AB_KERNEL_RATQUAD 3      /* george RationalQuadraticKernel: set with ab_gp_set_kernel_rq */
 
 /* utility ids: alabi/utility.py:729 (bape), :629 (agp), :853 (jones) */
 #define AB_UTILITY_BAPE 0
@@ -105,6 +106,13 @@ int ab_gp_set_inputs(ab_gp* h, const double* d_X, int64_t n, int d);
 int ab_gp_set_kernel(ab_gp* h, int kernel_id, double amp, const double* h_log_M, double mean,
                      double white_noise, double yerr2);
 
+/* ab_gp_set_kernel for george's RationalQuadraticKernel (AB_KERNEL_RATQUAD, the kernel with a
+ * parameter of its own): k(r^2) = (1 + r^2 / (2 alpha))^(-alpha), alpha = exp(log_alpha),
+ * r^2 = sum_k dx_k^2 / M_k.  Returns -1 when exp(log_alpha) is not finite and positive.
+ * ab_gp_set_kernel rejects kernel id 3: this is the only way to select it. */
+int ab_gp_set_kernel_rq(ab_gp* h, double amp, double log_alpha, const double* h_log_M, double mean,
+                        double white_noise, double yerr2);
+
 /* K1: kernel.get_value(x) [+ diagonal]: full symmetric n x n matrix into d_K
  * (ld = n).  with_diag != 0 adds yerr2 + exp(white_noise) like GP.compute. */
 int ab_gp_build_cov(ab_gp* h, double* d_K, int with_diag);
@@ -122,7 +130,8 @@ int ab_gp_set_targets(ab_gp* h, const double* d_y);
 /* gp.log_likelihood(y): -1/2 r^T K^-1 r - 1/2 logdet - n/2 ln 2pi.  alabi/core.py:1248 */
 int ab_gp_log_likelihood(ab_gp* h, const double* d_y, double* h_out);
 /* gp.grad_log_likelihood(y): h_out[0..d+2] = d/d[mean, white_noise, log_constant,
- * log_M_0..]; the caller drops frozen entries.  d_y == NULL reuses the alpha of
+ * log_M_0..]; for AB_KERNEL_RATQUAD h_out[0..d+3] = d/d[mean, white_noise, log_constant,
+ * log_alpha, log_M_0..] (george's order); the caller drops frozen entries.  d_y == NULL reuses the alpha of
  * the preceding ab_gp_set_targets / ab_gp_log_likelihood.  alabi/core.py:1261 */
 int ab_gp_grad_log_likelihood(ab_gp* h, const double* d_y, double* h_out);
 
@@ -307,7 +316,8 @@ int ab_peer_free(int device, void* d_ptr);
  * goes to h_loglik[b], the predictive mean at the rows d_val_idx[b][0 .. h_nval[b]) to
  * d_pred[b][...] (leading dimensions ld_train / ld_val), and h_status[b] is 0 or the 1-based index
  * of the first non-positive pivot (the reference scores such a fold as failed).  h_params holds,
- * per candidate, 3 + d doubles: mean, white_noise (ln variance), amp = exp(log_constant), log_M[d].
+ * per candidate, 3 + d doubles: mean, white_noise (ln variance), amp = exp(log_constant), log_M[d];
+ * for kernel_id AB_KERNEL_RATQUAD 4 + d doubles: mean, white_noise, amp, log_alpha, log_M[d].
  * All jobs of a call are factorised by ONE batched dataflow-Cholesky launch per workspace chunk:
  * d_work / work_bytes is caller-owned device scratch (ab_gp_cv_workspace_bytes gives the size that
  * takes all jobs in one launch; anything from one job's worth upwards works with more launches).
