@@ -80,6 +80,9 @@ SIGNATURES = {
     "ab_gp_log_likelihood": (ctypes.c_int, [_P, _P, c_double_p]),
     "ab_gp_grad_log_likelihood": (ctypes.c_int, [_P, _P, c_double_p]),
     "ab_gp_predict": (ctypes.c_int, [_P, _P, ctypes.c_int64, _P, _P]),
+    "ab_gp_predict_cov": (ctypes.c_int, [_P, _P, ctypes.c_int64, _P, _P, ctypes.c_int64]),
+    "ab_mvn_sample": (ctypes.c_int, [_P, _P, ctypes.c_int64, ctypes.c_int64, _P, ctypes.c_double, ctypes.c_int64,
+                                     ctypes.c_uint64, _P, ctypes.POINTER(ctypes.c_int)]),
     "ab_gp_predict_host": (ctypes.c_int, [_P, _P, ctypes.c_int64, _P, _P]),
     "ab_gp_utility_argmin": (ctypes.c_int, [_P, ctypes.c_int, _P, ctypes.c_int64, c_double_p, ctypes.c_double,
                                             ctypes.c_double, _P, c_int64_p, c_double_p]),

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(ROOT, "build", "obj")
 LIB = os.path.join(HERE, "libalabi_b200.so")
-SOURCES = ["api.cu", "cov.cu", "chol.cu", "chol_dataflow.cu", "trsv_dataflow.cu", "append.cu", "grad.cu", "predict.cu", "ensemble.cu", "ensemble_k0.cu", "ensemble_k1.cu", "ensemble_k2.cu", "ensemble_k3.cu", "nested.cu", "cv_batch.cu", "nccl_helpers.cu", "peak.cu"]
+SOURCES = ["api.cu", "cov.cu", "chol.cu", "chol_dataflow.cu", "trsv_dataflow.cu", "append.cu", "grad.cu", "predict.cu", "ensemble.cu", "ensemble_k0.cu", "ensemble_k1.cu", "ensemble_k2.cu", "ensemble_k3.cu", "nested.cu", "cv_batch.cu", "mvn.cu", "nccl_helpers.cu", "peak.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-I", os.path.join(ROOT, "include"), "-I", CSRC]

@@ -389,6 +389,17 @@ int ab_gp_predict(ab_gp* h, const double* d_Xq, int64_t m, double* d_mu, double*
     return ab_launch_predict(h, d_Xq, m, d_mu, d_var);
 }
 
+int ab_gp_predict_cov(ab_gp* h, const double* d_Xq, int64_t m, double* d_mu, double* d_cov, int64_t ldc) {
+    AB_REQUIRE(h && d_Xq && d_mu && d_cov, -1, "ab_gp_predict_cov: null argument");
+    AB_REQUIRE(m >= 0 && ldc >= m && ldc >= 1, -1, "ab_gp_predict_cov: need m >= 0 and ldc >= max(m, 1) (m=%lld ldc=%lld)",
+               (long long)m, (long long)ldc);
+    AB_REQUIRE(h->have_alpha, -2, "ab_gp_predict_cov: targets not set (call ab_gp_factor + ab_gp_set_targets)");
+    AB_CUDA(cudaSetDevice(h->device));
+    int rc = ensure_linv(h);
+    if (rc) return rc;
+    return ab_launch_predict_cov(h, d_Xq, m, d_mu, d_cov, ldc);
+}
+
 int ab_gp_predict_grad(ab_gp* h, const double* d_Xq, int64_t m, double* d_mu, double* d_var, double* d_dmu,
                        double* d_dvar) {
     AB_REQUIRE(h && d_Xq && d_mu && d_var && d_dmu && d_dvar, -1, "ab_gp_predict_grad: null argument");

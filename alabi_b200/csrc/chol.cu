@@ -366,8 +366,10 @@ int ab_launch_build_kinv(ab_gp* h) {
     return 0;
 }
 
-int ab_launch_mirror_lower(ab_gp* h, double* A, int64_t ld) {
-    int64_t n = h->npad;
+int ab_launch_mirror_lower(ab_gp* h, double* A, int64_t ld) { return ab_launch_mirror_lower_n(h, A, ld, h->npad); }
+
+// strict lower triangle of the leading n x n block of A -> upper
+int ab_launch_mirror_lower_n(ab_gp* h, double* A, int64_t ld, int64_t n) {
     unsigned nt = (unsigned)((n + 31) / 32);
     mirror_lower_kernel<<<dim3(nt, nt), dim3(32, 8), 0, h->stream>>>(A, ld, n);
     mirror_diag_tiles_kernel<<<nt, 256, 0, h->stream>>>(A, ld, n);

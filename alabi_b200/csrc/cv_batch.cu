@@ -216,17 +216,6 @@ size_t job_bytes(int npad, int d, int ld_val) {
     return (b + 255) / 256 * 256;
 }
 
-// carve `bytes` (256-aligned) out of the caller's workspace
-struct Carver {
-    char* p; size_t left;
-    void* take(size_t bytes) {
-        bytes = (bytes + 255) / 256 * 256;
-        if (bytes > left) return nullptr;
-        void* r = p; p += bytes; left -= bytes;
-        return r;
-    }
-};
-
 }  // namespace
 
 extern "C" int ab_gp_cv_batch(ab_gp* h, const double* d_X, const double* d_y, int64_t n, int d, int kernel_id, int ncand,

@@ -63,6 +63,16 @@ struct ab_gp {
 };
 
 int ab_ensure_scratch(ab_gp* h, size_t bytes);
+// carve `bytes` (256-aligned) out of a workspace; nullptr when it does not fit
+struct Carver {
+    char* p; size_t left;
+    void* take(size_t bytes) {
+        bytes = (bytes + 255) / 256 * 256;
+        if (bytes > left) return nullptr;
+        void* r = p; p += bytes; left -= bytes;
+        return r;
+    }
+};
 void ab_count_launches(long long n);
 // RAII-less scope helpers: record an event before / after a kernel family
 void ab_prof_begin(ab_gp* h, int family);
@@ -84,11 +94,15 @@ int ab_launch_solve_alpha(ab_gp* h, const double* y);
 int ab_launch_build_linv(ab_gp* h);
 int ab_launch_build_kinv(ab_gp* h);
 int ab_launch_mirror_lower(ab_gp* h, double* A, int64_t ld);
+int ab_launch_mirror_lower_n(ab_gp* h, double* A, int64_t ld, int64_t n);
 // grad.cu
 int ab_launch_grad(ab_gp* h, double* h_out);
 // predict.cu
 int ab_launch_predict(ab_gp* h, const double* Xq, int64_t m, double* mu, double* var);
 int64_t ab_predict_panel_queries(ab_gp* h);
+int ab_launch_predict_cov(ab_gp* h, const double* Xq, int64_t m, double* mu, double* C, int64_t ldc);
+int ab_launch_tri_gemm_lower(ab_gp* h, const double* L, int64_t ld, int T, const double* B, int64_t ldb, int ntiles,
+                             double* C);
 int ab_launch_predict_grad(ab_gp* h, const double* Xq, int64_t m, double* mu, double* var, double* dmu, double* dvar);
 int ab_launch_utility(ab_gp* h, int kind, const double* Xq, const double* mu, const double* var, int64_t m,
                       const double* h_bounds, double y_best, double zeta, double* util,

@@ -1065,3 +1065,149 @@ int ab_launch_utility(ab_gp* h, int kind, const double* Xq, const double* mu, co
     *h_argmin = (int64_t) * reinterpret_cast<long long*>(h->h_pinned + 1);
     return 0;
 }
+
+// ---------------------------------------------------------------------------
+// Full predictive covariance (george GP.predict(y, t, return_cov=True)):
+//   Sigma = K(t, t) - W^T W,  W = L^-1 P,  P[j][q] = amp k(x_j, t_q)
+// Stages: panel + mean (predict_mean_kernel, as ab_launch_predict), W (tri_gemm_kernel<false>),
+// the prior block K(t, t) straight into the caller's matrix (cov_kernel), the SYRK below over the
+// lower 128 x 128 tile pairs, the diagonal from W in the canonical order of predict_var_kernel
+// (so diag(Sigma) has the bits of predict(return_var=True)), and a mirror of the lower triangle.
+// Every entry (a, b) depends on queries a and b only, through a k order fixed by N.
+// ---------------------------------------------------------------------------
+namespace {
+
+// C[a-tile][b-tile] -= sum_k W[k][a] W[k][b] for the tile pair (a, b), b <= a, of blockIdx.x.
+// nk: BK chunks of the k range (fixed by N: rows of W past the training points are zero).
+// Masked element stores: the same expression for every element, ragged tile or not.
+__global__ void __launch_bounds__(abg::THREADS, 1)
+syrk_lower_kernel(const double* __restrict__ W, int64_t ldw, int nk, double* __restrict__ C, int64_t ldc,
+                  int64_t m) {
+    extern __shared__ __align__(16) double smem[];
+    int a, b;
+    abg::tri_decode(blockIdx.x, a, b);
+    abg::Acc acc;
+    acc.zero();
+    abg::mainloop<false, false>(acc, W + (int64_t)a * abg::BM, ldw, W + (int64_t)b * abg::BN, ldw, nk, smem);
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const int64_t r = (int64_t)a * abg::BM + abg::acc_row(i);
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+#pragma unroll
+            for (int e = 0; e < 2; e++) {
+                const int64_t c = (int64_t)b * abg::BN + abg::acc_col(j) + e;
+                if (r < m && c < m) {
+                    double* p = C + r * ldc + c;
+                    *p = *p - acc.v[i][j][e];
+                }
+            }
+    }
+}
+
+// sigma^2 of the 128 queries of blockIdx.x from W (npad x ldw): the W tiles are read back in the
+// accumulator layout store_tile wrote them from (alpha = 1: the accumulator's bits), then squared
+// and summed exactly like predict_var_kernel / var_combine_kernel
+__global__ void __launch_bounds__(abg::THREADS)
+var_from_w_kernel(const double* __restrict__ W, int64_t ldw, int T, int64_t m, double amp, double* __restrict__ var) {
+    __shared__ double red[256];
+    double tot[4][2];
+#pragma unroll
+    for (int j = 0; j < 4; j++) tot[j][0] = tot[j][1] = 0.0;
+    const double* Wq = W + (int64_t)blockIdx.x * abg::BN;
+    for (int i = 0; i < T; i++) {
+        abg::Acc acc;
+#pragma unroll
+        for (int a = 0; a < 8; a++) {
+            const double* row = Wq + ((int64_t)i * NB + abg::acc_row(a)) * ldw;
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const double2 v = *reinterpret_cast<const double2*>(row + abg::acc_col(j));
+                acc.v[a][j][0] = v.x;
+                acc.v[a][j][1] = v.y;
+            }
+        }
+        double blk[4][2];
+        tile_thread_sq(acc, blk);
+#pragma unroll
+        for (int j = 0; j < 4; j++) { tot[j][0] += blk[j][0]; tot[j][1] += blk[j][1]; }
+    }
+    tile_finish_var(tot, red, (int64_t)blockIdx.x * abg::BN + threadIdx.x, m, amp, var);
+}
+
+__global__ void set_diag_kernel(const double* __restrict__ v, int64_t m, double* __restrict__ C, int64_t ldc) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q < m) C[q * ldc + q] = v[q];
+}
+
+}  // namespace
+
+// C = op-free lower triangular product L B (tri_gemm_kernel<false>): L is T x T blocks of 128 with
+// leading dimension ld, lower, with the upper part of its diagonal blocks zero (L^-1, or a Cholesky
+// factor of the dataflow kernel); B and C are (T 128) x ldb, the first ntiles 128-column tiles are
+// computed.  Every column of C depends on the same column of B only.
+int ab_launch_tri_gemm_lower(ab_gp* h, const double* L, int64_t ld, int T, const double* B, int64_t ldb, int ntiles,
+                             double* C) {
+    AB_CUDA(cudaFuncSetAttribute(tri_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
+    tri_gemm_kernel<false><<<dim3((unsigned)ntiles, (unsigned)T), abg::THREADS, abg::SMEM_BYTES, h->stream>>>(L, ld, T, B,
+                                                                                                             ldb, C);
+    AB_CHECK_LAUNCH();
+    ab_count_launches(1);
+    return 0;
+}
+
+// mean mu (m) and covariance C (m x m, leading dimension ldc >= m) of the m queries Xq; needs L^-1.
+// Workspace: P and W (npad x ldp each, ldp = m rounded up to 256) from the handle scratch.
+int ab_launch_predict_cov(ab_gp* h, const double* Xq, int64_t m, double* mu, double* C, int64_t ldc) {
+    if (m <= 0) return 0;
+    cudaStream_t s = h->stream;
+    const int d = h->d, T = (int)(h->npad / NB);
+    const int64_t ldp = (m + QPB - 1) / QPB * QPB;
+    const int nsplit = (int)((h->npad + JCHUNK - 1) / JCHUNK);
+    const int ntq = (int)((m + abg::BN - 1) / abg::BN);
+    const size_t panel = (size_t)h->npad * ldp;
+    int rc = ab_ensure_scratch(h, (2 * panel + (size_t)nsplit * ldp + ldp + (size_t)m * d) * sizeof(double));
+    if (rc) {
+        cudaGetLastError();                    // a failed allocation is reported once, by the return code
+        return rc;
+    }
+    double* P = h->scratch;
+    double* W = P + panel;
+    double* partial = W + panel;
+    double* dv = partial + (size_t)nsplit * ldp;
+    double* XT = dv + ldp;
+    // 1. panel P and mean (the launches of ab_launch_predict's panel pass)
+    ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
+    dim3 grid((unsigned)(ldp / QPB), (unsigned)nsplit);
+    AB_DISPATCH_KIND(h->kp.kind, rc = (launch_mean<KIND, true>(h, d, grid, Xq, m, 0, mu, P, ldp, nsplit, partial, ldp)));
+    if (rc) return rc;
+    if (nsplit > 1) {
+        combine_splits_kernel<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(partial, ldp, m, nsplit, h->kp.amp, h->mean, mu, 0);
+        AB_CHECK_LAUNCH();
+    }
+    ab_prof_end(h, AB_PROF_PREDICT_PANEL);
+    ab_count_launches(nsplit > 1 ? 2 : 1);
+    // 2. W = L^-1 P
+    ab_prof_begin(h, AB_PROF_PREDICT_VAR);
+    rc = ab_launch_tri_gemm_lower(h, h->Linv, h->npad, T, P, ldp, ntq, W);
+    if (rc) return rc;
+    // 3. prior block K(t, t) into C
+    rc = ab_launch_scale_points(h, Xq, m, XT, m);
+    if (rc) return rc;
+    rc = ab_launch_cross_cov(h, XT, m, m, XT, m, m, C, ldc);
+    if (rc) return rc;
+    // 4. C -= W^T W on the lower tile pairs; k over the training rows rounded up to BK
+    const int nk = (int)((h->n + abg::BK - 1) / abg::BK);
+    AB_CUDA(cudaFuncSetAttribute(syrk_lower_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
+    syrk_lower_kernel<<<(unsigned)(ntq * (ntq + 1) / 2), abg::THREADS, abg::SMEM_BYTES, s>>>(W, ldp, nk, C, ldc, m);
+    AB_CHECK_LAUNCH();
+    // 5. the diagonal: sigma^2 with the bits of the variance path
+    var_from_w_kernel<<<(unsigned)ntq, abg::THREADS, 0, s>>>(W, ldp, T, m, h->kp.amp, dv);
+    set_diag_kernel<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(dv, m, C, ldc);
+    AB_CHECK_LAUNCH();
+    ab_count_launches(5);
+    // 6. exact symmetry
+    rc = ab_launch_mirror_lower_n(h, C, ldc, m);
+    ab_prof_end(h, AB_PROF_PREDICT_VAR);
+    return rc;
+}

@@ -396,22 +396,30 @@ class GP:
         return -self.grad_log_likelihood(y, quiet=quiet)
 
     def predict(self, y, t, return_cov=True, return_var=False, cache=True, kernel=None):
-        """Predictive mean (and variance) at ``t`` (K3).  ``t`` may be a NumPy
-        array (host buffers, copies included) or a CUDA torch tensor (device
-        buffers in, torch tensors out).  The full predictive covariance is not
-        on alabi's path and is not implemented."""
+        """Predictive mean at ``t`` and, as in george, the full predictive covariance
+        (``return_cov=True``, the default: ``(mu, cov)``, cov = K(t, t) - K(t, x) K^-1 K(x, t)
+        without white noise) or the variance (``return_var=True``, which takes precedence:
+        ``(mu, var)``).  ``t`` may be a NumPy array (host buffers, copies included) or a CUDA
+        torch tensor (device buffers in, torch tensors out).  ``mu`` has the same bits in every
+        mode, ``diag(cov)`` the bits of ``var``."""
         self.recompute()
         self._set_targets(y)
         hd = self._hd
         want_var = bool(return_var)
-        if not want_var and return_cov:
-            raise NotImplementedError("return_cov=True: the full predictive covariance is outside the alabi hot path; "
-                                      "pass return_cov=False or return_var=True")
+        want_cov = bool(return_cov) and not want_var
         try:
             import torch
             is_dev = isinstance(t, torch.Tensor) and t.is_cuda
         except ImportError:
             is_dev = False
+        if want_cov:
+            torch = _torch()
+            tq = (t.reshape(-1, self.kernel.ndim).to(dtype=torch.float64).contiguous() if is_dev
+                  else self._dev(self.parse_samples(t)))
+            mu, cov = self._predict_cov_dev(tq)
+            if is_dev:
+                return mu, cov
+            return mu.cpu().numpy(), cov.cpu().numpy()
         if is_dev:
             tq = t.reshape(-1, self.kernel.ndim).to(dtype=torch.float64).contiguous()
             m = tq.shape[0]
@@ -429,6 +437,73 @@ class GP:
         var = np.empty(m, dtype=np.float64) if want_var else None
         _lib.check(hd.lib.ab_gp_predict_host(hd.h, _lib.ptr(xs), m, _lib.ptr(mu), _lib.ptr(var)), "ab_gp_predict_host")
         return (mu, var) if want_var else mu
+
+    def _predict_cov_dev(self, tq):
+        """(mu, cov) as device tensors for the device query block ``tq`` (m x d); targets set."""
+        torch = _torch()
+        hd = self._hd
+        m = tq.shape[0]
+        mu = torch.empty(m, dtype=torch.float64, device=tq.device)
+        cov = torch.empty((m, m), dtype=torch.float64, device=tq.device)
+        if m > 0:
+            _check_alloc(hd.lib.ab_gp_predict_cov(hd.h, _lib.ptr(tq), m, _lib.ptr(mu), _lib.ptr(cov), m),
+                         "ab_gp_predict_cov", 16 * hd.lib.ab_gp_padded_size(hd.h) * ((m + 255) // 256 * 256))
+        return mu, cov
+
+    # -- draws (george GP.sample_conditional / GP.sample) ----------------------------------------------
+    def sample_conditional(self, y, t, size=1, seed=None, jitter=None):
+        """Draws from the GP posterior at ``t`` (george's ``sample_conditional``): returns
+        ``(size, M)``, or ``(M,)`` when ``size == 1``.  The covariance stays on the device
+        (``ab_gp_predict_cov`` then ``ab_mvn_sample``).  ``seed=None`` takes a seed from NumPy's
+        global stream, so ``np.random.seed`` makes runs reproducible; with the same seed the
+        first k draws of ``size=n`` equal the draws of ``size=k``.  ``jitter``: see ``sample``."""
+        torch = _torch()
+        self.recompute()
+        self._set_targets(y)
+        is_dev = isinstance(t, torch.Tensor) and t.is_cuda
+        tq = (t.reshape(-1, self.kernel.ndim).to(dtype=torch.float64).contiguous() if is_dev
+              else self._dev(self.parse_samples(t)))
+        mu, cov = self._predict_cov_dev(tq)
+        out = _mvn_draw(self._hd, cov, mu, size, seed, jitter, self.kernel.spec()[1])
+        return _draw_result(out, size, is_dev)
+
+    def sample(self, t=None, size=1, seed=None, jitter=None):
+        """Draws from the GP prior (george's ``sample``): at ``t``, N(mean, amp k(t, t));
+        with ``t=None`` at the training inputs from the full covariance K of ``compute``, white
+        noise and yerr^2 included (one more factorisation of the N x N matrix).  Returns
+        ``(size, M)``, or ``(M,)`` when ``size == 1``.
+
+        george draws through NumPy's SVD, which accepts a semi-definite covariance; a Cholesky
+        does not.  ``jitter=None`` therefore tries delta = 0, 1e-12, 1e-10, 1e-8 and 1e-6 times the
+        kernel amplitude on the diagonal, warns (RuntimeWarning) when delta > 0 was needed and
+        raises ``LinAlgError`` after the last step; a float uses exactly that jitter."""
+        torch = _torch()
+        amp = self.kernel.spec()[1]
+        if t is None:
+            if self._x is None:
+                raise RuntimeError("You need to compute the model first")
+            self.recompute()
+            hd = self._hd
+            n = self._x.shape[0]
+            dev = f"cuda:{hd.device}"
+            cov = torch.empty((n, n), dtype=torch.float64, device=dev)
+            _lib.check(hd.lib.ab_gp_build_cov(hd.h, _lib.ptr(cov), 1), "ab_gp_build_cov")
+            mean = torch.full((n,), float(self.mean_value), dtype=torch.float64, device=dev)
+            return _draw_result(_mvn_draw(hd, cov, mean, size, seed, jitter, amp), size, False)
+        is_dev = isinstance(t, torch.Tensor) and t.is_cuda
+        if self._x is not None:
+            self._push()
+            hd = self._hd
+        else:
+            hd = _scratch_handle(self.kernel, self.parse_samples(t)[:1])
+        tq = (t.reshape(-1, self.kernel.ndim).to(dtype=torch.float64).contiguous() if is_dev
+              else torch.from_numpy(self.parse_samples(t)).to(f"cuda:{hd.device}"))
+        m = tq.shape[0]
+        cov = torch.empty((m, m), dtype=torch.float64, device=tq.device)
+        if m > 0:
+            _lib.check(hd.lib.ab_gp_cross_cov(hd.h, _lib.ptr(tq), m, _lib.ptr(tq), m, _lib.ptr(cov)), "ab_gp_cross_cov")
+        mean = torch.full((m,), float(self.mean_value), dtype=torch.float64, device=tq.device)
+        return _draw_result(_mvn_draw(hd, cov, mean, size, seed, jitter, amp), size, is_dev)
 
     def predict_grad(self, y, t):
         """(mu, var, d mu / dx, d var / dx) at the query points ``t`` (M x d); the
@@ -599,7 +674,67 @@ def _set_kernel(hd, kernel, mean, white_noise, yerr2):
         _lib.check(hd.lib.ab_gp_set_kernel(hd.h, kid, amp, lm, mean, white_noise, yerr2), "ab_gp_set_kernel")
 
 
+JITTER_LADDER = (0.0, 1e-12, 1e-10, 1e-8, 1e-6)      # times the kernel amplitude
+
+
+def _check_alloc(rc, what, nbytes):
+    """_lib.check, with a failed device allocation (cudaErrorMemoryAllocation) as MemoryError."""
+    if rc == -102:
+        raise MemoryError(f"{what}: cannot allocate about {nbytes / 1e9:.2f} GB of device workspace "
+                          f"({_lib.last_error()})")
+    return _lib.check(rc, what)
+
+
+def _mvn_draw(hd, cov, mean, size, seed, jitter, amp):
+    """``size`` draws of N(mean, cov + delta I) as a (size, m) device tensor (ab_mvn_sample),
+    delta from the jitter ladder or exactly ``jitter``."""
+    import warnings
+    torch = _torch()
+    size = int(size)
+    if size < 1:
+        raise ValueError("size must be >= 1")
+    m = cov.shape[0]
+    out = torch.empty((size, m), dtype=torch.float64, device=cov.device)
+    if m == 0:
+        return out
+    if seed is None:
+        seed = int(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64))
+    seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    ladder = [float(d) * float(amp) for d in JITTER_LADDER] if jitter is None else [float(jitter)]
+    info = ctypes.c_int(0)
+    for delta in ladder:
+        rc = _check_alloc(hd.lib.ab_mvn_sample(hd.h, _lib.ptr(cov), m, m, _lib.ptr(mean), delta, size, seed,
+                                               _lib.ptr(out), ctypes.byref(info)),
+                          "ab_mvn_sample", 8 * ((m + 127) // 128 * 128) * (2 * ((size + 127) // 128 * 128) + m))
+        if rc == 0:
+            if delta > 0.0 and jitter is None:
+                warnings.warn(f"covariance is not positive definite; drew with jitter {delta:g} on its diagonal",
+                              RuntimeWarning, stacklevel=3)
+            return out
+    raise LinAlgError(f"{info.value}-th leading minor of the covariance matrix is not positive definite "
+                      f"(jitter {ladder[-1]:g})")
+
+
+def _draw_result(out, size, is_dev):
+    r = out[0] if int(size) == 1 else out
+    return r if is_dev else r.cpu().numpy()
+
+
 _SCRATCH_HANDLES = {}
+
+
+def _scratch_handle(kernel, x):
+    """The per-device scratch handle of _kernel_value with inputs ``x`` and ``kernel`` pushed."""
+    torch = _torch()
+    cur = torch.cuda.current_device()
+    hd = _SCRATCH_HANDLES.get(cur)
+    if hd is None or hd.stream != torch.cuda.current_stream(cur):
+        hd = _SCRATCH_HANDLES[cur] = _Handle(cur)
+    a = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64)).to(f"cuda:{hd.device}")
+    _lib.check(hd.lib.ab_gp_set_inputs(hd.h, _lib.ptr(a), a.shape[0], a.shape[1]), "ab_gp_set_inputs")
+    _set_kernel(hd, kernel, 0.0, -50.0, 0.0)
+    hd.stream.synchronize()                  # `a` may be freed after this call
+    return hd
 
 
 def _kernel_value(kernel, x1, x2=None, diag=False):

@@ -48,6 +48,8 @@ extern "C" {
 #define AB_STREAM_SPLIT 0
 #define AB_STREAM_PARTNER 1
 #define AB_STREAM_MOVE 2
+/* Philox counter stream of the multivariate-normal draws of ab_mvn_sample */
+#define AB_STREAM_MVN 3
 
 typedef struct ab_gp ab_gp;
 
@@ -138,6 +140,27 @@ int ab_gp_grad_log_likelihood(ab_gp* h, const double* d_y, double* h_out);
 /* K3: gp.predict(y, t, return_var).  d_var may be NULL (mean only).
  * alabi/core.py:85,95,1441,1486,1601 */
 int ab_gp_predict(ab_gp* h, const double* d_Xq, int64_t m, double* d_mu, double* d_var);
+
+/* gp.predict(y, t, return_cov=True) (george's default call; the oracle's GP.predict): the
+ * predictive mean d_mu (m) and the full predictive covariance
+ *   d_cov = K(t, t) - K(t, X) K^-1 K(X, t)     (m x m, leading dimension ldc >= m, white noise not added)
+ * from L^-1 by FP64 DMMA products (W = L^-1 K(X, t), then K(t, t) - W^T W on the lower tiles).
+ * d_mu has the bits of ab_gp_predict's mean, diag(d_cov) the bits of its variance, d_cov is exactly
+ * symmetric, and entry (a, b) depends on queries a and b only (the same bits in any batch).
+ * Device workspace: 16 npad m bytes (m rounded up to 256); when it cannot be allocated the call
+ * returns -102 (cudaErrorMemoryAllocation) and computes nothing. */
+int ab_gp_predict_cov(ab_gp* h, const double* d_Xq, int64_t m, double* d_mu, double* d_cov, int64_t ldc);
+
+/* Draws from N(mean, cov + jitter I), george's GP.sample_conditional / GP.sample (which go through
+ * numpy.random.multivariate_normal): d_cov is m x m (leading dimension ldc >= m, lower triangle
+ * read, not modified), d_mean m values or NULL (zero mean), d_out nsamples x m (george's (size, M)
+ * layout).  cov + jitter I is factorised by the dataflow Cholesky; returns 0, or the 1-based index of
+ * the first non-positive pivot (also in *h_info; nothing is written to d_out then).  Normals:
+ * Philox4x32-10, key = seed, counter = (row, sample / 2, 0, AB_STREAM_MVN), Box-Muller; draw s
+ * depends on column s of the normals only, so the first k draws of any call are the draws of a call
+ * with nsamples = k and the same seed. */
+int ab_mvn_sample(ab_gp* h, const double* d_cov, int64_t m, int64_t ldc, const double* d_mean /* or NULL */,
+                  double jitter, int64_t nsamples, uint64_t seed, double* d_out /* nsamples x m */, int* h_info);
 
 /* gp.predict plus the gradients of mean and variance w.r.t. the query point:
  * d_dmu, d_dvar are m x d row-major.  Replaces grad_gp_mean_prediction /
