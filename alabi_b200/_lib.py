@@ -117,6 +117,7 @@ SIGNATURES = {
     "ab_peer_free": (ctypes.c_int, [ctypes.c_int, _P]),
     "ab_sizeof_nested_config": (ctypes.c_int, []),
     "ab_nested_walk": (ctypes.c_int, [_P, ctypes.POINTER(NestedConfig), _P, _P, _P, _P]),
+    "ab_nested_rslice": (ctypes.c_int, [_P, ctypes.POINTER(NestedConfig), _P, _P, _P, _P]),
     "ab_ensemble_run_host": (ctypes.c_int, [_P, ctypes.POINTER(EnsembleConfig), _P, _P, _P, _P, _P, _P, _P, ctypes.c_int]),
 }
 

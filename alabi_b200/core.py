@@ -888,20 +888,25 @@ class SurrogateModel(object):
 
     def _builtin_nested_runner(self, ns, batch_like, lp, mode, skw, rkw, save_iter):
         """Closure running one built-in nested-sampling run (see run_dynesty)."""
-        allowed_s = {"nlive", "walks", "nbatch", "rstate", "seed", "bound", "sample", "pool", "queue_size", "use_pool"}
+        allowed_s = {"nlive", "walks", "slices", "nbatch", "rstate", "seed", "bound", "sample", "pool", "queue_size",
+                     "use_pool"}
         allowed_r = {"dlogz", "dlogz_init", "maxiter", "maxcall", "wt_kwargs", "stop_kwargs", "nlive_init", "nlive_batch",
                      "maxbatch", "n_effective", "print_progress"}
         bad = (set(skw) - allowed_s) | (set(rkw) - allowed_r)
         if bad:
             raise TypeError(f"run_dynesty (built-in sampler): unsupported keyword(s) {sorted(bad)}; sampler_kwargs "
                             f"{sorted(allowed_s)}, run_kwargs {sorted(allowed_r)}")
-        if str(skw.get("sample", "auto")).lower() not in ("auto", "rwalk"):
+        sample = str(skw.get("sample", "auto")).lower()
+        if sample not in ("auto", "rwalk", "rslice"):
             raise NotImplementedError(f"sample={skw['sample']!r}: the built-in sampler proposes by constrained random "
-                                      "walks (dynesty's 'rwalk')")
+                                      "walks (dynesty's 'rwalk', also for 'auto') or by random-direction slice "
+                                      "sampling ('rslice')")
+        sample = "rslice" if sample == "rslice" else "rwalk"
         if str(skw.get("bound", "multi")).lower() not in ("multi", "single", "none"):
             raise NotImplementedError(f"bound={skw['bound']!r} is not available in the built-in sampler")
         nlive = int(skw.get("nlive", 50 * self.ndim))
         walks = int(skw.get("walks", 25))
+        slices = int(skw.get("slices", 5))
         seed = skw.get("seed", skw.get("rstate"))
         if seed is not None and not isinstance(seed, (int, np.integer)):
             seed = int(np.random.default_rng(seed).integers(2 ** 62))
@@ -917,7 +922,7 @@ class SurrogateModel(object):
             else:
                 walker = ns.HostWalker(batch_like, self.prior_transform, self.ndim, rng=np.random.default_rng(rseed))
             ds = ns.BatchedNestedSampler(walker, self.ndim, nlive=nlive, walks=walks, nbatch=skw.get("nbatch"),
-                                         rstate=None if rseed is None else rseed + 1)
+                                         rstate=None if rseed is None else rseed + 1, sample=sample, slices=slices)
             if save_iter is not None:
                 path = os.path.join(self.savedir, f"dynesty_sampler_{self.like_fn_name}_run{run_number}.pkl")
                 ds.checkpoint, ds.checkpoint_every = ns.save_checkpoint(path), int(save_iter)
@@ -983,10 +988,11 @@ class SurrogateModel(object):
           :class:`alabi_b200.nested.BatchedNestedSampler` with the same two modes and result fields
           (``samples, logwt, logz, logzerr, niter``).  With the surrogate likelihood and one of the
           reference's prior transforms (``ut.prior_transform_uniform`` / ``_normal``, or None) every
-          batch of constrained random walks is one kernel launch (``ab_nested_walk``); a custom
-          Python ``like_fn`` / ``prior_transform`` runs the same algorithm with host-side walks.
-          ``sampler_kwargs``: nlive (50 ndim), walks (25), nbatch, rstate / seed, bound, sample
-          ("auto" / "rwalk"); ``run_kwargs``: dlogz, dlogz_init (0.5), maxiter (5e4), maxcall,
+          batch of constrained random walks is one kernel launch (``ab_nested_walk``, or
+          ``ab_nested_rslice`` for random-direction slice sampling); a custom Python ``like_fn`` /
+          ``prior_transform`` runs the same algorithms with host-side chains.
+          ``sampler_kwargs``: nlive (50 ndim), walks (25), slices (5), nbatch, rstate / seed, bound,
+          sample ("auto" = "rwalk", or "rslice"); ``run_kwargs``: dlogz, dlogz_init (0.5), maxiter (5e4), maxcall,
           wt_kwargs {"pfrac": 1.0}, nlive_init, nlive_batch, maxbatch, n_effective, print_progress;
           anything else raises.  ``save_iter`` pickles the dead points every that many iterations;
           ``multi_proc`` has no meaning here (the batch is the parallelism)."""

@@ -12,12 +12,14 @@ time through ``pool.map``).  This module provides
   the likelihood range that carries the posterior mass (importance = ``pfrac`` posterior +
   (1 - ``pfrac``) evidence, the reference passes ``pfrac = 1``), merged by birth / death likelihood
   until the requested effective sample size is reached.  Replacement points come from constrained
-  random walks (dynesty's ``sample="rwalk"``), a whole batch of chains at a time:
+  random walks (dynesty's ``sample="rwalk"``) or random-direction slice sampling
+  (``sample="rslice"``), a whole batch of chains at a time:
 * :class:`DeviceWalker` — surrogate likelihood with one of the two prior transforms the reference
-  ships: the whole batch of ``walks``-step chains is ONE kernel launch (``ab_nested_walk``), no
-  host round trip per step;
+  ships: the whole batch of ``walks``-step chains (or ``slices``-slice chains) is ONE kernel launch
+  (``ab_nested_walk`` / ``ab_nested_rslice``), no host round trip per step;
 * :class:`HostWalker` — any Python likelihood / prior transform (e.g. the true likelihood): chains
-  advance in lock-step on the host, one batched likelihood call per walk step;
+  advance in lock-step on the host, one batched likelihood call per walk step (per slice-sampling
+  round);
 * :class:`BatchPool` — ``pool``-shaped object for real dynesty: ``map`` turns the ``queue_size``
   points of one dynesty iteration into one batched surrogate predict (K3).
 
@@ -32,7 +34,12 @@ import warnings
 import numpy as np
 
 __all__ = ["BatchedNestedSampler", "DeviceWalker", "HostWalker", "BatchPool", "NestedResults", "resample_equal",
-           "compute_weights"]
+           "compute_weights", "rslice_scale"]
+
+# Step-out moves and failed shrink draws allowed per slice (the caps of ab_nested_rslice): a chain
+# that would need more stops at the end point of its last completed slice.
+RSLICE_MAX_EXPAND = 1024
+RSLICE_MAX_CONTRACT = 256
 
 
 class NestedResults(dict):
@@ -148,6 +155,88 @@ class HostWalker:
                 nacc += int(ok_in.sum())
         return u, theta, logl, nacc / float(max(k * int(walks), 1))
 
+    def _rslice_chain(self, c, u, theta, logl, counts, lmin, scale, chol, slices):
+        """Slice-sampling state machine of chain ``c`` (the algorithm of ``ab_nested_rslice``, with
+        draws from ``self.rng``): yields each in-cube proposal, is sent back its (theta, logl)."""
+        d = self.ndim
+        v = None
+
+        def F(x):
+            # point u + x v with its image and likelihood; outside the unit cube: -inf, no call
+            p = u[c] + x * v
+            if np.all((p > 0.0) & (p < 1.0)):
+                th, y = yield p
+                return p, th, y
+            return p, None, -np.inf
+        for _ in range(int(slices)):
+            z = self.rng.standard_normal(d)
+            v = (chol @ z) * (scale / np.sqrt(z @ z))
+            r0 = self.rng.random()
+            xl, xr = -r0, 1.0 - r0
+            nexp = 0
+            for left in (True, False):
+                while True:
+                    _, _, y = yield from F(xl if left else xr)
+                    if not y > lmin:
+                        break
+                    if nexp == RSLICE_MAX_EXPAND:
+                        return
+                    nexp += 1
+                    counts[c, 1] += 1
+                    if left:
+                        xl -= 1.0
+                    else:
+                        xr += 1.0
+            ncon = 0
+            while True:
+                x = xl + self.rng.random() * (xr - xl)
+                p, th, y = yield from F(x)
+                if y > lmin:
+                    u[c], theta[c], logl[c] = p, th, y
+                    counts[c, 0] += 1
+                    break
+                ncon += 1
+                counts[c, 2] += 1
+                if x < 0.0:
+                    xl = x
+                elif x > 0.0:
+                    xr = x
+                if ncon == RSLICE_MAX_CONTRACT:
+                    return
+
+    def rslice(self, u0, theta0, logl0, lmin, scale, chol, slices):
+        """``slices`` random-direction slices per chain (dynesty's ``sample="rslice"``).  All
+        unfinished chains advance in lock step, one batched likelihood call per round.  Returns
+        (u, theta, logl, counts) with counts (k, 4): slices completed, nexpand, ncontract, evaluations."""
+        u, theta, logl = u0.copy(), theta0.copy(), logl0.copy()
+        k = len(u)
+        counts = np.zeros((k, 4), dtype=np.int64)
+        chains = [self._rslice_chain(c, u, theta, logl, counts, lmin, scale, chol, slices) for c in range(k)]
+
+        def step(c, sent):
+            try:
+                return chains[c].send(sent)
+            except StopIteration:
+                return None
+        pending = {c: p for c in range(k) if (p := step(c, None)) is not None}
+        while pending:
+            idx = list(pending)
+            th = self.transform(np.array([pending[c] for c in idx]))
+            y = self.like(th)
+            counts[idx, 3] += 1
+            pending = {c: p for j, c in enumerate(idx) if (p := step(c, (th[j], y[j]))) is not None}
+        return u, theta, logl, counts
+
+
+def rslice_scale(scale, counts):
+    """Slice-scale update after one batch: scale * 2 E / (E + C) with E expansions and C
+    contractions summed over the batch (dynesty's rule as recalled: a window that had to grow asks for
+    a larger scale, one that had to shrink for a smaller), kept in [1e-6, 10]."""
+    e, c = float(np.sum(counts[:, 1])), float(np.sum(counts[:, 2]))
+    if e + c == 0.0:
+        return float(scale)
+    return float(np.clip(scale * 2.0 * e / (e + c), 1e-6, 10.0))
+
 
 class DeviceWalker:
     """Random walks on the surrogate, one launch per batch (``ab_nested_walk``).
@@ -200,15 +289,17 @@ class DeviceWalker:
         theta = self.transform(u)
         return u, theta, self.like(theta)
 
-    def walk(self, u0, theta0, logl0, lmin, scale, chol, walks):
+    def _launch(self, entry, u0, theta0, logl0, lmin, scale, chol, steps, ncount, chain_offset=0):
+        """One ``entry`` launch (ab_nested_walk / ab_nested_rslice) over the batch: the end points on the
+        host and the device counts (k x ncount int32)."""
         torch, _lib = self._torch, self._lib
         hd = self.gp._hd
         k, d = u0.shape
         cfg = _lib.NestedConfig()
-        cfg.nchains, cfg.walks, cfg.y_kind = int(k), int(walks), int(self.lp.y_kind)
+        cfg.nchains, cfg.walks, cfg.y_kind = int(k), int(steps), int(self.lp.y_kind)
         cfg.use_normal_prior = int(np.any(self.prior_sd > 0))
         cfg.scale, cfg.lmin = float(scale), float(lmin) if np.isfinite(lmin) else -1.7976931348623157e308
-        cfg.seed, cfg.counter, cfg.chain_offset = self.seed, self.counter, 0
+        cfg.seed, cfg.counter, cfg.chain_offset = self.seed, self.counter, int(chain_offset)
         self.counter += 1
         cfg.y_scale, cfg.y_offset = self.lp.y_scale, self.lp.y_offset
         for i in range(d):
@@ -217,16 +308,30 @@ class DeviceWalker:
             cfg.theta_scale[i], cfg.theta_offset[i] = self.lp.theta_scale[i], self.lp.theta_offset[i]
         cl = np.ascontiguousarray(np.tril(chol), dtype=np.float64).reshape(-1)
         ctypes.memmove(cfg.chol, cl.ctypes.data, cl.nbytes)
-        # one device block in, one out: [u | theta | logl] and the accept counts
+        # one device block in, one out: [u | theta | logl] and the counts
         blk = torch.from_numpy(np.concatenate([u0.reshape(-1), theta0.reshape(-1), logl0.reshape(-1)])).to(self._dev)
         du, dth, dl = blk[:k * d], blk[k * d:2 * k * d], blk[2 * k * d:]
-        nacc = torch.zeros(k, dtype=torch.int32, device=self._dev)
-        _lib.check(hd.lib.ab_nested_walk(hd.h, ctypes.byref(cfg), _lib.ptr(du), _lib.ptr(dl), _lib.ptr(dth), _lib.ptr(nacc)),
-                   "ab_nested_walk")
+        cnt = torch.zeros(k * ncount, dtype=torch.int32, device=self._dev)
+        _lib.check(getattr(hd.lib, entry)(hd.h, ctypes.byref(cfg), _lib.ptr(du), _lib.ptr(dl), _lib.ptr(dth), _lib.ptr(cnt)),
+                   entry)
         host = blk.cpu().numpy()
+        return host[:k * d].reshape(k, d), host[k * d:2 * k * d].reshape(k, d), host[2 * k * d:], cnt
+
+    def walk(self, u0, theta0, logl0, lmin, scale, chol, walks):
+        k = len(u0)
+        u, theta, logl, nacc = self._launch("ab_nested_walk", u0, theta0, logl0, lmin, scale, chol, walks, 1)
         self.ncall += k * int(walks)
-        return (host[:k * d].reshape(k, d), host[k * d:2 * k * d].reshape(k, d), host[2 * k * d:],
-                float(nacc.sum().item()) / float(max(k * int(walks), 1)))
+        return u, theta, logl, float(nacc.sum().item()) / float(max(k * int(walks), 1))
+
+    def rslice(self, u0, theta0, logl0, lmin, scale, chol, slices, chain_offset=0):
+        """``slices`` random-direction slices per chain, one launch (``ab_nested_rslice``); returns
+        (u, theta, logl, counts) as :meth:`HostWalker.rslice`.  Row i draws the random numbers of
+        chain ``chain_offset + i``, so a sub-batch reproduces its rows of a larger batch."""
+        u, theta, logl, cnt = self._launch("ab_nested_rslice", u0, theta0, logl0, lmin, scale, chol, slices, 4,
+                                           chain_offset)
+        counts = cnt.cpu().numpy().reshape(-1, 4).astype(np.int64)
+        self.ncall += int(counts[:, 3].sum())
+        return u, theta, logl, counts
 
 
 class BatchPool:
@@ -272,13 +377,21 @@ class BatchLikelihood:
 # -------------------------------------------------------------------------------------------------
 class BatchedNestedSampler:
     """``walker``: :class:`DeviceWalker` or :class:`HostWalker`.  ``nbatch`` chains are advanced
-    together whenever the queue of replacement candidates runs dry."""
+    together whenever the queue of replacement candidates runs dry, by ``walks`` random-walk steps
+    (``sample="rwalk"``) or ``slices`` random-direction slices (``sample="rslice"``)."""
 
-    def __init__(self, walker, ndim, nlive=500, walks=25, nbatch=None, rstate=None, max_failed_rounds=50):
+    def __init__(self, walker, ndim, nlive=500, walks=25, nbatch=None, rstate=None, max_failed_rounds=50,
+                 sample="rwalk", slices=5):
+        if sample not in ("rwalk", "rslice"):
+            raise ValueError(f"sample={sample!r}: choose 'rwalk' or 'rslice'")
+        if int(slices) < 1:
+            raise ValueError(f"slices={slices!r}: at least one slice per chain")
         self.walker = walker
         self.ndim = int(ndim)
         self.nlive = int(nlive)
         self.walks = int(walks)
+        self.sample = sample
+        self.slices = int(slices)
         self.nbatch = int(nbatch) if nbatch else max(self.nlive // 4, 32)
         self.rng = np.random.default_rng(rstate)
         self.max_failed_rounds = int(max_failed_rounds)
@@ -304,6 +417,12 @@ class BatchedNestedSampler:
         """One batch of walks from random live points; adapts the proposal scale."""
         k = self.nbatch
         start = self.rng.integers(0, len(live_l), size=k)
+        if self.sample == "rslice":
+            u, theta, logl, counts = self.walker.rslice(live_u[start], live_t[start], live_l[start], lmin, self.scale,
+                                                        self._proposal_chol(live_u), self.slices)
+            self.scale = rslice_scale(self.scale, counts)
+            moved = counts[:, 0] > 0             # a chain with no completed slice is a copy of a live point
+            return [(u[i], theta[i], logl[i]) for i in range(k) if moved[i] and logl[i] > lmin]
         u, theta, logl, acc = self.walker.walk(live_u[start], live_t[start], live_l[start], lmin, self.scale,
                                                self._proposal_chol(live_u), self.walks)
         self.scale = float(np.clip(self.scale * np.exp((acc - 0.5) / max(self.ndim, 1)), 1e-6, 10.0))
@@ -340,8 +459,9 @@ class BatchedNestedSampler:
             if new is None:
                 # likelihood plateau / exhausted budget: the worst point stays dead, the run ends
                 if failed >= self.max_failed_rounds:
+                    moves = f"{self.slices} slices" if self.sample == "rslice" else f"{self.walks} walk steps"
                     warnings.warn(f"nested sampling: no point above L = {lmin:.6g} found in {failed} rounds of "
-                                  f"{self.nbatch} x {self.walks} walk steps (likelihood plateau?); ending the run")
+                                  f"{self.nbatch} x {moves} (likelihood plateau?); ending the run")
                 live_u, live_t = np.delete(live_u, worst, axis=0), np.delete(live_t, worst, axis=0)
                 live_l, live_b = np.delete(live_l, worst), np.delete(live_b, worst)
                 break
@@ -429,7 +549,11 @@ class BatchedNestedSampler:
                     alive = np.nonzero(L > l_lo)[0][:max(2, nlb)]
                 start = self.rng.choice(alive, size=nlb, replace=True)
                 chol = self._proposal_chol(U[alive]) if len(alive) > self.ndim else np.eye(self.ndim) * 0.1
-                u, t, l, _ = self.walker.walk(U[start], T[start], L[start], l_lo, self.scale, chol, max(self.walks, 2 * self.ndim))
+                if self.sample == "rslice":
+                    u, t, l, _ = self.walker.rslice(U[start], T[start], L[start], l_lo, self.scale, chol, self.slices)
+                else:
+                    u, t, l, _ = self.walker.walk(U[start], T[start], L[start], l_lo, self.scale, chol,
+                                                  max(self.walks, 2 * self.ndim))
                 b = np.full(nlb, l_lo)
             else:
                 u, t, l = self.walker.initial(nlb)

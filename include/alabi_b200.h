@@ -298,6 +298,24 @@ typedef struct ab_nested_config {
 int ab_sizeof_nested_config(void);
 int ab_nested_walk(ab_gp* h, const ab_nested_config* cfg, double* d_u, double* d_logl, double* d_theta,
                    int* d_naccept);
+/* The same replacement step by random-direction slice sampling (dynesty's sample="rslice"), with
+ * the same configuration, argument checks and return codes; cfg->walks is the number of slices.
+ * Slice s of chain c (F(x) = surrogate mean at prior_transform(u + x v) inside (0, 1)^d, -inf and
+ * no evaluation outside):
+ *   direction  z as the walk's normals at step = s; v = (chol z) * (scale / |z|)
+ *   window     r0 = u53(words 0, 1) of Philox block j0 = ceil(d / 2), counter
+ *              (chain_offset + c, s, j0, counter); x_l = -r0, x_r = 1 - r0
+ *   step out   while F(x_l) > lmin: x_l -= 1; then while F(x_r) > lmin: x_r += 1 (one nexpand each)
+ *   shrink     draw i = 0, 1, ...: x = x_l + u_i (x_r - x_l), u_i = u53(words 0, 1) of block
+ *              j0 + 1 + i; F(x) > lmin accepts u <- u + x v, otherwise x_l = x (x < 0) or
+ *              x_r = x (x > 0) (one ncontract)
+ * Window and point arithmetic is rounded operation by operation (no fused multiply-add).  Caps:
+ * a slice that needs more than 1024 expansions or more than 256 contractions ends its chain at the
+ * end point of the last completed slice, so every launch ends.  On return d_u / d_logl / d_theta are as for ab_nested_walk and d_counts (nchains x 4)
+ * holds per chain: slices completed (< walks for a chain stopped by a cap), nexpand, ncontract and
+ * surrogate evaluations.  A chain's result does not depend on the other chains of the batch. */
+int ab_nested_rslice(ab_gp* h, const ab_nested_config* cfg, double* d_u, double* d_logl, double* d_theta,
+                     int* d_counts);
 
 /* ---- NCCL helpers (SURVEY 8b / 8e): one process per GPU; the factor is trained once and
  *      broadcast over NVLink, argmin records and chain blocks are all_gathered.  The reference has
