@@ -63,9 +63,7 @@ SIGNATURES = {
     "ab_gp_create": (ctypes.c_int, [ctypes.POINTER(_P), ctypes.c_int, _P]),
     "ab_gp_destroy": (ctypes.c_int, [_P]),
     "ab_gp_set_few_query_path": (ctypes.c_int, [_P, ctypes.c_int]),
-    "ab_gp_set_variance_schedule": (ctypes.c_int, [_P, ctypes.c_int]),
     "ab_gp_append_point": (ctypes.c_int, [_P, _P]),
-    "ab_gp_debug_stamps": (ctypes.c_int, [_P, _P]),
     "ab_gp_predict_grad": (ctypes.c_int, [_P, _P, ctypes.c_int64, _P, _P, _P, _P]),
     "ab_gp_set_inputs": (ctypes.c_int, [_P, _P, ctypes.c_int64, ctypes.c_int]),
     "ab_gp_set_kernel": (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_double, c_double_p, ctypes.c_double,

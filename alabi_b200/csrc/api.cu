@@ -164,19 +164,6 @@ int ab_gp_destroy(ab_gp* h) {
     return 0;
 }
 
-int ab_gp_debug_stamps(ab_gp* h, void* d_buf) {
-    AB_REQUIRE(h, -1, "null handle");
-    h->df_dbg = d_buf;
-    return 0;
-}
-
-int ab_gp_set_variance_schedule(ab_gp* h, int mode) {
-    AB_REQUIRE(h, -1, "null handle");
-    AB_REQUIRE(mode >= 0 && mode <= 2, -1, "ab_gp_set_variance_schedule: mode must be 0 (auto), 1 or 2");
-    h->var_schedule = mode;
-    return 0;
-}
-
 int ab_gp_set_few_query_path(ab_gp* h, int enabled) {
     AB_REQUIRE(h, -1, "null handle");
     h->few_path = enabled != 0;

@@ -86,16 +86,8 @@ struct DfArgs {
     unsigned int* next_task;      // task counter
     int* abort_flag;
     const int2* tasks; int ntasks;
-    unsigned long long* dbg;      // optional: 6 globaltimer stamps per task (development)
     int64_t strideA, strideD;     // batch strides in doubles
 };
-
-__device__ __forceinline__ unsigned long long gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define DF_STAMP(slot) do { if (a.dbg && tid == 0) a.dbg[(size_t)task * 6 + (slot)] = gtime(); } while (0)
 
 __device__ __forceinline__ int ld_acquire(const int* p) {
     int v;
@@ -196,7 +188,6 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
         w.prog = prog_b;
         const int64_t row0 = (int64_t)i * NB, col0 = (int64_t)j * NB;
         int seen_i = 0, seen_j = 0;
-        DF_STAMP(0);
         // the tile of K itself is only needed after the long accumulation: pull it into L2 now
         for (int c = tid; c < NB * 8; c += Core::THREADS)
             asm volatile("prefetch.global.L2 [%0];" ::"l"(Ab + (row0 + (c >> 3)) * a.ld + col0 + (c & 7) * 16));
@@ -211,7 +202,6 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
             seen_i = gate.seen_i;
             seen_j = gate.seen_j;
         }
-        DF_STAMP(1);
         // ---- C = A_ij - S, staged in shared memory ------------------------------------
         // (A_ij still holds the covariance values written before this launch)
 #pragma unroll
@@ -228,7 +218,6 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
             }
         }
         __syncthreads();
-        DF_STAMP(2);
 
         if (i == j) {
             // ---- diagonal tile: Cholesky + inverse by 2 x 2 recursion on 64 x 64 blocks ----
@@ -342,7 +331,6 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
         } else {
             // ---- off-diagonal tile: L_ij = C D_j^-T (A operand resident, D_j^-1 streamed) ----
             w.wait(j, j, seen_j);                                    // diagonal tile of column j is final
-            DF_STAMP(3);
             const double* Dj = Db + (int64_t)j * NB * NB;
             abg::Acc out;
             out.zero();
@@ -391,20 +379,18 @@ chol_dataflow_kernel(const __grid_constant__ DfArgs a) {
             }
         }
         // ---- publish: the tile (and D_j^-1) is final -------------------------------------
-        DF_STAMP(4);
         __threadfence();
         __syncthreads();
         if (tid == 0) st_release(prog_b + i, j + 1);
-        DF_STAMP(5);
     }
 }
 
 // Factorisation of `nmat` matrices of T x T tiles (leading dimension T * 128), matrix b at
 // A + b * strideA etc. as described at DfArgs.  ctrl: 2 + nmat * T ints ([0] task counter,
 // [1] abort word, then prog), zeroed here with the info words; tasks: nmat * T (T + 1) / 2
-// entries.  Only the handle's own factor is timed (`profile`) and carries debug stamps.
+// entries.  Only the handle's own factor is timed (`profile`).
 int launch_dataflow(ab_gp* h, double* A, int64_t strideA, int T, int nmat, double* Dinv, double* logdet_parts,
-                    int* info, int* ctrl, const int2* tasks, unsigned long long* dbg, bool profile) {
+                    int* info, int* ctrl, const int2* tasks, bool profile) {
     static unsigned long long configured = 0;   // per-device bit: cudaFuncSetAttribute is per device
     if (h->device >= 64 || !((configured >> h->device) & 1ULL)) {
         AB_CUDA(cudaFuncSetAttribute(chol_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DF_SMEM_BYTES));
@@ -421,7 +407,6 @@ int launch_dataflow(ab_gp* h, double* A, int64_t strideA, int T, int nmat, doubl
     a.abort_flag = ctrl + 1;
     a.prog = ctrl + 2;
     a.tasks = tasks; a.ntasks = (int)ntasks;
-    a.dbg = dbg;
     a.strideA = strideA; a.strideD = (int64_t)T * NB * NB;
     const int grid = ntasks < h->nsm ? (int)ntasks : h->nsm;
     if (profile) ab_prof_begin(h, AB_PROF_FACTOR);
@@ -455,7 +440,7 @@ int ab_launch_factor_dataflow(ab_gp* h) {
     }
     int* ctrl = reinterpret_cast<int*>(h->scratch);
     rc = launch_dataflow(h, h->L, 0, T, 1, h->Dinv, h->logdet_parts, h->d_info, ctrl,
-                         reinterpret_cast<const int2*>(h->df_tasks), reinterpret_cast<unsigned long long*>(h->df_dbg), true);
+                         reinterpret_cast<const int2*>(h->df_tasks), true);
     if (rc) return rc;
     AB_CUDA(cudaMemcpyAsync(h->h_pinned + 9, ctrl + 1, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     return 0;
@@ -466,7 +451,7 @@ int ab_launch_factor_dataflow(ab_gp* h) {
 int ab_launch_factor_dataflow_batch(ab_gp* h, double* d_A, int64_t strideA, int T, int nmat, double* d_Dinv,
                                     double* d_logdet_parts, int* d_info, int* d_ctrl, const int2* d_tasks) {
     if (T < 1 || T > 4095 || nmat < 1 || nmat >= (1 << 19)) { ab_set_error("batched factorisation: bad shape"); return -1; }
-    return launch_dataflow(h, d_A, strideA, T, nmat, d_Dinv, d_logdet_parts, d_info, d_ctrl, d_tasks, nullptr, false);
+    return launch_dataflow(h, d_A, strideA, T, nmat, d_Dinv, d_logdet_parts, d_info, d_ctrl, d_tasks, false);
 }
 
 // task list of a batch: column by column over all matrices (host vector)

@@ -21,19 +21,19 @@
 //
 // This file: the C entry points; the kernel lives in ensemble_kernel.cuh (instantiated per kernel
 // family by ensemble_k0 / k1 / k2.cu).
-#include <stdio.h>
 #include <cmath>
 #include <vector>
 #include "ensemble_args.h"
 
-// Enqueue one sampler kernel on the handle's stream.  `first`: clear the barrier counter, the
-// NaN flag and the debug counters; later pieces of the same run clear the barrier counter only.
+// Enqueue one sampler kernel on the handle's stream.  `first`: clear the barrier counter and the
+// NaN flag; later pieces of the same run clear the barrier counter only.
 static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords, double* d_logp,
                        long long* d_naccept, double* d_chain, double* d_logp_chain, double* d_rec_q,
                        double* d_rec_lp, bool first) {
     if (!h->have_alpha) { ab_set_error("ab_ensemble_run: targets not set (call ab_gp_set_targets)"); return -2; }
     if (cfg->nwalkers < 2 || cfg->nsteps < 0 || cfg->thin_by < 1) { ab_set_error("bad ensemble configuration"); return -1; }
-    // scratch: [0, 4096) barrier word, NaN flag, debug counters; then the completion counters and the
+    if (cfg->reserved != 0) { ab_set_error("ab_ensemble_run: ab_ensemble_config.reserved must be 0"); return -1; }
+    // scratch: [0, 4096) barrier word and NaN flag; then the completion counters and the
     // segment sums of split wide units (3 kinds of half-step x units x AB_ENS_MAXSEG segments x 32 proposals)
     const int max_units = (cfg->nwalkers + 31) / 32;
     const size_t cnt_bytes = ((size_t)3 * max_units * sizeof(unsigned) + 255) / 256 * 256;
@@ -44,8 +44,6 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     // proposals per unit: 2 (small ensembles, many units), 32 = one lane per proposal once
     // there are enough proposals for one 32-wide unit per SM
     int p = (n_half >= 16 * nsm) ? 32 : 2;
-    if (cfg->reserved >= 2)                                                        // development override
-        p = (cfg->reserved == 32) ? 32 : 2;
     // dataflow schedule (ab_ensemble_config.schedule 0 = automatic, 1 = grid barriers): small ensembles
     // whose half-steps are latency bound; the launcher drops it when the training set is not resident
     const int dpad = h->d <= 2 ? 2 : h->d <= 4 ? 4 : h->d <= 8 ? 8 : h->d <= 24 ? (h->d + 3) / 4 * 4 : 32;   // the dispatch below
@@ -57,7 +55,7 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     // evaluates 32 proposals against 128-512 points, the segment sums meet in global memory and the CTA
     // that delivers a unit's last segment accepts (the ranged schedule of the large ensembles).
     int ch_hint = 0, maxseg = AB_ENS_MAXSEG;
-    if (p == 2 && !resident_small && cfg->reserved < 2 && cfg->schedule != 3) {
+    if (p == 2 && !resident_small && cfg->schedule != 3) {
         p = 32;
         const long long units = (n_half + 31) / 32;
         ch_hint = 128;
@@ -103,8 +101,7 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
         if (reinterpret_cast<uintptr_t>(A.chain_dst[q]) & 15) A.chain_vec = 0;
     A.barrier = reinterpret_cast<unsigned long long*>(h->scratch);
     A.nan_flag = reinterpret_cast<int*>(h->scratch + 1);
-    A.dbg = cfg->reserved == 1 ? reinterpret_cast<long long*>(h->scratch + 16) : nullptr;
-    AB_CUDA(cudaMemsetAsync(h->scratch, 0, first ? 256 : 8, h->stream));
+    AB_CUDA(cudaMemsetAsync(h->scratch, 0, first ? 16 : 8, h->stream));
     A.XsT = h->XsT; A.alpha = h->alpha; A.n = h->n; A.npad = h->npad; A.kp = h->kp; A.mean = h->mean;
     A.nwalkers = cfg->nwalkers; A.d = h->d; A.nsteps = cfg->nsteps; A.thin_by = cfg->thin_by;
     A.init_logp = cfg->init_logp; A.randomize_split = cfg->randomize_split; A.a = cfg->a;
@@ -132,20 +129,18 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     const int units_half = (n_half + p - 1) / p;
     int ws = 1;
     if (p == 32) ws = 16;                      // wide unit = the whole CTA (16 warps)
-    else if (cfg->warps_per_unit > 0 && cfg->warps_per_unit != 104) ws = cfg->warps_per_unit;
+    else if (cfg->warps_per_unit > 0) ws = cfg->warps_per_unit;
     else while (ws < 8 && units_half * ws * 2 <= nsm * 8) ws *= 2;   // the half-step in ONE pass of one 8-warp CTA per SM
-    if (ws != 1 && ws != 2 && ws != 4 && ws != 8 && !(p == 32 && ws == 16)) { ab_set_error("warps_per_unit must be 1, 2, 4, 8 or 104"); return -1; }
+    if (ws != 1 && ws != 2 && ws != 4 && ws != 8 && !(p == 32 && ws == 16)) { ab_set_error("warps_per_unit must be 0, 1, 2, 4 or 8"); return -1; }
     A.ws = ws;
     // 4-warp CTAs (one unit each, several per SM) when 8-warp CTAs would run several units in lockstep
-    // and every unit still gets a co-resident CTA; warps_per_unit = 104 forces them (development)
-    const int small_cta = (p != 2) ? 0 : (cfg->warps_per_unit == 104) ? 2 : (cfg->warps_per_unit == 0 && ws < 8) ? 1 : 0;
+    // and every unit still gets a co-resident CTA
+    const bool small_cta = p == 2 && cfg->warps_per_unit == 0 && ws < 8;
     rc = (h->kp.kind == 0) ? ab_ens_launch_k0(h, A, n_half, p, small_cta, ws)
        : (h->kp.kind == 1) ? ab_ens_launch_k1(h, A, n_half, p, small_cta, ws)
        : (h->kp.kind == 2) ? ab_ens_launch_k2(h, A, n_half, p, small_cta, ws)
                            : ab_ens_launch_k3(h, A, n_half, p, small_cta, ws);
-    if (rc) return rc;
-    h->ens_dbg = A.dbg != nullptr; h->ens_ws = A.ws;
-    return 0;
+    return rc;
 }
 
 extern "C" int ab_ensemble_launch(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords, double* d_logp,
@@ -156,7 +151,7 @@ extern "C" int ab_ensemble_launch(ab_gp* h, const ab_ensemble_config* cfg, doubl
     AB_CUDA(cudaSetDevice(h->device));
     int rc = ens_enqueue(h, cfg, d_coords, d_logp, d_naccept, d_chain, d_logp_chain, d_rec_q, d_rec_lp, true);
     if (rc) return rc;
-    AB_CUDA(cudaMemcpyAsync(h->h_pinned, h->scratch, 256, cudaMemcpyDeviceToHost, h->stream));
+    AB_CUDA(cudaMemcpyAsync(h->h_pinned, h->scratch, 16, cudaMemcpyDeviceToHost, h->stream));
     h->ens_pending = true;
     return 0;
 }
@@ -195,7 +190,6 @@ extern "C" int ab_ensemble_run_host(ab_gp* h, const ab_ensemble_config* cfg, dou
         c.nsteps = (int)(nr * cfg->thin_by);
         c.first_step = cfg->first_step + done * cfg->thin_by;
         c.init_logp = first ? cfg->init_logp : 0;
-        c.reserved = 0;
         rc = ens_enqueue(h, &c, d_coords, d_logp, d_naccept, d_chain + done * nw * d, d_logp_chain + done * nw, nullptr,
                          nullptr, first);
         if (rc) break;
@@ -208,7 +202,7 @@ extern "C" int ab_ensemble_run_host(ab_gp* h, const ab_ensemble_config* cfg, dou
         first = false;
     } while (done < rows);
     if (!rc) {
-        cudaMemcpyAsync(h->h_pinned, h->scratch, 256, cudaMemcpyDeviceToHost, h->stream);
+        cudaMemcpyAsync(h->h_pinned, h->scratch, 16, cudaMemcpyDeviceToHost, h->stream);
         for (size_t b = 0; b < pieces.size() && !rc; b++) {
             const Piece& p = pieces[b];
             cudaError_t e = cudaStreamWaitEvent(h->copy_stream, evs[b], 0);
@@ -245,11 +239,6 @@ extern "C" int ab_ensemble_finish(ab_gp* h) {
     h->ens_pending = false;
     AB_CUDA(cudaSetDevice(h->device));
     AB_CUDA(cudaStreamSynchronize(h->stream));
-    if (h->ens_dbg) {
-        const long long* dd = reinterpret_cast<const long long*>(h->h_pinned + 16);
-        fprintf(stderr, "[ensemble dbg] cycles/half-step: proposal %.0f compute %.0f accept %.0f barrier %.0f (n=%lld, ws=%d)\n",
-                (double)dd[0] / dd[4], (double)dd[1] / dd[4], (double)dd[2] / dd[4], (double)dd[3] / dd[4], dd[4], h->ens_ws);
-    }
     if (reinterpret_cast<int*>(h->h_pinned + 1)[0] == 2) {
         ab_set_error("ensemble sampler: a partner record did not arrive within the watchdog time (dataflow schedule); "
                      "the chain of this run is invalid");

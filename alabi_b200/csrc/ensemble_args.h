@@ -13,7 +13,7 @@ struct EnsArgs {
     // state and outputs
     double* coords; double* logp; long long* naccept;
     double* chain; double* logp_chain; double* rec_q; double* rec_lp;
-    unsigned long long* barrier; int* nan_flag; long long* dbg;   // dbg: optional phase cycle counters (block 0)
+    unsigned long long* barrier; int* nan_flag;
     // surrogate
     const double* XsT; const double* alpha; long long n, npad;
     KernParams kp; double mean;
@@ -49,7 +49,7 @@ struct EnsArgs {
 
 // one per kernel family (KIND = 0 ExpSquared, 1 Matern-3/2, 2 Matern-5/2): picks the padded dimension
 // and the unit shape, launches on the handle's stream.  Defined in ensemble_k<KIND>.cu.
-int ab_ens_launch_k0(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
-int ab_ens_launch_k1(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
-int ab_ens_launch_k2(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
-int ab_ens_launch_k3(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws);
+int ab_ens_launch_k0(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws);
+int ab_ens_launch_k1(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws);
+int ab_ens_launch_k2(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws);
+int ab_ens_launch_k3(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws);

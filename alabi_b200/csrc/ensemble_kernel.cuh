@@ -332,8 +332,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                     b = it;
                     it += gridDim.x;
                 }
-                long long t0 = 0, t1 = 0, t2 = 0;
-                if (A.dbg) t0 = clock64();
                 if (!PW && !first_seg) prep(step, split, b);         // wide: further units of this CTA inline
                 first_seg = false;
                 item_sync();                                         // small units: this item's prep buffer is complete
@@ -491,7 +489,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                     sInside[unit][e] = inside;
                 }
                 csync();
-                if (A.dbg) t1 = clock64();
                 // ---- surrogate mean of the two proposals of this unit ------------
                 if constexpr (WIDE) {
                     double qv[D];
@@ -617,7 +614,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                 }
                 }
                 csync();
-                if (A.dbg) t2 = clock64();
                 // ---- split units: publish this slice's sums; the CTA that completes the unit goes on ----
                 bool finisher = true;
                 if (WIDE && nseg > 1) {
@@ -736,10 +732,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                         }
                     }
                 }
-                if (A.dbg && blockIdx.x == 0 && tid == 0) {
-                    long long t3 = clock64();
-                    A.dbg[0] += t1 - t0; A.dbg[1] += t2 - t1; A.dbg[2] += t3 - t2;
-                }
                 // wide: the proposal lanes own sW.. of their unit, the next prep / gather by the same
                 // lanes follows in program order; small units: the next item's values sit in the other
                 // prep buffer since the barrier after the compute phase.  sQs / sPart readers are fenced
@@ -747,8 +739,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                 csync();
                 if constexpr (PW) pbuf = (pbuf + 1) % 3;
             }
-            long long tb = 0;
-            if (A.dbg) { csync(); tb = clock64(); }
             const bool flow_step = FLOW && step >= 0;
             if (!flow_step) grid_arrive(A.barrier, bar_target, csync);
             {   // random-stream part of the next half-step, overlapped with the barrier
@@ -766,7 +756,6 @@ ensemble_kernel(const __grid_constant__ EnsArgs A) {
                 flow_prev_target = bar_target;
                 flow_have_prev = true;
             }
-            if (A.dbg && blockIdx.x == 0 && tid == 0) { A.dbg[3] += clock64() - tb; A.dbg[4] += 1; }
         }
     }
 }
@@ -842,9 +831,9 @@ int launch_ens_p(ab_gp* h, EnsArgs& A, int n_half, bool one_pass_only = false) {
 }
 
 // n_half: proposals of the larger half-step (or all walkers for a log-prob-only call)
-// small_cta: 0 = 8-warp CTAs (ws8 warps per unit), 1 = try 4-warp CTAs first, 2 = 4-warp CTAs in any case
+// small_cta: try 4-warp CTAs first; else (or when they would not all be co-resident) 8-warp CTAs, ws8 warps per unit
 template <int KIND, int D>
-int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws8) {
+int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws8) {
     // wide unit: 16 warps split the training points (4 warps per scheduler hide the FP64 dependency
     // latency that 2 leave exposed: ncu, c5 share, FP64 pipe 56 % with 8 warps); one CTA per SM
     if (p == 32) return launch_ens_p<KIND, D, 32, 16>(h, A, n_half);
@@ -854,7 +843,7 @@ int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws8) 
         // is covered by its neighbour's kernel evaluations on the same SM.
         uint4* ring = A.ring;
         A.ws = 4;
-        const int rc = launch_ens_p<KIND, D, 2, 4>(h, A, n_half, small_cta == 1);
+        const int rc = launch_ens_p<KIND, D, 2, 4>(h, A, n_half, true);
         if (rc != 1) return rc;
         A.ring = ring;
     }
@@ -864,7 +853,7 @@ int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws8) 
 
 // padded-dimension dispatch of one kernel family
 template <int KIND>
-int launch_ens_kind(ab_gp* h, EnsArgs& A, int n_half, int p, int small_cta, int ws) {
+int launch_ens_kind(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws) {
     const int d = h->d;
 #define AB_ENS(DD) return launch_ens<KIND, DD>(h, A, n_half, p, small_cta, ws)
     if (d <= 2) AB_ENS(2);

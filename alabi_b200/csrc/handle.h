@@ -47,19 +47,16 @@ struct ab_gp {
     bool profiling = false;
     std::vector<cudaEvent_t> prof_ev[AB_PROF_FAMILIES];
 
-    int var_schedule = 0;                 // variance GEMM over full panels: 0 auto, 1 one CTA per query tile, 2 row-block pairs per CTA
     bool few_path = true;                 // m <= 8 queries: the spread-one-query kernels of predict.cu (false: batched kernels)
     void* df_tasks = nullptr;             // dataflow task list (device) for df_tasks_T block rows
     int df_tasks_T = 0;
     void* cov_items = nullptr;            // work list of cov_strip_kernel for cov_items_nt tile rows
     int cov_items_nt = 0, cov_items_seg = 0, cov_items_count = 0;
-    void* df_dbg = nullptr;               // development: per-task time stamps of the dataflow kernel (caller-owned)
     bool factored = false, have_linv = false, have_kinv = false, have_alpha = false;
     int info = 0;
     double logdet = 0.0, quad = 0.0;
     // ab_ensemble_launch -> ab_ensemble_finish
-    bool ens_pending = false, ens_dbg = false;
-    int ens_ws = 0;
+    bool ens_pending = false;
 };
 
 int ab_ensure_scratch(ab_gp* h, size_t bytes);

@@ -844,7 +844,8 @@ static int launch_variance(ab_gp* h, int T, const double* P, int64_t ldp, int64_
                            double* var, double* part) {
     cudaStream_t s = h->stream;
     const unsigned ntq = (unsigned)((cnt + abg::BN - 1) / abg::BN);
-    const bool pair = part && T >= 2 && (h->var_schedule == 2 || (h->var_schedule == 0 && T >= 48 && (int)ntq * 2 > h->nsm));   // auto: N >= 6144 (measured: 0.2 % slower at N = 8192 for a quarter of the DRAM traffic, 3 % slower at N = 4000)
+    // row-block pairs of a tile on adjacent CTAs from N >= 6144 (measured: 0.2 % slower at N = 8192 for a quarter of the DRAM traffic, 3 % slower at N = 4000)
+    const bool pair = part && T >= 48 && (int)ntq * 2 > h->nsm;
     if (pair) {
         const long long nitems = (long long)((T + 1) / 2) * ntq;
         const unsigned grid = (unsigned)(nitems < h->nsm ? nitems : h->nsm);

@@ -151,7 +151,6 @@ class EnsembleSampler:
         cfg.nwalkers, cfg.nsteps, cfg.thin_by = self.nwalkers, int(nsteps), int(thin_by)
         cfg.init_logp, cfg.randomize_split = int(init_logp), int(self.randomize_split)
         cfg.warps_per_unit, cfg.y_kind = self.warps_per_unit, lp.y_kind
-        cfg.reserved = int(getattr(self, 'debug_timing', 0))       # development aid, see ab_ensemble_config.reserved
         cfg.a, cfg.seed = self.a, self.seed
         cfg.first_step, cfg.walker_offset = self._step_counter, int(walker_offset)
         cfg.y_scale, cfg.y_offset = lp.y_scale, lp.y_offset

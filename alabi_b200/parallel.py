@@ -333,15 +333,10 @@ class PeerChainBuffers:
         """What ``EnsembleSampler.run_mcmc(gather=...)`` takes: this rank's walkers are columns
         [column, column + nwalkers_local) of every row.  ``row0`` / ``rows``: the stored rows a piece of a
         longer run writes; ``keep_local=False``: the sampler keeps no copy of its own columns."""
-        import os
         rows = self.shape[0] - row0 if rows is None else int(rows)
         c_off = row0 * self.shape[1] * self.shape[2] * 8
         l_off = self._lp_off + row0 * self.shape[1] * 8
         peers = list(self.peers)
-        rep = int(os.environ.get("ALABI_B200_PEER_REPEAT", "1"))     # development: the store volume of more ranks on few GPUs
-        if rep > 1:
-            from . import _lib
-            peers = (peers * rep)[:_lib.MAX_PEERS]
         return {"chain": self.chain[row0:row0 + rows], "log_prob": self.log_prob[row0:row0 + rows],
                 "nwalkers_total": self.shape[1], "column": int(column), "keep_local": bool(keep_local),
                 "peer_chain_ptrs": [p + c_off for p in peers], "peer_log_prob_ptrs": [p + l_off for p in peers]}

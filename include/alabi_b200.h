@@ -81,14 +81,6 @@ int ab_gp_destroy(ab_gp* h);
  * alabi/utility.py:629-946) use kernels that spread one query over the GPU and reproduce the
  * batched kernels' bits; 0 sends them through the batched kernels (cross-check), default 1 */
 int ab_gp_set_few_query_path(ab_gp* h, int enabled);
-/* schedule of the variance GEMM over full query panels: 1 = one CTA per 128-query tile loops over
- * all row blocks (its panel slice is re-streamed from HBM once per row block when N is large),
- * 2 = the row blocks of a tile are spread over adjacent CTAs in pairs (p, T - 1 - p) that share
- * the slice through the L2, 0 (default) = 2 for N >= 6144 on full panels, else 1.  Same bits. */
-int ab_gp_set_variance_schedule(ab_gp* h, int mode);
-/* development aid: device buffer (6 x uint64 per tile task, column-major task order) that the
- * dataflow Cholesky fills with %globaltimer stamps; NULL (default) disables it */
-int ab_gp_debug_stamps(ab_gp* h, void* d_buf);
 
 /* Append ONE training point (d doubles on the device, same space as X) to a
  * factorised model in O(N^2): bordered Cholesky update instead of the full
@@ -205,12 +197,9 @@ typedef struct ab_ensemble_config {
     int thin_by;           /* store every thin_by-th step (>= 1) */
     int init_logp;         /* 1: evaluate log-prob of d_coords first */
     int randomize_split;   /* 1: coin per walker pair, 0: parity split */
-    int warps_per_unit;    /* 0 = auto; 1/2/4/8 = that many warps per unit inside 8-warp CTAs; 104 = one 4-warp
-                            * unit per CTA, several CTAs per SM (what auto picks when every unit of a half-step
-                            * then has a co-resident CTA) */
+    int warps_per_unit;    /* 0 = auto; 1/2/4/8 = that many warps per unit inside 8-warp CTAs */
     int y_kind;            /* y = ys*y_scale + y_offset (0), -10^ys (1), 10^ys (2) */
-    int reserved;            /* 0 in production.  Development aids: 1 = print per-phase cycle counts of
-                              * block 0 to stderr; 2 / 32 = force that many proposals per unit */
+    int reserved;          /* must be 0 */
     double a;              /* stretch scale (emcee default 2.0) */
     uint64_t seed;
     int64_t first_step;    /* step counter of the first step (continuing chains) */

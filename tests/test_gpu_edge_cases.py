@@ -1,7 +1,7 @@
 """Edge cases of the GPU path (through the C ABI): smallest and ragged sizes, the
 padding boundaries of the 128-row blocking, the maximum dimension, empty query
 sets, duplicated training points, non-finite inputs, the ill-conditioned default
-white noise, and P = 4 proposals per unit in the sampler."""
+white noise, and both unit sizes of the sampler."""
 import numpy as np
 import pytest
 
@@ -121,32 +121,43 @@ def test_non_finite_inputs_are_reported():
 
 
 def test_sampler_proposals_per_unit_variants_replay():
-    """P = 2, 4 proposals per unit and the wide 32-proposal unit (one lane per proposal,
-    the large-ensemble configuration), each replayed on the CPU from the same draws."""
+    """P = 2 proposals per unit (90 walkers) and the wide 32-proposal unit (one lane per proposal,
+    the large-ensemble configuration: 32 walkers per SM plus 26, so the last unit is partly
+    filled), each replayed on the CPU from the same draws; a configuration with
+    ab_ensemble_config.reserved != 0 is refused."""
     import alabi_b200 as ab
     from alabi_b200.ensemble import EnsembleSampler, SurrogateLogProb
     rng = np.random.default_rng(8)
-    n, d, nw = 700, 3, 90
+    n, d = 700, 3
     X = rng.uniform(-2, 2, size=(n, d))
     y = -0.5 * np.sum((X / 0.9) ** 2, axis=1)
     o, g = _pair("ExpSquaredKernel", X, y, np.array([0.3, 0.1, 0.5]))
     b = np.array([(-2.0, 2.0)] * d)
     lp = SurrogateLogProb(g, y, b)
-    p0 = rng.uniform(-1, 1, size=(nw, d))
 
     def lp_o(q):
         q = np.atleast_2d(q)
         inside = np.all((q > b[:, 0]) & (q < b[:, 1]), axis=1)
         return np.where(inside, o.predict(y, q), -np.inf)
-    chains = []
-    for mode in (2, 4, 32):
+    nsm = ab._lib.load().ab_device_sm_count(g._hd.device)
+    assert nsm > 0
+    for nw in (90, 32 * nsm + 26):
+        p0 = rng.uniform(-1, 1, size=(nw, d))
         s = EnsembleSampler(nw, d, lp, seed=21)
-        s.debug_timing = mode                                   # development override: proposals per unit
         s.run_mcmc(p0, 25)
-        chains.append(s.get_chain())
-    ref, _, _, _ = oem.replay_device_chain(p0, lp_o, 25, 21)
-    for c in chains:
-        assert np.allclose(c, ref, rtol=1e-9, atol=1e-12)
+        ref, _, _, _ = oem.replay_device_chain(p0, lp_o, 25, 21)
+        assert np.allclose(s.get_chain(), ref, rtol=1e-9, atol=1e-12)
+
+    s = EnsembleSampler(90, d, lp, seed=21)
+    config = s._config
+
+    def reserved_config(*args, **kwargs):
+        cfg = config(*args, **kwargs)
+        cfg.reserved = 1
+        return cfg
+    s._config = reserved_config
+    with pytest.raises(ab._lib.AlabiB200Error, match="reserved must be 0"):
+        s.run_mcmc(rng.uniform(-1, 1, size=(90, d)), 5)
 
 
 def test_round2_paths_at_their_smallest_sizes():
