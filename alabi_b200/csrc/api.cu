@@ -358,7 +358,7 @@ int ab_gp_grad_log_likelihood(ab_gp* h, const double* d_y, double* h_out) {
     AB_CUDA(cudaSetDevice(h->device));
     rc = ensure_kinv(h);
     if (rc) return rc;
-    rc = ab_launch_grad(h, nullptr);
+    rc = ab_launch_grad(h);
     if (rc) return rc;
     AB_CUDA(cudaStreamSynchronize(h->stream));
     memcpy(h_out, h->h_pinned, (h->d + 3 + (h->kp.kind == AB_KERNEL_RATQUAD ? 1 : 0)) * sizeof(double));

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
+#include <type_traits>
 
 #define AB_MAX_DIM 32     // maximum input dimension (per-dimension metric)
 #define AB_NB 128         // block size of every blocked dense algorithm; matrices are padded to it
@@ -218,6 +219,32 @@ __device__ __forceinline__ void ab_radial_both(double r2, double alpha, double i
         kv = (1.0 + r + r * r * 0.3333333333333333) * e; gv = -5.0 * (1.0 + r) * e * 0.16666666666666666;
     }
 }
+
+// The input dimensions the kernels are compiled for.  A kernel templated on D handles d <= D only
+// (coordinates past D would be dropped), so every launcher picks D here.
+inline int ab_padded_dim(int d) {
+    return d <= 2 ? 2 : d <= 4 ? 4 : d <= 8 ? 8 : d <= 12 ? 12 : d <= 16 ? 16 : d <= 20 ? 20 : d <= 24 ? 24 : 32;
+}
+
+// f(std::integral_constant<int, D>{}) for the padded dimension D of d
+template <class F>
+auto ab_dispatch_dim(int d, F&& f) {
+    switch (ab_padded_dim(d)) {
+        case 2: return f(std::integral_constant<int, 2>{});
+        case 4: return f(std::integral_constant<int, 4>{});
+        case 8: return f(std::integral_constant<int, 8>{});
+        case 12: return f(std::integral_constant<int, 12>{});
+        case 16: return f(std::integral_constant<int, 16>{});
+        case 20: return f(std::integral_constant<int, 20>{});
+        case 24: return f(std::integral_constant<int, 24>{});
+        default: return f(std::integral_constant<int, 32>{});
+    }
+}
+
+// Shared memory the samplers give a training set they keep resident: n points of D padded coordinates
+// plus alpha.  A set within the budget is loaded once per run; a larger one is streamed in chunks.
+constexpr size_t AB_RESIDENT_SMEM = 160 * 1024;
+inline bool ab_resident(long long n, int D) { return (size_t)n * (D + 1) * 8 <= AB_RESIDENT_SMEM; }
 
 #define AB_DISPATCH_KIND(kind, ...)                                   \
     do {                                                              \

@@ -46,8 +46,7 @@ static int ens_enqueue(ab_gp* h, const ab_ensemble_config* cfg, double* d_coords
     int p = (n_half >= 16 * nsm) ? 32 : 2;
     // dataflow schedule (ab_ensemble_config.schedule 0 = automatic, 1 = grid barriers): small ensembles
     // whose half-steps are latency bound; the launcher drops it when the training set is not resident
-    const int dpad = h->d <= 2 ? 2 : h->d <= 4 ? 4 : h->d <= 8 ? 8 : h->d <= 24 ? (h->d + 3) / 4 * 4 : 32;   // the dispatch below
-    const bool resident_small = (size_t)h->n * (dpad + 1) * 8 <= 160 * 1024;
+    const bool resident_small = ab_resident(h->n, ab_padded_dim(h->d));
     // Small ensemble on a training set that does not fit shared memory (emcee's default 10 x ndim walkers on
     // an N = 8192 surrogate): a 2-proposal unit would stream all N points through ONE CTA per half-step
     // (86 us per step at N = 8192, d = 10, whatever the walker count).  "Spread" mode runs the wide unit

@@ -766,11 +766,10 @@ int launch_ens_p(ab_gp* h, EnsArgs& A, int n_half, bool one_pass_only = false) {
     constexpr int ETHREADS = EW * 32 + (P == 32 ? 0 : 32);     // small units: + the prep warp
     void (*kern)(const EnsArgs) = ensemble_kernel<KIND, D, EW, P>;
     // shared memory: resident when the whole training set fits, else two chunk buffers
-    const size_t budget = 160 * 1024;
-    long long need = (long long)A.n * (D + 1) * 8;
+    const bool resident = ab_resident(A.n, D);
     int ch;
     size_t smem;
-    if ((size_t)need <= budget) {
+    if (resident) {
         ch = (int)((A.n + 31) / 32 * 32);
         if (ch < 32) ch = 32;
         smem = (size_t)ch * (D + 1) * 8;
@@ -785,11 +784,11 @@ int launch_ens_p(ab_gp* h, EnsArgs& A, int n_half, bool one_pass_only = false) {
     }
     A.ch = ch;
     if constexpr (P == 32 && EW == 16) {
-        if ((size_t)need > budget && ch == 512 && A.ch_hint == 0) kern = ensemble_kernel<KIND, D, EW, P, 512>;
+        if (!resident && ch == 512 && A.ch_hint == 0) kern = ensemble_kernel<KIND, D, EW, P, 512>;
     }
     if constexpr (P == 2) {
         // dataflow schedule: resident training set, a ring was provided by the caller
-        if (A.ring && (size_t)need <= budget) kern = ensemble_kernel<KIND, D, EW, P, 0, true>;
+        if (A.ring && resident) kern = ensemble_kernel<KIND, D, EW, P, 0, true>;
         else A.ring = nullptr;
     } else {
         A.ring = nullptr;
@@ -804,7 +803,7 @@ int launch_ens_p(ab_gp* h, EnsArgs& A, int n_half, bool one_pass_only = false) {
     if (one_pass_only && grid_max < nbatch) return 1;
     int grid = grid_max;
     A.ranged = 0;
-    if (P == 32 && (size_t)need > budget) {
+    if (P == 32 && !resident) {
         // streamed wide unit: equal contiguous ranges of (unit, chunk) pairs per CTA when every CTA
         // gets at least 4 chunks and no unit is cut into more than AB_ENS_MAXSEG segments
         const long long nch = A.npad / ch;
@@ -854,17 +853,7 @@ int launch_ens(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws8)
 // padded-dimension dispatch of one kernel family
 template <int KIND>
 int launch_ens_kind(ab_gp* h, EnsArgs& A, int n_half, int p, bool small_cta, int ws) {
-    const int d = h->d;
-#define AB_ENS(DD) return launch_ens<KIND, DD>(h, A, n_half, p, small_cta, ws)
-    if (d <= 2) AB_ENS(2);
-    else if (d <= 4) AB_ENS(4);
-    else if (d <= 8) AB_ENS(8);
-    else if (d <= 12) AB_ENS(12);
-    else if (d <= 16) AB_ENS(16);
-    else if (d <= 20) AB_ENS(20);
-    else if (d <= 24) AB_ENS(24);
-    else AB_ENS(32);
-#undef AB_ENS
+    return ab_dispatch_dim(h->d, [&](auto D) { return launch_ens<KIND, D>(h, A, n_half, p, small_cta, ws); });
 }
 
 }  // namespace

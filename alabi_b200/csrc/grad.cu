@@ -123,7 +123,7 @@ grad_final_kernel(const double* __restrict__ partials, int ntiles, const double*
 
 // Needs h->Kinv and h->alpha.  Leaves d + 3 doubles (d + 4 for the rational quadratic kernel) in
 // h->h_pinned (async copy).
-int ab_launch_grad(ab_gp* h, double* /*unused*/) {
+int ab_launch_grad(ab_gp* h) {
     const int T = (int)(h->npad / NB);
     const int ntiles = T * (T + 1) / 2;
     const int nx = (h->kp.kind == 3) ? kExtra<3> : 0;
@@ -134,24 +134,16 @@ int ab_launch_grad(ab_gp* h, double* /*unused*/) {
     cudaStream_t s = h->stream;
     // the per-dimension loops are unrolled over the template dimension: instantiate the padded
     // dimension of the problem, not AB_MAX_DIM (d = 10 ran 32-long predicated loops with 230 registers)
-#define AB_GT(DM)                                                                                                    \
-    do {                                                                                                             \
-        AB_DISPATCH_KIND(h->kp.kind, {                                                                               \
-            const int smem = (2 * DM * NB + 2 * NB + 8 * (DM + 2 + kExtra<KIND>)) * 8;                               \
-            AB_CUDA(cudaFuncSetAttribute(grad_tiles_kernel<KIND, DM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-            grad_tiles_kernel<KIND, DM><<<ntiles, 256, smem, s>>>(h->Kinv, h->npad, h->XsT, h->npad, h->n, h->alpha,  \
-                                                                  h->kp, partials);                                  \
-        });                                                                                                          \
-    } while (0)
-    if (h->d <= 2) AB_GT(2);
-    else if (h->d <= 4) AB_GT(4);
-    else if (h->d <= 8) AB_GT(8);
-    else if (h->d <= 12) AB_GT(12);
-    else if (h->d <= 16) AB_GT(16);
-    else if (h->d <= 20) AB_GT(20);
-    else if (h->d <= 24) AB_GT(24);
-    else AB_GT(32);
-#undef AB_GT
+    rc = ab_dispatch_dim(h->d, [&](auto DM) {
+        AB_DISPATCH_KIND(h->kp.kind, {
+            const int smem = (2 * DM * NB + 2 * NB + 8 * (DM + 2 + kExtra<KIND>)) * 8;
+            AB_CUDA(cudaFuncSetAttribute(grad_tiles_kernel<KIND, DM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            grad_tiles_kernel<KIND, DM><<<ntiles, 256, smem, s>>>(h->Kinv, h->npad, h->XsT, h->npad, h->n, h->alpha,
+                                                                  h->kp, partials);
+        });
+        return 0;
+    });
+    if (rc) return rc;
     AB_CHECK_LAUNCH();
     if (nx) grad_final_kernel<1><<<1, 256, 0, s>>>(partials, ntiles, h->alpha, h->n, h->d, exp(h->white_noise), h->scratch);
     else grad_final_kernel<0><<<1, 256, 0, s>>>(partials, ntiles, h->alpha, h->n, h->d, exp(h->white_noise), h->scratch);

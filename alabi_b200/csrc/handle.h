@@ -93,7 +93,7 @@ int ab_launch_build_kinv(ab_gp* h);
 int ab_launch_mirror_lower(ab_gp* h, double* A, int64_t ld);
 int ab_launch_mirror_lower_n(ab_gp* h, double* A, int64_t ld, int64_t n);
 // grad.cu
-int ab_launch_grad(ab_gp* h, double* h_out);
+int ab_launch_grad(ab_gp* h);
 // predict.cu
 int ab_launch_predict(ab_gp* h, const double* Xq, int64_t m, double* mu, double* var);
 int64_t ab_predict_panel_queries(ab_gp* h);

@@ -381,12 +381,11 @@ nested_rslice_kernel(const __grid_constant__ WalkArgs A) {
 
 template <int D>
 int launch_nested(ab_gp* h, WalkArgs& A, void (*kern)(const WalkArgs)) {
-    const size_t budget = 160 * 1024;
     int ch;
-    if ((size_t)A.n * (D + 1) * 8 <= budget) {
+    if (ab_resident(A.n, D)) {
         ch = (int)((A.n + 31) / 32 * 32);
     } else {
-        ch = (int)(budget / ((D + 1) * 8)) / 32 * 32;
+        ch = (int)(AB_RESIDENT_SMEM / ((D + 1) * 8)) / 32 * 32;
     }
     if (ch < 32) ch = 32;
     A.ch = ch;
@@ -430,20 +429,12 @@ int nested_args(const char* what, ab_gp* h, const ab_nested_config* cfg, double*
 }
 
 int dispatch_nested(ab_gp* h, WalkArgs& A, bool rslice) {
-    int rc = 0;
-    const int d = A.d;
-#define AB_NW(DD) AB_DISPATCH_KIND(h->kp.kind, rc = (launch_nested<DD>(h, A, rslice ? nested_rslice_kernel<KIND, DD> \
-                                                                                    : nested_walk_kernel<KIND, DD>)))
-    if (d <= 2) AB_NW(2);
-    else if (d <= 4) AB_NW(4);
-    else if (d <= 8) AB_NW(8);
-    else if (d <= 12) AB_NW(12);
-    else if (d <= 16) AB_NW(16);
-    else if (d <= 20) AB_NW(20);
-    else if (d <= 24) AB_NW(24);
-    else AB_NW(32);
-#undef AB_NW
-    return rc;
+    return ab_dispatch_dim(A.d, [&](auto D) {
+        int rc = 0;
+        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_nested<D>(h, A, rslice ? nested_rslice_kernel<KIND, D>
+                                                                          : nested_walk_kernel<KIND, D>)));
+        return rc;
+    });
 }
 
 }  // namespace

@@ -18,6 +18,7 @@
 //             few_* kernels spread one query over the GPU and reproduce the batched
 //             kernels' summation order, so a query has the same bits in any batch.
 #include <float.h>
+#include <algorithm>
 #include "handle.h"
 #include "dmma_gemm.cuh"
 
@@ -140,13 +141,36 @@ __device__ __forceinline__ void tile_finish_var(double (&tot)[4][2], double* red
     if (threadIdx.x < 128 && q < m) var[q] = amp - (red[threadIdx.x] + red[128 + threadIdx.x]);
 }
 
+// Per-thread block values (tile_thread_sq) of row block i of L^-1 P for the query tile at Bp.
+// NL = number of 8-row groups of the LAST row block (last = true) that hold training points (rows
+// >= n of L^-1 are identity padding and k* is zero there, so their products are exactly zero and
+// skipping them changes no bit of the result).
+template <int NL>
+__device__ __forceinline__ void var_row_block(const double* __restrict__ Linv, int64_t ld, int i, bool last,
+                                              const double* __restrict__ Bp, int64_t ldp, double* smem,
+                                              double (&blk)[4][2]) {
+    abg::Acc acc;
+    acc.zero();
+    if (NL < 16 && last)
+        abg::Main::mainloop<true, false, true, abg::NoGate, NL>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp,
+                                                               (i + 1) * (NB / abg::BK), smem);
+    else
+        abg::mainloop<true, false, true>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp, (i + 1) * (NB / abg::BK), smem);
+    tile_thread_sq(acc, blk);
+}
+
+// the 8 block values of this thread for one (row block, query tile) item of the split schedules,
+// where var_combine_kernel reads them
+__device__ __forceinline__ void store_part(double* __restrict__ part, int64_t item, const double (&blk)[4][2]) {
+    double* dst = part + (item * abg::THREADS + threadIdx.x) * 8;
+#pragma unroll
+    for (int j = 0; j < 4; j++) *reinterpret_cast<double2*>(dst + 2 * j) = make_double2(blk[j][0], blk[j][1]);
+}
+
 // sigma^2 for the 128 queries of this CTA:  amp - sum_i ( sum_k Linv[i][k] P[k][q] )^2.
 // Canonical summation order (shared with the split path below, so both give identical
 // bits): per thread, per row block a chain over the m-fragments starting at zero; the
 // block values added in block order; then the reduction tree of tile_finish_var.
-// NL = number of 8-row groups of the LAST row block that hold training points (rows >= n of
-// L^-1 are identity padding and k* is zero there, so their products are exactly zero and
-// skipping them changes no bit of the result).
 template <int NL>
 __global__ void __launch_bounds__(abg::THREADS, 1)
 predict_var_kernel(const double* __restrict__ Linv, int64_t ld, int T, const double* __restrict__ P, int64_t ldp,
@@ -157,15 +181,8 @@ predict_var_kernel(const double* __restrict__ Linv, int64_t ld, int T, const dou
 #pragma unroll
     for (int j = 0; j < 4; j++) tot[j][0] = tot[j][1] = 0.0;
     for (int i = 0; i < T; i++) {
-        abg::Acc acc;
-        acc.zero();
-        if (NL < 16 && i == T - 1)
-            abg::Main::mainloop<true, false, true, abg::NoGate, NL>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp,
-                                                                   (i + 1) * (NB / abg::BK), smem);
-        else
-            abg::mainloop<true, false, true>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp, (i + 1) * (NB / abg::BK), smem);
         double blk[4][2];
-        tile_thread_sq(acc, blk);
+        var_row_block<NL>(Linv, ld, i, i == T - 1, Bp, ldp, smem, blk);
 #pragma unroll
         for (int j = 0; j < 4; j++) { tot[j][0] += blk[j][0]; tot[j][1] += blk[j][1]; }
     }
@@ -182,15 +199,9 @@ predict_var_split_kernel(const double* __restrict__ Linv, int64_t ld, const doub
                          double* __restrict__ part) {
     extern __shared__ __align__(16) double smem[];
     const int i = blockIdx.y;
-    const double* Bp = P + (int64_t)blockIdx.x * abg::BN;
-    abg::Acc acc;
-    acc.zero();
-    abg::mainloop<true, false, true>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp, (i + 1) * (NB / abg::BK), smem);
     double blk[4][2];
-    tile_thread_sq(acc, blk);
-    double* dst = part + (((int64_t)i * gridDim.x + blockIdx.x) * abg::THREADS + threadIdx.x) * 8;
-#pragma unroll
-    for (int j = 0; j < 4; j++) *reinterpret_cast<double2*>(dst + 2 * j) = make_double2(blk[j][0], blk[j][1]);
+    var_row_block<16>(Linv, ld, i, false, P + (int64_t)blockIdx.x * abg::BN, ldp, smem, blk);
+    store_part(part, (int64_t)i * gridDim.x + blockIdx.x, blk);
 }
 
 // Full panels with many row blocks: predict_var_kernel gives one CTA the whole row-block loop of its
@@ -217,18 +228,9 @@ predict_var_pair_kernel(const double* __restrict__ Linv, int64_t ld, int T, int 
         for (int h = 0; h < 2; h++) {
             const int i = (h == 0) ? p : T - 1 - p;
             if (h == 1 && i == p) break;                         // middle row block of an odd T
-            abg::Acc acc;
-            acc.zero();
-            if (NL < 16 && i == T - 1)      // last row block: only the 8-row groups that hold training points
-                abg::Main::mainloop<true, false, true, abg::NoGate, NL>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp,
-                                                                       (i + 1) * (NB / abg::BK), smem);
-            else
-                abg::mainloop<true, false, true>(acc, Linv + (int64_t)i * NB * ld, ld, Bp, ldp, (i + 1) * (NB / abg::BK), smem);
             double blk[4][2];
-            tile_thread_sq(acc, blk);
-            double* dst = part + (((int64_t)i * ntq + q) * abg::THREADS + threadIdx.x) * 8;
-#pragma unroll
-            for (int j = 0; j < 4; j++) *reinterpret_cast<double2*>(dst + 2 * j) = make_double2(blk[j][0], blk[j][1]);
+            var_row_block<NL>(Linv, ld, i, i == T - 1, Bp, ldp, smem, blk);
+            store_part(part, (int64_t)i * ntq + q, blk);
         }
     }
 }
@@ -454,7 +456,6 @@ argmin_final_kernel(const double* __restrict__ bval, const long long* __restrict
 constexpr int FEW_MQ = 8;
 constexpr int FEW_ST = 4;                           // cp.async ring depth of few_gemv_kernel (8 stages measured: no gain, the warp is issue / chain bound)
 constexpr int FEW_GEMV_SMEM = FEW_ST * (32 * 34 + 32 * FEW_MQ) * 8;
-int padded_dim(int d);
 
 template <int KIND, int D>
 __global__ void __launch_bounds__(JCHUNK)
@@ -727,38 +728,13 @@ __global__ void few_grad_finish_kernel(const double* __restrict__ gpart, int nsp
     dvar[(int64_t)q * d + k] = -2.0 * f * sv;
 }
 
-template <int KIND>
-int launch_few_grad(ab_gp* h, int Dp, int nsplit, const double* Xq, int m, const double* V, double* gpart) {
-#define AB_FG(DD)                                                                                               \
-    few_grad_kernel<KIND, DD><<<nsplit, 512, 0, h->stream>>>(Xq, m, h->Xs, h->alpha, V, h->npad, h->n, h->npad, h->kp, gpart)
-    if (Dp <= 2) AB_FG(2);
-    else if (Dp <= 4) AB_FG(4);
-    else if (Dp <= 8) AB_FG(8);
-    else if (Dp <= 12) AB_FG(12);
-    else if (Dp <= 16) AB_FG(16);
-    else if (Dp <= 20) AB_FG(20);
-    else if (Dp <= 24) AB_FG(24);
-    else AB_FG(32);
-#undef AB_FG
-    AB_CHECK_LAUNCH();
-    return 0;
-}
-
-template <int KIND>
-int launch_few_cross(ab_gp* h, int Dp, int nsplit, const double* Xq, int m, double* P, double* partial) {
-#define AB_FC(DD)                                                                                              \
-    few_cross_kernel<KIND, DD><<<nsplit, JCHUNK, 0, h->stream>>>(Xq, m, h->Xs, h->alpha, h->n, h->npad, h->kp, P, partial)
-    if (Dp <= 2) AB_FC(2);
-    else if (Dp <= 4) AB_FC(4);
-    else if (Dp <= 8) AB_FC(8);
-    else if (Dp <= 12) AB_FC(12);
-    else if (Dp <= 16) AB_FC(16);
-    else if (Dp <= 20) AB_FC(20);
-    else if (Dp <= 24) AB_FC(24);
-    else AB_FC(32);
-#undef AB_FC
-    AB_CHECK_LAUNCH();
-    return 0;
+// f(std::integral_constant<int, MQ>{}) for the query count MQ of the few-query kernels that covers m
+template <class F>
+auto dispatch_mq(int m, F&& f) {
+    if (m == 1) return f(std::integral_constant<int, 1>{});
+    if (m == 2) return f(std::integral_constant<int, 2>{});
+    if (m <= 4) return f(std::integral_constant<int, 4>{});
+    return f(std::integral_constant<int, 8>{});
 }
 
 // mean (and variance, and their gradients w.r.t. the query) of m <= FEW_MQ queries;
@@ -777,109 +753,114 @@ int launch_few(ab_gp* h, const double* Xq, int m, double* mu, double* var, doubl
     double* partial = V + (size_t)h->npad * FEW_MQ;
     double* gpart = partial + (size_t)nsplit * FEW_MQ;
     ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
-    AB_DISPATCH_KIND(h->kp.kind, rc = (launch_few_cross<KIND>(h, h->d, nsplit, Xq, m, P, partial)));
+    AB_DISPATCH_KIND(h->kp.kind, ab_dispatch_dim(h->d, [&](auto D) {
+        few_cross_kernel<KIND, D><<<nsplit, JCHUNK, 0, s>>>(Xq, m, h->Xs, h->alpha, h->n, h->npad, h->kp, P, partial);
+    }));
     ab_prof_end(h, AB_PROF_PREDICT_PANEL);
-    if (rc) return rc;
+    AB_CHECK_LAUNCH();
+    const unsigned nb = (unsigned)(h->npad / 32);
     if (var) {
         ab_prof_begin(h, AB_PROF_PREDICT_VAR);
-        const unsigned nb = (unsigned)(h->npad / 32);
-#define AB_FGV(MQV)                                                                                                  \
-    do {                                                                                                             \
-        AB_CUDA(cudaFuncSetAttribute(few_gemv_kernel<MQV>, cudaFuncAttributeMaxDynamicSharedMemorySize, FEW_GEMV_SMEM)); \
-        few_gemv_kernel<MQV><<<nb, 32, FEW_GEMV_SMEM, s>>>(h->Linv, h->npad, P, Z);                                  \
-    } while (0)
-        if (m == 1) AB_FGV(1);
-        else if (m == 2) AB_FGV(2);
-        else if (m <= 4) AB_FGV(4);
-        else AB_FGV(8);
-#undef AB_FGV
+        rc = dispatch_mq(m, [&](auto MQ) {
+            AB_CUDA(cudaFuncSetAttribute(few_gemv_kernel<MQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, FEW_GEMV_SMEM));
+            few_gemv_kernel<MQ><<<nb, 32, FEW_GEMV_SMEM, s>>>(h->Linv, h->npad, P, Z);
+            return 0;
+        });
         ab_prof_end(h, AB_PROF_PREDICT_VAR);
+        if (rc) return rc;
         AB_CHECK_LAUNCH();
     }
     few_finish_kernel<<<1, 16 * FEW_MQ, 0, s>>>(var ? Z : nullptr, h->npad, T, partial, nsplit, m, h->kp.amp, h->mean, mu, var);
     AB_CHECK_LAUNCH();
     ab_count_launches(var ? 3 : 2);
     if (var && dmu && dvar) {
-        const unsigned nb = (unsigned)(h->npad / 32);
-        if (m == 1) few_gemv_t_kernel<1><<<nb, 32, 0, s>>>(h->Linv, h->npad, Z, V);
-        else if (m == 2) few_gemv_t_kernel<2><<<nb, 32, 0, s>>>(h->Linv, h->npad, Z, V);
-        else if (m <= 4) few_gemv_t_kernel<4><<<nb, 32, 0, s>>>(h->Linv, h->npad, Z, V);
-        else few_gemv_t_kernel<8><<<nb, 32, 0, s>>>(h->Linv, h->npad, Z, V);
-        AB_CHECK_LAUNCH();
-        const int Dp = padded_dim(h->d);
-        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_few_grad<KIND>(h, h->d, nsplit_g, Xq, m, V, gpart)));
-        if (rc) return rc;
-        few_grad_finish_kernel<<<1, FEW_MQ * AB_MAX_DIM, 0, s>>>(gpart, nsplit_g, Dp, m, h->kp, dmu, dvar);
+        dispatch_mq(m, [&](auto MQ) { few_gemv_t_kernel<MQ><<<nb, 32, 0, s>>>(h->Linv, h->npad, Z, V); });
+        AB_DISPATCH_KIND(h->kp.kind, ab_dispatch_dim(h->d, [&](auto D) {
+            few_grad_kernel<KIND, D><<<nsplit_g, 512, 0, s>>>(Xq, m, h->Xs, h->alpha, V, h->npad, h->n, h->npad, h->kp, gpart);
+        }));
+        few_grad_finish_kernel<<<1, FEW_MQ * AB_MAX_DIM, 0, s>>>(gpart, nsplit_g, ab_padded_dim(h->d), m, h->kp, dmu, dvar);
         AB_CHECK_LAUNCH();
         ab_count_launches(3);
     }
     return 0;
 }
 
-template <int KIND, bool STORE>
-int launch_mean(ab_gp* h, int Dp, dim3 grid, const double* Xq, int64_t m, int64_t q_off, double* mu, double* P,
-                int64_t ldp, int nsplit, double* partial, int64_t part_ld) {
-#define AB_PM(DD)                                                                                              \
-    predict_mean_kernel<KIND, DD, STORE><<<grid, 128, 0, h->stream>>>(Xq, m, q_off, h->Xs, h->alpha, h->n, h->npad, \
-                                                                      h->kp, h->mean, mu, P, ldp, nsplit, partial, part_ld)
-    if (Dp <= 2) AB_PM(2);
-    else if (Dp <= 4) AB_PM(4);
-    else if (Dp <= 8) AB_PM(8);
-    else if (Dp <= 12) AB_PM(12);
-    else if (Dp <= 16) AB_PM(16);
-    else if (Dp <= 20) AB_PM(20);
-    else if (Dp <= 24) AB_PM(24);
-    else AB_PM(32);
-#undef AB_PM
-    AB_CHECK_LAUNCH();
-    return 0;
+// f(std::integral_constant<int, NL>{}) for nl = 1..16 (the NL of predict_var_kernel)
+template <int NL = 1, class F>
+int dispatch_nl(int nl, F&& f) {
+    if constexpr (NL < 16) {
+        if (nl == NL) return f(std::integral_constant<int, NL>{});
+        return dispatch_nl<NL + 1>(nl, f);
+    } else {
+        return f(std::integral_constant<int, 16>{});
+    }
 }
+
+// chunks of JCHUNK training points the panel pass splits the training range into (grid.y)
+int panel_splits(const ab_gp* h) { return (int)((h->npad + JCHUNK - 1) / JCHUNK); }
 
 }  // namespace
 
+// The panel pass of queries [q0, q0 + cnt): their means, and with P their cross-covariance panel
+// P[j][q] (npad x ldp, ldp >= cnt rounded up to QPB).  predict_mean_kernel covers the training range
+// in panel_splits(h) fixed chunks (more CTAs, a summation order fixed by N); combine_splits_kernel
+// adds the chunk partials (panel_splits(h) x ldp) in chunk order.
+static int launch_panel(ab_gp* h, const double* Xq, int64_t m, int64_t q0, int64_t cnt, double* mu, double* P,
+                        int64_t ldp, double* partial) {
+    cudaStream_t s = h->stream;
+    const int nsplit = panel_splits(h);
+    const dim3 grid((unsigned)((cnt + QPB - 1) / QPB), (unsigned)nsplit);
+    ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
+    AB_DISPATCH_KIND(h->kp.kind, ab_dispatch_dim(h->d, [&](auto D) {
+        if (P)
+            predict_mean_kernel<KIND, D, true><<<grid, 128, 0, s>>>(Xq, m, q0, h->Xs, h->alpha, h->n, h->npad, h->kp,
+                                                                    h->mean, mu, P, ldp, nsplit, partial, ldp);
+        else
+            predict_mean_kernel<KIND, D, false><<<grid, 128, 0, s>>>(Xq, m, q0, h->Xs, h->alpha, h->n, h->npad, h->kp,
+                                                                     h->mean, mu, P, ldp, nsplit, partial, ldp);
+    }));
+    if (nsplit > 1)
+        combine_splits_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(partial, ldp, cnt, nsplit, h->kp.amp, h->mean,
+                                                                            mu, q0);
+    ab_prof_end(h, AB_PROF_PREDICT_PANEL);
+    AB_CHECK_LAUNCH();
+    ab_count_launches(nsplit > 1 ? 2 : 1);
+    return 0;
+}
 
 // sigma^2 for `cnt` queries of the panel P: one CTA per 128 queries looping over the row
-// blocks, or (few query tiles) the row blocks spread over the grid
+// blocks, or the row blocks spread over the grid (few query tiles, or full panels with many
+// row blocks), their per-thread block values in `part` (T x ldp x 16)
 static int launch_variance(ab_gp* h, int T, const double* P, int64_t ldp, int64_t m, int64_t q0, int64_t cnt,
                            double* var, double* part) {
     cudaStream_t s = h->stream;
     const unsigned ntq = (unsigned)((cnt + abg::BN - 1) / abg::BN);
+    const int nl = (int)((h->n - (int64_t)(T - 1) * NB + 7) / 8);        // 1..16 row groups in the last block
     // row-block pairs of a tile on adjacent CTAs from N >= 6144 (measured: 0.2 % slower at N = 8192 for a quarter of the DRAM traffic, 3 % slower at N = 4000)
-    const bool pair = part && T >= 48 && (int)ntq * 2 > h->nsm;
-    if (pair) {
+    if (T >= 48 && (int)ntq * 2 > h->nsm) {
         const long long nitems = (long long)((T + 1) / 2) * ntq;
         const unsigned grid = (unsigned)(nitems < h->nsm ? nitems : h->nsm);
-        const int nlp = (int)((h->n - (int64_t)(T - 1) * NB + 7) / 8);       // 1..16 row groups in the last block
-#define AB_PP(NLV)                                                                                                 \
-    case NLV:                                                                                                      \
-        AB_CUDA(cudaFuncSetAttribute(predict_var_pair_kernel<NLV>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES)); \
-        predict_var_pair_kernel<NLV><<<grid, abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, (int)ntq, P, ldp, part); \
-        break
-        switch (nlp) {
-            AB_PP(1); AB_PP(2); AB_PP(3); AB_PP(4); AB_PP(5); AB_PP(6); AB_PP(7); AB_PP(8);
-            AB_PP(9); AB_PP(10); AB_PP(11); AB_PP(12); AB_PP(13); AB_PP(14); AB_PP(15);
-            default: AB_PP(16);
-        }
-#undef AB_PP
+        const int rc = dispatch_nl(nl, [&](auto NL) {
+            AB_CUDA(cudaFuncSetAttribute(predict_var_pair_kernel<NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
+            predict_var_pair_kernel<NL><<<grid, abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, (int)ntq, P, ldp, part);
+            return 0;
+        });
+        if (rc) return rc;
         var_combine_kernel<<<ntq, abg::THREADS, 0, s>>>(part, T, m, q0, h->kp.amp, var);
-        ab_count_launches(1);
-    } else if (T > 1 && (int)ntq * 2 <= h->nsm && part) {
+        ab_count_launches(2);
+    } else if (T > 1 && (int)ntq * 2 <= h->nsm) {
+        AB_CUDA(cudaFuncSetAttribute(predict_var_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
         predict_var_split_kernel<<<dim3(ntq, T), abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, P, ldp, part);
         var_combine_kernel<<<ntq, abg::THREADS, 0, s>>>(part, T, m, q0, h->kp.amp, var);
-        ab_count_launches(1);
+        ab_count_launches(2);
     } else {
-        const int nl = (int)((h->n - (int64_t)(T - 1) * NB + 7) / 8);        // 1..16 row groups in the last block
-#define AB_PV(NLV)                                                                                                 \
-    case NLV:                                                                                                      \
-        AB_CUDA(cudaFuncSetAttribute(predict_var_kernel<NLV>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES)); \
-        predict_var_kernel<NLV><<<ntq, abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, P, ldp, m, q0, h->kp.amp, var); \
-        break
-        switch (nl) {
-            AB_PV(1); AB_PV(2); AB_PV(3); AB_PV(4); AB_PV(5); AB_PV(6); AB_PV(7); AB_PV(8);
-            AB_PV(9); AB_PV(10); AB_PV(11); AB_PV(12); AB_PV(13); AB_PV(14); AB_PV(15);
-            default: AB_PV(16);
-        }
-#undef AB_PV
+        const int rc = dispatch_nl(nl, [&](auto NL) {
+            AB_CUDA(cudaFuncSetAttribute(predict_var_kernel<NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
+            predict_var_kernel<NL><<<ntq, abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, P, ldp, m, q0, h->kp.amp, var);
+            return 0;
+        });
+        if (rc) return rc;
+        ab_count_launches(1);
     }
     AB_CHECK_LAUNCH();
     return 0;
@@ -888,7 +869,8 @@ static int launch_variance(ab_gp* h, int T, const double* P, int64_t ldp, int64_
 // queries per variance panel: one wave of CTAs (148 SMs x 128 queries)
 static const int64_t kPanelQueries = 148 * 128;
 
-// queries per variance panel for the current training-set size (what ab_launch_predict uses)
+// queries per variance panel for the current training-set size: whole waves of variance CTAs, as many
+// as fit a ~2 GB cross-covariance panel
 int64_t ab_predict_panel_queries(ab_gp* h) {
     int64_t waves = (int64_t)((2ULL << 30) / ((size_t)h->npad * kPanelQueries * sizeof(double)));
     if (waves < 1) waves = 1;
@@ -899,145 +881,76 @@ int64_t ab_predict_panel_queries(ab_gp* h) {
 int ab_launch_predict(ab_gp* h, const double* Xq, int64_t m, double* mu, double* var) {
     if (m <= 0) return 0;
     if (m <= FEW_MQ && h->few_path) return launch_few(h, Xq, (int)m, mu, var);
-    cudaStream_t s = h->stream;
-    const int d = h->d;
+    const int nsplit = panel_splits(h);
     if (!var) {
-        int64_t nblk = (m + QPB - 1) / QPB;
-        const int nsplit = (int)((h->npad + JCHUNK - 1) / JCHUNK);
-        double* partial = nullptr;
-        const int64_t part_ld = nblk * QPB;
+        const int64_t ldp = (m + QPB - 1) / QPB * QPB;
         if (nsplit > 1) {
-            int rc = ab_ensure_scratch(h, (size_t)nsplit * part_ld * sizeof(double));
+            const int rc = ab_ensure_scratch(h, (size_t)nsplit * ldp * sizeof(double));
             if (rc) return rc;
-            partial = h->scratch;
         }
-        dim3 grid((unsigned)nblk, (unsigned)nsplit);
-        int rc = 0;
-        ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
-        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_mean<KIND, false>(h, d, grid, Xq, m, 0, mu, nullptr, 0, nsplit, partial, part_ld)));
-        ab_prof_end(h, AB_PROF_PREDICT_PANEL);
-        ab_count_launches(nsplit > 1 ? 2 : 1);
-        if (rc) return rc;
-        if (nsplit > 1) {
-            combine_splits_kernel<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(partial, part_ld, m, nsplit, h->kp.amp,
-                                                                              h->mean, mu, 0);
-            AB_CHECK_LAUNCH();
-        }
-        return 0;
+        return launch_panel(h, Xq, m, 0, m, mu, nullptr, ldp, nsplit > 1 ? h->scratch : nullptr);
     }
-    // mean + variance, processed in panels.  Panel width: whole waves of variance CTAs
-    // (148 x 128 queries), as many as fit a ~2 GB cross-covariance panel.
+    // mean + variance, processed in panels
     const int T = (int)(h->npad / NB);
-    int64_t waves = (int64_t)((2ULL << 30) / ((size_t)h->npad * kPanelQueries * sizeof(double)));
-    if (waves < 1) waves = 1;
-    if (waves > 16) waves = 16;
-    int64_t mq = waves * kPanelQueries;
-    if (m < mq) mq = m;
+    const int64_t mq = std::min(m, ab_predict_panel_queries(h));
     const int64_t ldp = (mq + QPB - 1) / QPB * QPB;                 // multiple of 256 (and of 128)
-    const int64_t nblk = ldp / QPB;
-    // the training range is split over grid.y in fixed chunks (more CTAs, fixed summation order)
-    const int nsplit = (int)((h->npad + JCHUNK - 1) / JCHUNK);
-    (void)nblk;
     const size_t panel_elems = (size_t)h->npad * ldp;
-    const bool few = true;            // per-thread block values: split-T (few tiles) and paired (full panels) schedules
-    int rc = ab_ensure_scratch(h, (panel_elems + (size_t)nsplit * ldp + (few ? (size_t)T * ldp * 16 : 0)) * sizeof(double));
+    int rc = ab_ensure_scratch(h, (panel_elems + (size_t)nsplit * ldp + (size_t)T * ldp * 16) * sizeof(double));
     if (rc) return rc;
-    AB_CUDA(cudaFuncSetAttribute(predict_var_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
     double* P = h->scratch;
     double* partial = h->scratch + panel_elems;
-    double* vpart = few ? partial + (size_t)nsplit * ldp : nullptr;
+    double* vpart = partial + (size_t)nsplit * ldp;
     for (int64_t q0 = 0; q0 < m; q0 += mq) {
-        int64_t cnt = (m - q0 < mq) ? (m - q0) : mq;
-        dim3 grid((unsigned)((cnt + QPB - 1) / QPB), (unsigned)nsplit);
-        ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
-        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_mean<KIND, true>(h, d, grid, Xq, m, q0, mu, P, ldp, nsplit, partial, ldp)));
+        const int64_t cnt = (m - q0 < mq) ? (m - q0) : mq;
+        rc = launch_panel(h, Xq, m, q0, cnt, mu, P, ldp, partial);
         if (rc) return rc;
-        if (nsplit > 1) {
-            combine_splits_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(partial, ldp, cnt, nsplit, h->kp.amp,
-                                                                                h->mean, mu, q0);
-            AB_CHECK_LAUNCH();
-        }
-        ab_prof_end(h, AB_PROF_PREDICT_PANEL);
         ab_prof_begin(h, AB_PROF_PREDICT_VAR);
         rc = launch_variance(h, T, P, ldp, m, q0, cnt, var, vpart);
         ab_prof_end(h, AB_PROF_PREDICT_VAR);
         if (rc) return rc;
-        ab_count_launches(nsplit > 1 ? 3 : 2);
     }
     return 0;
 }
-
-
-template <int KIND>
-static int launch_grad_points(ab_gp* h, int Dp, dim3 grid, const double* Xq, int64_t m, int64_t q0, const double* V,
-                              int64_t ldp, double* partial) {
-#define AB_PG(DD)                                                                                                 \
-    predict_grad_kernel<KIND, DD><<<grid, 128, 0, h->stream>>>(Xq, m, q0, h->Xs, h->alpha, V, ldp, h->n, h->npad, h->kp, \
-                                                                partial, ldp)
-    if (Dp <= 2) AB_PG(2);
-    else if (Dp <= 4) AB_PG(4);
-    else if (Dp <= 8) AB_PG(8);
-    else if (Dp <= 12) AB_PG(12);
-    else if (Dp <= 16) AB_PG(16);
-    else if (Dp <= 20) AB_PG(20);
-    else if (Dp <= 24) AB_PG(24);
-    else AB_PG(32);
-#undef AB_PG
-    AB_CHECK_LAUNCH();
-    return 0;
-}
-
-namespace {
-int padded_dim(int d) {
-    const int opts[] = {2, 4, 8, 12, 16, 20, 24, 32};
-    for (int o : opts) if (d <= o) return o;
-    return 32;
-}
-}  // namespace
 
 // mean, variance and their gradients w.r.t. the query coordinates (row-major m x d)
 int ab_launch_predict_grad(ab_gp* h, const double* Xq, int64_t m, double* mu, double* var, double* dmu, double* dvar) {
     if (m <= 0) return 0;
     if (m <= FEW_MQ && h->few_path) return launch_few(h, Xq, (int)m, mu, var, dmu, dvar);
     cudaStream_t s = h->stream;
-    const int d = h->d, D = padded_dim(d);
+    const int d = h->d, Dp = ab_padded_dim(d);
     AB_CUDA(cudaFuncSetAttribute(tri_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
     AB_CUDA(cudaFuncSetAttribute(tri_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
     const int T = (int)(h->npad / NB);
     int64_t mq = m < 1024 ? m : 1024;                              // queries per panel
     const int64_t ldp = (mq + QPB - 1) / QPB * QPB;
-    const int nsplit = (int)((h->npad + JCHUNK - 1) / JCHUNK);
+    const int nsplit = panel_splits(h);
     const size_t panel = (size_t)h->npad * ldp;
-    int rc = ab_ensure_scratch(h, (3 * panel + (size_t)nsplit * ldp * (1 + 2 * D) + (size_t)T * ldp * 16) * sizeof(double));
+    int rc = ab_ensure_scratch(h, (3 * panel + (size_t)nsplit * ldp * (1 + 2 * Dp) + (size_t)T * ldp * 16) * sizeof(double));
     if (rc) return rc;
-    AB_CUDA(cudaFuncSetAttribute(predict_var_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, abg::SMEM_BYTES));
     double* P = h->scratch;
     double* W = P + panel;
     double* V = W + panel;
     double* partial = V + panel;                                   // [nsplit][ldp] mean partials
-    double* gpartial = partial + (size_t)nsplit * ldp;             // [nsplit][2 D][ldp]
+    double* gpartial = partial + (size_t)nsplit * ldp;             // [nsplit][2 Dp][ldp]
     for (int64_t q0 = 0; q0 < m; q0 += mq) {
         const int64_t cnt = (m - q0 < mq) ? (m - q0) : mq;
-        dim3 grid((unsigned)((cnt + QPB - 1) / QPB), (unsigned)nsplit);
-        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_mean<KIND, true>(h, d, grid, Xq, m, q0, mu, P, ldp, nsplit, partial, ldp)));
+        rc = launch_panel(h, Xq, m, q0, cnt, mu, P, ldp, partial);
         if (rc) return rc;
-        if (nsplit > 1) {
-            combine_splits_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(partial, ldp, cnt, nsplit, h->kp.amp,
-                                                                              h->mean, mu, q0);
-        }
         const unsigned ntq = (unsigned)((cnt + abg::BN - 1) / abg::BN);
-        rc = launch_variance(h, T, P, ldp, m, q0, cnt, var, gpartial + (size_t)nsplit * 2 * D * ldp);
+        rc = launch_variance(h, T, P, ldp, m, q0, cnt, var, gpartial + (size_t)nsplit * 2 * Dp * ldp);
         if (rc) return rc;
         tri_gemm_kernel<false><<<dim3(ntq, T), abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, P, ldp, W);
         tri_gemm_kernel<true><<<dim3(ntq, T), abg::THREADS, abg::SMEM_BYTES, s>>>(h->Linv, h->npad, T, W, ldp, V);
         AB_CHECK_LAUNCH();
         dim3 ggrid((unsigned)((cnt + 127) / 128), (unsigned)nsplit);
-        AB_DISPATCH_KIND(h->kp.kind, rc = (launch_grad_points<KIND>(h, d, ggrid, Xq, m, q0, V, ldp, gpartial)));
-        if (rc) return rc;
-        grad_combine_kernel<<<(unsigned)((cnt * d + 255) / 256), 256, 0, s>>>(gpartial, ldp, cnt, nsplit, D, d, h->kp, dmu,
+        AB_DISPATCH_KIND(h->kp.kind, ab_dispatch_dim(d, [&](auto D) {
+            predict_grad_kernel<KIND, D><<<ggrid, 128, 0, s>>>(Xq, m, q0, h->Xs, h->alpha, V, ldp, h->n, h->npad, h->kp,
+                                                               gpartial, ldp);
+        }));
+        grad_combine_kernel<<<(unsigned)((cnt * d + 255) / 256), 256, 0, s>>>(gpartial, ldp, cnt, nsplit, Dp, d, h->kp, dmu,
                                                                             dvar, q0);
         AB_CHECK_LAUNCH();
-        ab_count_launches(7);
+        ab_count_launches(4);
     }
     return 0;
 }
@@ -1164,7 +1077,7 @@ int ab_launch_predict_cov(ab_gp* h, const double* Xq, int64_t m, double* mu, dou
     cudaStream_t s = h->stream;
     const int d = h->d, T = (int)(h->npad / NB);
     const int64_t ldp = (m + QPB - 1) / QPB * QPB;
-    const int nsplit = (int)((h->npad + JCHUNK - 1) / JCHUNK);
+    const int nsplit = panel_splits(h);
     const int ntq = (int)((m + abg::BN - 1) / abg::BN);
     const size_t panel = (size_t)h->npad * ldp;
     int rc = ab_ensure_scratch(h, (2 * panel + (size_t)nsplit * ldp + ldp + (size_t)m * d) * sizeof(double));
@@ -1177,17 +1090,9 @@ int ab_launch_predict_cov(ab_gp* h, const double* Xq, int64_t m, double* mu, dou
     double* partial = W + panel;
     double* dv = partial + (size_t)nsplit * ldp;
     double* XT = dv + ldp;
-    // 1. panel P and mean (the launches of ab_launch_predict's panel pass)
-    ab_prof_begin(h, AB_PROF_PREDICT_PANEL);
-    dim3 grid((unsigned)(ldp / QPB), (unsigned)nsplit);
-    AB_DISPATCH_KIND(h->kp.kind, rc = (launch_mean<KIND, true>(h, d, grid, Xq, m, 0, mu, P, ldp, nsplit, partial, ldp)));
+    // 1. panel P and mean
+    rc = launch_panel(h, Xq, m, 0, m, mu, P, ldp, partial);
     if (rc) return rc;
-    if (nsplit > 1) {
-        combine_splits_kernel<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(partial, ldp, m, nsplit, h->kp.amp, h->mean, mu, 0);
-        AB_CHECK_LAUNCH();
-    }
-    ab_prof_end(h, AB_PROF_PREDICT_PANEL);
-    ab_count_launches(nsplit > 1 ? 2 : 1);
     // 2. W = L^-1 P
     ab_prof_begin(h, AB_PROF_PREDICT_VAR);
     rc = ab_launch_tri_gemm_lower(h, h->Linv, h->npad, T, P, ldp, ntq, W);

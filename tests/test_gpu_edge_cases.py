@@ -40,14 +40,27 @@ def test_ragged_sizes_around_the_block_boundaries(n):
     _check(o, g, y, rng.uniform(-1, 1, size=(17, 2)))
 
 
-@pytest.mark.parametrize("d", [1, 3, 17, 32])
+# both ends of every compiled dimension bucket (2, 4, 8, 12, 16, 20, 24, 32)
+@pytest.mark.parametrize("d", [1, 2, 3, 4, 5, 8, 9, 12, 13, 16, 17, 20, 21, 24, 25, 32])
 def test_dimensions_up_to_the_maximum(d):
     rng = np.random.default_rng(d)
     n = 200
     X = rng.uniform(-1, 1, size=(n, d))
     y = np.sin(X.sum(axis=1)) + 0.01 * rng.normal(size=n)
     o, g = _pair("ExpSquaredKernel", X, y, rng.uniform(0.5, 1.5, size=d))
-    _check(o, g, y, rng.uniform(-1, 1, size=(33, d)))
+    t = rng.uniform(-1, 1, size=(33, d))
+    _check(o, g, y, t)
+    amp = np.exp(o.log_const)
+    # one query (the few-query kernels)
+    m1, v1 = g.predict(y, t[:1], return_var=True)
+    mo, vo = o.predict(y, t[:1], return_var=True)
+    assert abs(m1[0] - mo[0]) <= 1e-9 * max(abs(mo[0]), 1e-3) and abs(v1[0] - vo[0]) <= 1e-9 * amp
+    # gradients of the mean and variance: few-query and batched kernels
+    for tq in (t[:3], t):
+        _, _, dmu_g, dvar_g = g.predict_grad(y, tq)
+        dmu_o, dvar_o = o.predict_grad(y, tq)
+        assert np.max(np.abs(dmu_g - dmu_o)) <= 1e-8 * np.max(np.abs(dmu_o))
+        assert np.max(np.abs(dvar_g - dvar_o)) <= 1e-8 * max(np.max(np.abs(dvar_o)), 1e-6 * amp)
     import alabi_b200 as ab
     with pytest.raises(Exception):
         ab.GP(kernel=ab.kernels.ExpSquaredKernel(metric=np.ones(33), ndim=33)).compute(rng.uniform(size=(10, 33)))

@@ -34,7 +34,9 @@ def surrogate(kind, n, d, seed, bounds):
 @pytest.mark.parametrize("kind,n,d,nw,rs,wpu", [("ExpSquaredKernel", 200, 2, 32, True, 0),
                                                 ("Matern32Kernel", 300, 3, 41, False, 1),
                                                 ("Matern52Kernel", 700, 5, 64, True, 2),
-                                                ("ExpSquaredKernel", 150, 2, 10, True, 8)])
+                                                ("ExpSquaredKernel", 150, 2, 10, True, 8),
+                                                ("Matern32Kernel", 250, 15, 48, True, 0),
+                                                ("ExpSquaredKernel", 300, 23, 64, False, 0)])
 def test_chain_replay_and_per_proposal_logp(kind, n, d, nw, rs, wpu):
     from alabi_b200.ensemble import EnsembleSampler
     bounds = [(-2.0, 2.0)] * d

@@ -30,7 +30,9 @@ def _surrogate(kind, n, d, seed, bounds, y_scale=1.0, y_offset=0.0):
 
 @pytest.mark.parametrize("kind,n,d,nchains,normal", [("ExpSquaredKernel", 300, 2, 37, False),
                                                      ("Matern52Kernel", 900, 5, 96, True),
-                                                     ("Matern32Kernel", 2600, 12, 64, False)])
+                                                     ("Matern32Kernel", 2600, 12, 64, False),
+                                                     ("Matern52Kernel", 500, 14, 48, True),
+                                                     ("ExpSquaredKernel", 600, 22, 40, False)])
 def test_device_walk_replays_on_the_cpu(kind, n, d, nchains, normal):
     from alabi_b200.nested import DeviceWalker
     g, lp, like_o, rng, b = _surrogate(kind, n, d, 5, [(-2.0, 2.0)] * d, y_scale=1.5, y_offset=-0.25)
